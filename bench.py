@@ -1,6 +1,6 @@
 """bench.py -- env-steps/s of the batched WaypointQuadEnv step on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload rollout|step] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload rollout|step] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +18,12 @@ Printed JSON (one line, rank 0): the base contract + `roofline` (dominant kernel
 tensor peak; `roofline_other`: the HBM-bound env step), `cpu_baseline` (the CPU oracle port of the reference step on the host
 cores), `e2e` (same metric through the SB3-style VecEnv / predict calls with pinned host buffers, copies inside the timed
 region), `gpu_launches`, `clocks`.
+
+--dump-outputs DIR: after the K timed steps, the arrays the last timed step handed its caller (env step: obs, reward, flags,
+terminal_obs, ep_return, ep_len; rollout: also the policy's actions, actions_clipped, values, log_prob and the VecNormalize
+running statistics) go to DIR/<name>.npy as float32 / float64 (integers as float64), rank 0's shard only.  Per-env arrays keep
+a fixed, seeded sample of at most 65,536 envs (their indices in env_index.npy).  Seeds, weights and step counts come from the
+arguments alone, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -256,6 +262,31 @@ def workload_name(args) -> str:
     return f"v2_{args.workload}_{tag}_{args.precision}"
 
 
+DUMP_MAX_ENVS = 1 << 16       # about 15 MB of .npy files for the v2 rollout outputs
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path: str, per_env: dict, whole: dict, n: int) -> None:
+    """Write device tensors as DIR/<name>.npy: `per_env` ([n, ...] rows) on a fixed, seeded sample of the envs, `whole` as they are.
+    float64 stays float64, every other dtype becomes float32 (floats) or float64 (integers, exact)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    idx = np.arange(n) if n <= DUMP_MAX_ENVS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_ENVS, replace=False))
+    arrays = {"env_index": idx.astype(np.float64)}
+    for name, t in per_env.items():
+        arrays[name] = t.index_select(0, torch.from_numpy(idx).to(t.device)).cpu().numpy()
+    arrays.update({name: t.cpu().numpy() for name, t in whole.items()})
+    for name, a in arrays.items():
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64 if a.dtype.kind in "iub" else np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------
 # GPU arm
 # --------------------------------------------------------------------------------------------------
@@ -458,6 +489,15 @@ def run_gpu(args) -> None:
         raise RuntimeError(f"rollout kernel: an internal hand-over timed out (code {fused.status()}); the timed region is invalid")
     if vn is not None and vn.exchange_failed():
         raise RuntimeError("peer-memory moment exchange timed out waiting for a rank; the timed region is invalid")
+    if args.dump_outputs and rank == 0:
+        # before anything below steps the env again: the buffers still hold the last timed step's results
+        per_env = {"obs": env.obs, "reward": env.reward, "flags": env.flags, "terminal_obs": env.terminal_obs,
+                   "ep_return": env.ep_return, "ep_len": env.ep_len}
+        src = fused if fused is not None else policy
+        if src is not None:
+            per_env.update(actions=src.actions, actions_clipped=src.actions_clipped, values=src.values, log_prob=src.logp)
+        whole = {"obs_rms_count": vn.count.reshape(1), "obs_rms_mean": vn.mean, "obs_rms_var": vn.var} if vn is not None else {}
+        dump_outputs(args.dump_outputs, per_env, whole, n)
 
     # ---- per-kernel durations for the roofline: each component alone, replayed from its own CUDA graph (no host launch gaps), on one
     # rank at a time only where it has no rendezvous.  With one component the step IS the kernel.
@@ -620,6 +660,8 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra single-GPU workload lines (configs[2], float64, LSODA)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-baseline-only", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (rank 0; per-env arrays on a fixed sample of <= 65,536 envs)")
     args = ap.parse_args()
     if args.workload is None:
         args.workload = "rollout" if os.path.exists(os.path.join(ROOT, "rl-aerial-manipulator_b200", "policy.py")) else "step"

@@ -203,3 +203,27 @@ def test_ctypes_structs_match_the_header_layout(tmp_path):
         assert int(val) == want, (cname, field, int(val), want)
         seen += 1
     assert seen == sum(len(c._fields_) + 1 for c in structs.values())
+
+
+def test_bench_dump_outputs_sample_and_dtypes(tmp_path):
+    """bench.py --dump-outputs: per-env rows on the same seeded env sample every time, float32 / float64 only, within 64 MB."""
+    import bench
+    n = bench.DUMP_MAX_ENVS + 1000
+    g = torch.Generator().manual_seed(0)
+    per_env = {"obs": torch.randn((n, 20), generator=g), "reward": torch.randn(n, generator=g, dtype=torch.float64),
+               "flags": torch.randint(0, 256, (n,), generator=g, dtype=torch.uint8), "ep_len": torch.arange(n, dtype=torch.int32)}
+    whole = {"obs_rms_mean": torch.randn(20, generator=g, dtype=torch.float64)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), per_env, whole, n)
+    got = {f: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert sorted(got) == ["env_index.npy", "ep_len.npy", "flags.npy", "obs.npy", "obs_rms_mean.npy", "reward.npy"]
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / f)) for f, a in got.items())
+    idx = got["env_index.npy"].astype(np.int64)
+    assert len(idx) == bench.DUMP_MAX_ENVS and np.all(np.diff(idx) > 0) and idx[-1] < n
+    assert got["obs.npy"].dtype == np.float32 and np.array_equal(got["obs.npy"], per_env["obs"].numpy()[idx])
+    assert got["reward.npy"].dtype == np.float64 and np.array_equal(got["reward.npy"], per_env["reward"].numpy()[idx])
+    assert got["flags.npy"].dtype == np.float64 and np.array_equal(got["flags.npy"], per_env["flags"].numpy()[idx])
+    assert np.array_equal(got["ep_len.npy"], idx.astype(np.float64))
+    assert np.array_equal(got["obs_rms_mean.npy"], whole["obs_rms_mean"].numpy())
+    with pytest.raises(RuntimeError, match="budget"):
+        bench.dump_outputs(str(tmp_path / "c"), {"obs": torch.zeros((n, 300))}, {}, n)

@@ -34,18 +34,6 @@ def test_vecnormalize_pkl_roundtrip_and_class_paths(tmp_path, golden_dir):
     assert "stable_baselines3" not in sys.modules   # the spoofed module entries are removed again
 
 
-@pytest.mark.reference
-def test_reads_the_reference_pkl_directly(golden_dir):
-    ref = "/root/reference/initial-implementation-v1/vec_normalize.pkl"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present")
-    from rl_aerial_manipulator_b200 import sb3_compat as sc
-    st = sc.load_vecnormalize_pkl(ref)
-    z = np.load(os.path.join(golden_dir, "vecnorm_v1.npz"))
-    np.testing.assert_array_equal(st["obs_mean"], z["obs_mean"])
-    assert st["obs_count"] == 2031632.0001 and st["ret_count"] == 2031616.0001
-
-
 def test_policy_zip_writer(tmp_path, golden_dir):
     from rl_aerial_manipulator_b200 import sb3_compat as sc
     z = np.load(os.path.join(golden_dir, "policy_v2.npz"))
