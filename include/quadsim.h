@@ -198,6 +198,31 @@ int qs_reset_uniforms(qs_handle* h, const int64_t* env_ids, const int32_t* episo
                       void* stream);
 
 /*
+ * Dynamics randomisation (opt-in): per env and per episode, the true mass m*k_m, inertia k_I*I (inverse I^-1/k_I), per-prop
+ * thrust factors eta[4] (prop i delivers eta_i * clamp((invA [Fcmd; Mcmd])_i, tmin, tmax), F and M re-mixed from that) and a
+ * constant world-frame wind force f_wind[3] in N (dv/dt += f_wind / (m*k_m)).  The action scaling keeps the nominal mass: the
+ * controller commands thrust in units of the nominal m*g.  Observations, reward, termination and the reset draws are unchanged.
+ * Drawn at every reset (qs_reset, and the auto-reset of qs_step / qs_step_range / qs_step_many) for the episode number that
+ * reset uses:  u[0..9] = u53 pairs of Philox4x32-10, key = seed, counter = (global env id lo, hi, episode, 0x100 + b), b = 0..4;
+ *   k_m = 1 + mass_rel*(2u0-1),  k_I = 1 + inertia_rel*(2u1-1),  eta_i = 1 + thrust_rel*(2u_{2+i}-1),  f_wind_j = wind*(2u_{6+j}-1)
+ * in float64 with round-to-nearest products and sums (stored rounded to float on a QS_F32 handle).
+ * Valid: 0 <= mass_rel < 1, 0 <= inertia_rel < 1, 0 <= thrust_rel <= 1 (eta = 0 is a dead motor), wind >= 0, all finite.
+ * RK4 handles only; while armed, qs_rollout_step and the QS_STEP_F32_TMA opt-in kernel refuse (QS_EINVAL).
+ * qs_dynamics_randomization: cfg NULL disarms.  May be called before or after the first qs_reset; on a reset handle it draws every
+ *   env's parameters for its current episode.
+ * qs_get_dynamics / qs_set_dynamics: f64[n, QS_DYN_PARAMS] device rows (k_m, k_I, eta[4], f_wind[3]); set values hold until that
+ *   env's next reset.  Both need an armed handle.
+ */
+#define QS_DYN_PARAMS 9   /* k_m, k_I, eta[4], f_wind[3] */
+typedef struct qs_dynamics_rand {
+    uint64_t seed;
+    double mass_rel, inertia_rel, thrust_rel, wind;
+} qs_dynamics_rand;
+int qs_dynamics_randomization(qs_handle* h, const qs_dynamics_rand* cfg, void* stream);
+int qs_get_dynamics(qs_handle* h, double* out, void* stream);
+int qs_set_dynamics(qs_handle* h, const double* in, void* stream);
+
+/*
  * LSODA diagnostics of the most recent qs_step in QS_LSODA mode: i32[n,4] = nst, nfe, nqu, status and
  * f64[n,2] = hu, tcur -- the counters scipy's odeint(full_output=True) reports.  Either may be NULL.
  */

@@ -83,6 +83,15 @@ def make_config(env_version=2, n_envs=1, precision="f32", integrator="rk4", subs
     return c
 
 
+DYN_PARAMS = 9   # k_m, k_I, eta[4], f_wind[3]
+
+
+class QsDynamicsRand(C.Structure):
+    """qs_dynamics_rand of include/quadsim.h."""
+    _fields_ = [("seed", C.c_uint64), ("mass_rel", C.c_double), ("inertia_rel", C.c_double), ("thrust_rel", C.c_double),
+                ("wind", C.c_double)]
+
+
 class QsRolloutArgs(C.Structure):
     """qs_rollout_args of include/quadsim.h."""
     _fields_ = [("policy_image", C.c_void_p), ("obs", C.c_void_p), ("norm_stats", C.c_void_p),
@@ -155,6 +164,9 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.qs_set_state.argtypes = [vp, C.POINTER(QsStateView), vp]
     lib.qs_reset_uniforms.argtypes = [vp, vp, vp, i64, vp, vp]
     lib.qs_lsoda_stats.argtypes = [vp, vp, vp, vp]
+    lib.qs_dynamics_randomization.argtypes = [vp, C.POINTER(QsDynamicsRand), vp]
+    lib.qs_get_dynamics.argtypes = [vp, vp, vp]
+    lib.qs_set_dynamics.argtypes = [vp, vp, vp]
     lib.qs_policy_image_bytes.restype = i64
     lib.qs_policy_prepare.argtypes = [vp, i32, vp, vp]
     lib.qs_policy_prepare.restype = C.c_int
@@ -179,7 +191,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.qs_pid_run.argtypes = [vp, C.POINTER(QsPidGains), C.c_double] + [vp] * 8 + [i32, vp]
     lib.qs_pid_run.restype = C.c_int
     for name in ("qs_create", "qs_destroy", "qs_obs_dim", "qs_reset", "qs_step", "qs_get_state", "qs_set_state",
-                 "qs_reset_uniforms", "qs_lsoda_stats", "qs_step_moments"):
+                 "qs_reset_uniforms", "qs_lsoda_stats", "qs_step_moments", "qs_dynamics_randomization", "qs_get_dynamics",
+                 "qs_set_dynamics"):
         getattr(lib, name).restype = C.c_int
     if lib.qs_abi_version() != QS_ABI_VERSION:
         raise RuntimeError(f"libquadsim ABI {lib.qs_abi_version()} != binding ABI {QS_ABI_VERSION}; rebuild")

@@ -56,12 +56,17 @@ class BatchedQuadEnv:
     """N independent WaypointQuadEnv instances stepped by one fused sm_100a kernel.
 
     v2_random_waypoints (env_version 2): False = `num_waypoints = 1` as the reference ships it (rl_env_scaledObs.py:47); True = the
-    `np.random.randint(2, 4)` alternative it keeps commented out at :46 -- trajectories of 2 or 3 waypoints."""
+    `np.random.randint(2, 4)` alternative it keeps commented out at :46 -- trajectories of 2 or 3 waypoints.
+
+    dynamics_randomization (RK4 only): None = the nominal airframe, or a dict {"mass", "inertia", "thrust", "wind"[, "seed"]} --
+    every episode of every env then draws its own true mass mass*(1 +- mass), inertia I*(1 +- inertia), per-prop thrust factors
+    1 +- thrust and a constant world-frame wind force of up to +-wind N per axis (uniform; seed defaults to the env seed).  The
+    action scaling keeps the nominal mass.  See `randomize_dynamics`, `dynamics`, `set_dynamics`."""
 
     def __init__(self, n_envs: int, env_version: int = 2, precision: str = "f32", integrator: str = "rk4",
                  substeps: int = 1, obs_scaled: bool = True, action_scale_f32: bool = True, auto_reset: bool = True,
                  device: int | torch.device | None = None, env_id_offset: int = 0, seed: int = 0,
-                 v2_random_waypoints: bool = False):
+                 v2_random_waypoints: bool = False, dynamics_randomization: dict | None = None):
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedQuadEnv needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         if device is None:
@@ -89,6 +94,10 @@ class BatchedQuadEnv:
         self.terminal_obs = torch.zeros((n, d), dtype=torch.float32, device=dev)
         self.ep_return = torch.zeros((n,), dtype=self.real_dtype, device=dev)
         self.ep_len = torch.zeros((n,), dtype=torch.int32, device=dev)
+        self.seed = int(seed)
+        self.dynamics_randomization = None
+        if dynamics_randomization is not None:
+            self.randomize_dynamics(dynamics_randomization)
 
     # -- lifecycle ---------------------------------------------------------------------------------
     def close(self) -> None:
@@ -244,6 +253,60 @@ class BatchedQuadEnv:
         check(self.lib, self._h, self.lib.qs_reset_uniforms(self._h, C.c_void_p(env_ids.data_ptr()), C.c_void_p(episodes.data_ptr()),
                                                            env_ids.numel(), C.c_void_p(out.data_ptr()), self._stream()), "qs_reset_uniforms")
         return out
+
+    # -- dynamics randomisation ------------------------------------------------------------------
+    def randomize_dynamics(self, cfg: dict | None) -> None:
+        """Arm (dict with keys mass, inertia, thrust, wind and optional seed, default the env seed) or disarm (None) dynamics
+        randomisation.  Arming draws every env's parameters for its current episode; every later reset draws its episode's."""
+        if cfg is None:
+            check(self.lib, self._h, self.lib.qs_dynamics_randomization(self._h, None, self._stream()), "qs_dynamics_randomization")
+            self.dynamics_randomization = None
+            return
+        unknown = set(cfg) - {"mass", "inertia", "thrust", "wind", "seed"}
+        if unknown:
+            raise ValueError(f"dynamics_randomization: unknown keys {sorted(unknown)} (mass, inertia, thrust, wind, seed)")
+        r = _cabi.QsDynamicsRand()
+        r.seed = int(cfg.get("seed", self.seed)) & 0xFFFFFFFFFFFFFFFF
+        r.mass_rel, r.inertia_rel = float(cfg.get("mass", 0.0)), float(cfg.get("inertia", 0.0))
+        r.thrust_rel, r.wind = float(cfg.get("thrust", 0.0)), float(cfg.get("wind", 0.0))
+        check(self.lib, self._h, self.lib.qs_dynamics_randomization(self._h, C.byref(r), self._stream()), "qs_dynamics_randomization")
+        self.dynamics_randomization = dict(cfg)
+
+    def _dyn_rows(self) -> torch.Tensor:
+        out = torch.empty((self.n_envs, _cabi.DYN_PARAMS), dtype=torch.float64, device=self.device)
+        check(self.lib, self._h, self.lib.qs_get_dynamics(self._h, C.c_void_p(out.data_ptr()), self._stream()), "qs_get_dynamics")
+        return out
+
+    def dynamics(self) -> dict[str, torch.Tensor]:
+        """The current episode's parameters of every env (float64 device tensors): mass_scale [n], inertia_scale [n],
+        thrust_scale [n,4], wind [n,3] (N, world frame)."""
+        d = self._dyn_rows()
+        return {"mass_scale": d[:, 0].clone(), "inertia_scale": d[:, 1].clone(), "thrust_scale": d[:, 2:6].clone(),
+                "wind": d[:, 6:9].clone()}
+
+    def set_dynamics(self, mass_scale=None, inertia_scale=None, thrust_scale=None, wind=None) -> None:
+        """Overwrite the parameters of every env (fields left None keep their values) until that env's next reset.  Scalars
+        broadcast.  Needs armed randomisation; mass_scale and inertia_scale must be > 0, thrust_scale >= 0, all finite."""
+        d = self._dyn_rows()
+        n = self.n_envs
+        for name, val, cols, shape in (("mass_scale", mass_scale, slice(0, 1), (n,)), ("inertia_scale", inertia_scale, slice(1, 2), (n,)),
+                                       ("thrust_scale", thrust_scale, slice(2, 6), (n, 4)), ("wind", wind, slice(6, 9), (n, 3))):
+            if val is None:
+                continue
+            t = torch.as_tensor(val, dtype=torch.float64, device=self.device)
+            try:
+                t = torch.broadcast_to(t, shape)
+            except RuntimeError:
+                raise ValueError(f"{name}: expected shape {shape} (or broadcastable), got {tuple(t.shape)}") from None
+            if not bool(torch.isfinite(t).all()):
+                raise ValueError(f"{name}: values must be finite")
+            if name in ("mass_scale", "inertia_scale") and not bool((t > 0).all()):
+                raise ValueError(f"{name}: values must be > 0")
+            if name == "thrust_scale" and not bool((t >= 0).all()):
+                raise ValueError(f"{name}: values must be >= 0")
+            d[:, cols] = t.reshape(n, -1)
+        check(self.lib, self._h, self.lib.qs_set_dynamics(self._h, C.c_void_p(d.data_ptr()), self._stream()), "qs_set_dynamics")
+        torch.cuda.current_stream(self.device).synchronize()  # `d` must outlive the kernel
 
     def lsoda_stats(self):
         """(i32[n,4] = nst, nfe, nqu, status ; f64[n,2] = hu, tcur) of the last step in LSODA mode."""

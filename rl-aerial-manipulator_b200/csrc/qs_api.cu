@@ -83,6 +83,32 @@ __global__ void reset_uniforms_kernel(uint64_t seed, const int64_t* env_ids, con
     for (int k = 0; k < QS_N_UNIFORMS; ++k) out[i * QS_N_UNIFORMS + k] = u[k];
 }
 
+// ---- dynamics randomisation planes <-> f64 rows -------------------------------------------------------------
+// arming a reset handle: every env's parameters for the episode it is in
+template <typename Real, int VER>
+__global__ void dyn_arm_kernel(const void* pool, int64_t n, Real* dyn, int64_t stride, DynRand dr, int64_t env_id_offset) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    EnvState<Real, VER> s;
+    pool_load<Real, VER>(pool, n, e, s);
+    Real d[N_DYN];
+    dyn_redraw(dyn, stride, dr, (uint64_t)(env_id_offset + e), s.episode, e, d);
+}
+
+template <typename Real>
+__global__ void dyn_get_kernel(const Real* dyn, int64_t stride, int64_t n, double* out) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    for (int k = 0; k < N_DYN; ++k) out[e * N_DYN + k] = (double)dyn[k * stride + e];
+}
+
+template <typename Real>
+__global__ void dyn_set_kernel(Real* dyn, int64_t stride, int64_t n, const double* in) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    for (int k = 0; k < N_DYN; ++k) dyn[k * stride + e] = (Real)in[e * N_DYN + k];
+}
+
 template <typename Real, int VER>
 static size_t pool_bytes(int64_t n) { return (size_t)PoolLayout<Real, VER>::TILE_BYTES * (size_t)((n + 31) / 32); }   // whole warp tiles
 
@@ -216,6 +242,7 @@ int qs_destroy(qs_handle* h) {
     if (h->ls_tables) cudaFree(h->ls_tables);
     if (h->ls_counters) cudaFree(h->ls_counters);
     if (h->ls_steps) cudaFree(h->ls_steps);
+    if (h->dyn) cudaFree(h->dyn);
     delete h;
     return QS_OK;
 }
@@ -233,8 +260,12 @@ int qs_reset(qs_handle* h, const uint8_t* env_mask, float* obs_out, void* stream
     const unsigned blocks = (unsigned)((n + 255) / 256);
     ResetConsts rc;
     for (int i = 0; i < QS_TRIG_TAB; ++i) { rc.sin_tab[i] = h->cfg.sin_tab[i]; rc.cos_tab[i] = h->cfg.cos_tab[i]; }
-    QS_DISPATCH(h, (env_reset_kernel<Real, VER><<<blocks, 256, 0, st>>>(h->pool, n, env_mask, obs_out, h->cfg.obs_scaled, h->cfg.seed,
-                                                                        h->cfg.env_id_offset, rc, h->initialized ? 0 : 1)););
+    QS_DISPATCH(h, {
+        Real* dyn = static_cast<Real*>(h->dyn);
+        auto k = h->dyn_on ? env_reset_kernel<Real, VER, true> : env_reset_kernel<Real, VER, false>;
+        k<<<blocks, 256, 0, st>>>(h->pool, n, env_mask, obs_out, h->cfg.obs_scaled, h->cfg.seed, h->cfg.env_id_offset, rc,
+                                  h->initialized ? 0 : 1, dyn, h->dyn_stride, h->dyn_cfg);
+    });
     QS_CUDA(h, cudaGetLastError());
     h->initialized = true;
     return QS_OK;
@@ -343,6 +374,62 @@ int qs_reset_uniforms(qs_handle* h, const int64_t* env_ids, const int32_t* episo
     if (n == 0) return QS_OK;
     QS_CUDA(h, cudaSetDevice(h->cfg.device));
     reset_uniforms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(h->cfg.seed, env_ids, episodes, n, out);
+    QS_CUDA(h, cudaGetLastError());
+    return QS_OK;
+}
+
+int qs_dynamics_randomization(qs_handle* h, const qs_dynamics_rand* cfg, void* stream) {
+    if (!h) { set_error(nullptr, "qs_dynamics_randomization: null handle"); return QS_EINVAL; }
+    if (!cfg) { h->dyn_on = false; return QS_OK; }
+    if (h->cfg.integrator != QS_RK4) { set_error(h, "qs_dynamics_randomization: RK4 handles only (no dynamics randomisation in QS_LSODA)"); return QS_EINVAL; }
+    const bool ok = isfinite(cfg->mass_rel) && isfinite(cfg->inertia_rel) && isfinite(cfg->thrust_rel) && isfinite(cfg->wind) &&
+                    cfg->mass_rel >= 0 && cfg->mass_rel < 1 && cfg->inertia_rel >= 0 && cfg->inertia_rel < 1 &&
+                    cfg->thrust_rel >= 0 && cfg->thrust_rel <= 1 && cfg->wind >= 0;
+    if (!ok) {
+        set_error(h, "qs_dynamics_randomization: need finite 0 <= mass_rel < 1, 0 <= inertia_rel < 1, 0 <= thrust_rel <= 1, wind >= 0");
+        return QS_EINVAL;
+    }
+    QS_CUDA(h, cudaSetDevice(h->cfg.device));
+    const int64_t n = h->cfg.n_envs;
+    if (!h->dyn) {
+        h->dyn_stride = (n + 31) / 32 * 32;
+        const size_t real = h->cfg.precision == QS_F32 ? sizeof(float) : sizeof(double);
+        QS_CUDA(h, cudaMalloc(&h->dyn, real * QS_DYN_PARAMS * (size_t)h->dyn_stride));
+    }
+    h->dyn_cfg.seed = cfg->seed;
+    h->dyn_cfg.mass_rel = cfg->mass_rel;
+    h->dyn_cfg.inertia_rel = cfg->inertia_rel;
+    h->dyn_cfg.thrust_rel = cfg->thrust_rel;
+    h->dyn_cfg.wind = cfg->wind;
+    h->dyn_on = true;
+    // every env's parameters for the episode its record holds (0 in the zeroed pool of a handle that was never reset)
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    QS_DISPATCH(h, (dyn_arm_kernel<Real, VER><<<blocks, 128, 0, (cudaStream_t)stream>>>(h->pool, n, static_cast<Real*>(h->dyn), h->dyn_stride,
+                                                                                    h->dyn_cfg, h->cfg.env_id_offset)););
+    QS_CUDA(h, cudaGetLastError());
+    return QS_OK;
+}
+
+int qs_get_dynamics(qs_handle* h, double* out, void* stream) {
+    if (!h || !out) { set_error(h, "qs_get_dynamics: null argument"); return QS_EINVAL; }
+    if (!h->dyn_on) { set_error(h, "qs_get_dynamics: dynamics randomisation is not armed (qs_dynamics_randomization)"); return QS_EINVAL; }
+    QS_CUDA(h, cudaSetDevice(h->cfg.device));
+    const int64_t n = h->cfg.n_envs;
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    if (h->cfg.precision == QS_F32) dyn_get_kernel<float><<<blocks, 128, 0, (cudaStream_t)stream>>>(static_cast<float*>(h->dyn), h->dyn_stride, n, out);
+    else dyn_get_kernel<double><<<blocks, 128, 0, (cudaStream_t)stream>>>(static_cast<double*>(h->dyn), h->dyn_stride, n, out);
+    QS_CUDA(h, cudaGetLastError());
+    return QS_OK;
+}
+
+int qs_set_dynamics(qs_handle* h, const double* in, void* stream) {
+    if (!h || !in) { set_error(h, "qs_set_dynamics: null argument"); return QS_EINVAL; }
+    if (!h->dyn_on) { set_error(h, "qs_set_dynamics: dynamics randomisation is not armed (qs_dynamics_randomization)"); return QS_EINVAL; }
+    QS_CUDA(h, cudaSetDevice(h->cfg.device));
+    const int64_t n = h->cfg.n_envs;
+    const unsigned blocks = (unsigned)((n + 127) / 128);
+    if (h->cfg.precision == QS_F32) dyn_set_kernel<float><<<blocks, 128, 0, (cudaStream_t)stream>>>(static_cast<float*>(h->dyn), h->dyn_stride, n, in);
+    else dyn_set_kernel<double><<<blocks, 128, 0, (cudaStream_t)stream>>>(static_cast<double*>(h->dyn), h->dyn_stride, n, in);
     QS_CUDA(h, cudaGetLastError());
     return QS_OK;
 }

@@ -325,6 +325,37 @@ QS_HD double add_rn(double a, double b) {
 }
 QS_HD double uniform_rn(double lo, double hi, double u) { return add_rn(lo, mul_rn(hi - lo, u)); }
 
+// ------------------------------------------------------------------------------------------------
+// dynamics randomisation: the 9 per-env parameters of an episode, d = (k_m, k_I, eta[4], f_wind[3]) (qs_dynamics_rand).
+// u[0..9]: Philox4x32-10 keyed on r.seed, counter = (env id lo, env id hi, episode, 0x100 + b), b = 0..4 -- word 3 never
+// meets the reset's blocks (j < 9), so the two streams are independent even under one seed.  Round-to-nearest products and
+// sums, in float64: a NumPy restatement reproduces the parameters bit for bit.
+// ------------------------------------------------------------------------------------------------
+struct DynRand {
+    uint64_t seed;
+    double mass_rel, inertia_rel, thrust_rel, wind;
+};
+constexpr int N_DYN = 9;
+
+QS_HD double dyn_sym(double u) { return add_rn(mul_rn(2.0, u), -1.0); }   // 2u - 1 in [-1, 1)
+
+QS_HD void dyn_draw(const DynRand& r, uint64_t env_gid, uint32_t episode, double* d /*[N_DYN]*/) {
+    double u[10];
+#pragma unroll
+    for (uint32_t b = 0; b < 5; ++b) {
+        uint32_t w[4];
+        philox4x32_10((uint32_t)env_gid, (uint32_t)(env_gid >> 32), episode, 0x100u + b, (uint32_t)r.seed, (uint32_t)(r.seed >> 32), w);
+        u[2 * b] = u53(w[0], w[1]);
+        u[2 * b + 1] = u53(w[2], w[3]);
+    }
+    d[0] = add_rn(1.0, mul_rn(r.mass_rel, dyn_sym(u[0])));
+    d[1] = add_rn(1.0, mul_rn(r.inertia_rel, dyn_sym(u[1])));
+#pragma unroll
+    for (int i = 0; i < 4; ++i) d[2 + i] = add_rn(1.0, mul_rn(r.thrust_rel, dyn_sym(u[2 + i])));
+#pragma unroll
+    for (int j = 0; j < 3; ++j) d[6 + j] = mul_rn(r.wind, dyn_sym(u[6 + j]));
+}
+
 template <typename Real, int VER>
 QS_HD void reset_env(EnvState<Real, VER>& s, const ResetConsts& rc, uint64_t seed, uint64_t env_gid) {
     constexpr int NWP = EnvState<Real, VER>::NWP;

@@ -20,6 +20,10 @@ struct qs_handle {
     double* ls_steps;
     unsigned int* ro_ticket;  // qs_rollout_step: last-CTA election counter
     int64_t range_first, range_count;   // qs_step_range: the sub-range the next launch covers (count 0 = all envs)
+    void* dyn;                // dynamics randomisation: Real planes [QS_DYN_PARAMS][dyn_stride]; null = never armed
+    int64_t dyn_stride;       // n_envs rounded up to whole warp tiles
+    bool dyn_on;              // armed (qs_dynamics_randomization)
+    qs::DynRand dyn_cfg;
     int num_sms;
     bool initialized;
     char error[512];
@@ -77,6 +81,9 @@ inline StepParams<Real> base_params(const qs_handle* h) {
     m.tmax = (Real)c.max_prop_thrust;
     m.tmin = (Real)c.min_prop_thrust;
     for (int i = 0; i < QS_TRIG_TAB; ++i) { p.rc.sin_tab[i] = c.sin_tab[i]; p.rc.cos_tab[i] = c.cos_tab[i]; }
+    p.dyn = h->dyn_on ? static_cast<Real*>(h->dyn) + (h->range_count > 0 ? h->range_first : 0) : nullptr;   // planes: offset like the pool
+    p.dyn_stride = h->dyn_stride;
+    p.dr = h->dyn_cfg;
     return p;
 }
 

@@ -55,8 +55,10 @@ template <typename Real> QS_HD Real qs_max(Real a, Real b) { return a > b ? a : 
 //          Rodrigues with cos/sin(theta).  arccos is ill-conditioned near qw = 1, so this form carries
 //          ~1e-13 relative noise; LSODA's step control keys on it near hover, which is why the parity
 //          integrator must reproduce the route and not just the value.
-template <typename Real, bool AXIS_ANGLE = false>
-QS_HD void state_dot(const Model<Real>& m, const Real* y, Real F, const Real* M, Real* dy) {
+//
+// WIND (dynamics randomisation): aw is a constant acceleration added to dy[3..5] (the episode's wind force over the true mass).
+template <typename Real, bool AXIS_ANGLE = false, bool WIND = false>
+QS_HD void state_dot(const Model<Real>& m, const Real* y, Real F, const Real* M, Real* dy, const Real* aw = nullptr) {
     const Real qw = y[6], qx = y[7], qy = y[8], qz = y[9];
     const Real p = y[10], q = y[11], r = y[12];
     const Real n2 = ((qw * qw + qx * qx) + qy * qy) + qz * qz;
@@ -83,6 +85,7 @@ QS_HD void state_dot(const Model<Real>& m, const Real* y, Real F, const Real* M,
         dy[3] = (Real(2) * (qx * qz - qw * qy) * inv_n2) * fm;
         dy[4] = (Real(2) * (qy * qz + qw * qx) * inv_n2) * fm;
         dy[5] = (Real(1) - Real(2) * (qx * qx + qy * qy) * inv_n2) * fm - m.g;
+        if constexpr (WIND) { dy[3] += aw[0]; dy[4] += aw[1]; dy[5] += aw[2]; }
     }
     const Real qerr = Real(2) * (Real(1) - n2);
     dy[6] = Real(-0.5) * (-p * qx - q * qy - r * qz) + qerr * qw;
@@ -102,14 +105,16 @@ QS_HD void state_dot(const Model<Real>& m, const Real* y, Real F, const Real* M,
 }
 
 // Commanded (F, M) -> per-prop thrusts through invA, clamp, re-mix (quadcopter.py:109-112).
-template <typename Real>
-QS_HD void mix_and_clamp(const Model<Real>& m, Real Fcmd, const Real* Mcmd, Real& F, Real* M) {
+// ETA (dynamics randomisation): prop i delivers eta[i] times its clamped thrust.
+template <typename Real, bool ETA = false>
+QS_HD void mix_and_clamp(const Model<Real>& m, Real Fcmd, const Real* Mcmd, Real& F, Real* M, const Real* eta = nullptr) {
     Real t[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         Real v = m.inv_mix[4 * i + 0] * Fcmd + m.inv_mix[4 * i + 1] * Mcmd[0] + m.inv_mix[4 * i + 2] * Mcmd[1] +
                  m.inv_mix[4 * i + 3] * Mcmd[2];
         t[i] = qs_max(qs_min(v, m.tmax), m.tmin);
+        if constexpr (ETA) t[i] = eta[i] * t[i];
     }
     F = ((t[0] + t[1]) + t[2]) + t[3];
 #pragma unroll
@@ -151,25 +156,40 @@ QS_HD void scale_action(const Model<Real>& m, const float* a, int scale_f32, Rea
 // Classical RK4 over one env step split into `substeps` equal sub-intervals (the throughput integrator;
 // the reference uses adaptive LSODA -- see qs_lsoda.cuh for the parity integrator).
 // Storage: y, the stage argument, one derivative and the running sum = 4 x 13 Reals live.
-template <typename Real>
-QS_HD void rk4_step(const Model<Real>& m, Real* y, Real F, const Real* M, int substeps) {
+// WIND: aw[3] is added to the acceleration of every stage (see state_dot).
+template <typename Real, bool WIND = false>
+QS_HD void rk4_step(const Model<Real>& m, Real* y, Real F, const Real* M, int substeps, const Real* aw = nullptr) {
     const Real h = m.dt / (Real)substeps;
     const Real h2 = Real(0.5) * h, h6 = h / Real(6), h3 = h / Real(3);
     for (int s = 0; s < substeps; ++s) {
         Real k[13], yt[13], acc[13];
-        state_dot(m, y, F, M, k);
+        state_dot<Real, false, WIND>(m, y, F, M, k, aw);
 #pragma unroll
         for (int i = 0; i < 13; ++i) { acc[i] = y[i] + h6 * k[i]; yt[i] = y[i] + h2 * k[i]; }
-        state_dot(m, yt, F, M, k);
+        state_dot<Real, false, WIND>(m, yt, F, M, k, aw);
 #pragma unroll
         for (int i = 0; i < 13; ++i) { acc[i] += h3 * k[i]; yt[i] = y[i] + h2 * k[i]; }
-        state_dot(m, yt, F, M, k);
+        state_dot<Real, false, WIND>(m, yt, F, M, k, aw);
 #pragma unroll
         for (int i = 0; i < 13; ++i) { acc[i] += h3 * k[i]; yt[i] = y[i] + h * k[i]; }
-        state_dot(m, yt, F, M, k);
+        state_dot<Real, false, WIND>(m, yt, F, M, k, aw);
 #pragma unroll
         for (int i = 0; i < 13; ++i) y[i] = acc[i] + h6 * k[i];
     }
+}
+
+// Dynamics randomisation, per env: d = (k_m, k_I, eta[4], f_wind[3]).  Prop i delivers eta_i times its clamped thrust; the true
+// mass m*k_m and inertia k_I*I (inverse J/k_I) are folded into the forces, F' = F/k_m and M' = M/k_I, so that state_dot's thrust
+// and rotational terms are the nominal ones: J/k_I*(M - w x k_I*I*w) = J*(M/k_I - w x I*w).  Only the wind acceleration
+// aw = f_wind/(m*k_m) stays live through the RK4 stages.
+template <typename Real>
+QS_HD void dyn_forces(const Model<Real>& m, Real Fcmd, const Real* Mcmd, const Real* d, Real& F, Real* M, Real* aw) {
+    mix_and_clamp<Real, true>(m, Fcmd, Mcmd, F, M, d + 2);
+    const Real ikm = qs_rcp<Real>(d[0]), ikI = qs_rcp<Real>(d[1]);
+    F *= ikm;
+    M[0] *= ikI; M[1] *= ikI; M[2] *= ikI;
+    const Real im = m.inv_mass * ikm;
+    aw[0] = d[6] * im; aw[1] = d[7] * im; aw[2] = d[8] * im;
 }
 
 // The same arithmetic with the four stages as a rolled loop (same operations in the same order: acc = y, acc += w_j k_j,

@@ -1178,6 +1178,7 @@ int qs_rollout_step(qs_handle* h, const qs_rollout_args* a, void* stream) {
     if (!h || !a) { set_error(h, "qs_rollout_step: null argument"); return QS_EINVAL; }
     if (h->cfg.precision != QS_F32 || h->cfg.integrator != QS_RK4) { set_error(h, "qs_rollout_step: float32 / RK4 handles only"); return QS_EINVAL; }
     if (!h->initialized) { set_error(h, "qs_rollout_step: call qs_reset first"); return QS_EINVAL; }
+    if (h->dyn_on) { set_error(h, "qs_rollout_step: the fused rollout kernel has no dynamics randomisation; use qs_policy_forward + qs_step, or disarm qs_dynamics_randomization"); return QS_EINVAL; }
     if (!a->policy_image || !a->obs || !a->obs_next || !a->actions_out || !a->values_out || !a->logp_out || !a->reward_out || !a->flags_out) {
         set_error(h, "qs_rollout_step: policy_image, obs, obs_next, actions_out, values_out, logp_out, reward_out and flags_out are required");
         return QS_EINVAL;

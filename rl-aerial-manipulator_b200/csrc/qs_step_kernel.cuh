@@ -44,7 +44,29 @@ struct StepParams {
     double rtol, atol;
     Model<Real> model;
     ResetConsts rc;
+    Real* dyn;                  // dynamics randomisation: planes [N_DYN][dyn_stride] (k_m, k_I, eta[4], f_wind[3]), or null = off
+    int64_t dyn_stride;
+    DynRand dr;                 // ... and how a reset draws them
+    int64_t pad_;               // 64 bytes appended in all: the fields of ManyParams behind it keep their 16-byte alignment, and the
+                                // nominal qs_step_many kernels their constant loads
 };
+
+// One env's parameters: N_DYN coalesced plane reads; a reset draws the new episode's and stores them.
+template <typename Real>
+QS_HD void dyn_load(const StepParams<Real>& p, int64_t e, Real* d) {
+#pragma unroll
+    for (int k = 0; k < N_DYN; ++k) d[k] = p.dyn[k * p.dyn_stride + e];
+}
+template <typename Real>
+QS_HD void dyn_redraw(Real* planes, int64_t stride, const DynRand& r, uint64_t env_gid, uint32_t episode, int64_t e, Real* d) {
+    double v[N_DYN];
+    dyn_draw(r, env_gid, episode, v);
+#pragma unroll
+    for (int k = 0; k < N_DYN; ++k) {
+        d[k] = (Real)v[k];
+        planes[k * stride + e] = d[k];
+    }
+}
 
 #if defined(__CUDACC__)
 constexpr int STEP_BLOCK = 128;
@@ -91,8 +113,10 @@ __device__ __forceinline__ void warp_store_rows(float* __restrict__ dst, const f
     }
 }
 
-template <typename Real, int VER, int INTEG, bool MOMENTS = false>
+// DYN: dynamics randomisation (RK4 only) -- the env's parameters are read from p.dyn every step and redrawn at an auto-reset.
+template <typename Real, int VER, int INTEG, bool MOMENTS = false, bool DYN = false>
 __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_step_kernel(const StepParams<Real> p) {
+    static_assert(!DYN || INTEG == INTEG_RK4, "dynamics randomisation is RK4 only");
     constexpr int OBS = EnvTraits<VER>::OBS;
     __shared__ float s_tile[STEP_BLOCK / 32][32 * (OBS + 1)];
     __shared__ double s_mom[MOMENTS ? STEP_BLOCK / 32 : 1][2 * OBS];
@@ -133,6 +157,13 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
                 a_nx = __ldcs(reinterpret_cast<const float4*>(p.actions) + en);
             }
         }
+        if constexpr (DYN) {
+            // the next tile's parameter planes are pulled into L2 (no registers held): their loads then wait on L2, not HBM
+            constexpr int LINES = (int)sizeof(Real) * 32 / 128;
+            const int64_t wn = wt + warps_total;
+            if (wn < n_warp_tiles && lane < N_DYN * LINES)
+                asm volatile("prefetch.global.L2 [%0];" ::"l"(p.dyn + (lane / LINES) * p.dyn_stride + wn * 32 + (lane % LINES) * (128 / (int)sizeof(Real))));
+        }
 #ifdef QS_STEP_L2_PREFETCH          // A/B: no register prefetch, but the next tile's record and actions are pulled into L2
         if (!PREFETCH) {
             using L = PoolLayout<Real, VER>;
@@ -154,9 +185,14 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
 
             Real Fcmd, Mcmd[3], F, M[3];
             scale_action<Real>(p.model, act, p.scale_f32, Fcmd, Mcmd);
-            mix_and_clamp<Real>(p.model, Fcmd, Mcmd, F, M);
             uint32_t flags = 0;
-            if constexpr (INTEG == INTEG_LSODA) {
+            if constexpr (DYN) {
+                Real d[N_DYN], aw[3];
+                dyn_load(p, e, d);
+                dyn_forces<Real>(p.model, Fcmd, Mcmd, d, F, M, aw);
+                rk4_step<Real, true>(p.model, s.y, F, M, p.substeps, aw);
+            } else if constexpr (INTEG == INTEG_LSODA) {
+                mix_and_clamp<Real>(p.model, Fcmd, Mcmd, F, M);
                 LsodaResult r;
                 lsoda_advance(p.model, *p.ls_tables, s.y, F, M, p.model.dt, p.rtol, p.atol, r);
                 if (r.status & ~LS_WOULD_SWITCH) flags |= FLAG_LSODA_FAIL;
@@ -165,6 +201,7 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
                     reinterpret_cast<double2*>(p.ls_steps)[e] = make_double2(r.hu, r.tcur);
                 }
             } else {
+                mix_and_clamp<Real>(p.model, Fcmd, Mcmd, F, M);
                 rk4_step<Real>(p.model, s.y, F, M, p.substeps);
             }
             renormalise_quat<Real>(s.y);
@@ -189,6 +226,10 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
                     s.episode += 1;
                     reset_env<Real, VER>(s, p.rc, p.seed, (uint64_t)(p.env_id_offset + e));
                     make_obs<Real, VER>(s, p.obs_scaled, obs);
+                    if constexpr (DYN) {
+                        Real d[N_DYN];
+                        dyn_redraw(p.dyn, p.dyn_stride, p.dr, (uint64_t)(p.env_id_offset + e), s.episode, e, d);
+                    }
                 }
             }
             pool_store<Real, VER>(p.pool, p.n, e, s);
@@ -416,11 +457,11 @@ __global__ void __launch_bounds__(STEP_BLOCK, 4) env_step_tma_kernel(const StepP
     }
 }
 
-// Reset (all envs or a mask) and write their observation.
-template <typename Real, int VER>
+// Reset (all envs or a mask) and write their observation; DYN: also draw the new episode's dynamics parameters into `dyn`.
+template <typename Real, int VER, bool DYN = false>
 __global__ void __launch_bounds__(256) env_reset_kernel(void* pool, int64_t n, const uint8_t* mask, float* obs_out,
                                                          int obs_scaled, uint64_t seed, int64_t env_id_offset,
-                                                         ResetConsts rc, int first) {
+                                                         ResetConsts rc, int first, Real* dyn, int64_t dyn_stride, DynRand dr) {
     constexpr int OBS = EnvTraits<VER>::OBS;
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
@@ -434,6 +475,10 @@ __global__ void __launch_bounds__(256) env_reset_kernel(void* pool, int64_t n, c
     }
     reset_env<Real, VER>(s, rc, seed, (uint64_t)(env_id_offset + e));
     pool_store<Real, VER>(pool, n, e, s);
+    if constexpr (DYN) {
+        Real d[N_DYN];
+        dyn_redraw(dyn, dyn_stride, dr, (uint64_t)(env_id_offset + e), s.episode, e, d);
+    }
     if (obs_out) {
         float obs[OBS];
         make_obs<Real, VER>(s, obs_scaled, obs);

@@ -60,7 +60,9 @@ __device__ __forceinline__ float4 philox_uniform_action(uint64_t seed, uint64_t 
 template <typename Real> struct ManyOcc { static constexpr int MINB = 3; };
 template <> struct ManyOcc<float> { static constexpr int MINB = 4; };
 
-template <typename Real, int VER>
+// DYN: dynamics randomisation -- an env's parameters are read once per launch, stay in registers across the T steps, and are
+// redrawn (and written back) only where an auto-reset starts a new episode.
+template <typename Real, int VER, bool DYN = false>
 __global__ void __launch_bounds__(STEP_BLOCK, ManyOcc<Real>::MINB) env_step_many_kernel(const ManyParams<Real> p) {
     constexpr int OBS = EnvTraits<VER>::OBS;
     __shared__ float s_tile[STEP_BLOCK / 32][32 * (OBS + 1)];
@@ -79,6 +81,10 @@ __global__ void __launch_bounds__(STEP_BLOCK, ManyOcc<Real>::MINB) env_step_many
         const int rows = rem < 32 ? (int)rem : 32;
         EnvState<Real, VER> s;
         if (live) pool_load<Real, VER>(sp.pool, sp.n, e, s);
+        Real d[DYN ? N_DYN : 1];
+        if constexpr (DYN) {
+            if (live) dyn_load(sp, e, d);
+        }
         float4 a_next = make_float4(0.f, 0.f, 0.f, 0.f);
         if (live && p.actions) a_next = __ldcs(reinterpret_cast<const float4*>(p.actions) + e);
 #pragma unroll 1
@@ -97,8 +103,14 @@ __global__ void __launch_bounds__(STEP_BLOCK, ManyOcc<Real>::MINB) env_step_many
                 const float act[4] = {a4.x, a4.y, a4.z, a4.w};
                 Real Fcmd, Mcmd[3], F, M[3];
                 scale_action<Real>(sp.model, act, sp.scale_f32, Fcmd, Mcmd);
-                mix_and_clamp<Real>(sp.model, Fcmd, Mcmd, F, M);
-                rk4_step<Real>(sp.model, s.y, F, M, sp.substeps);
+                if constexpr (DYN) {
+                    Real aw[3];
+                    dyn_forces<Real>(sp.model, Fcmd, Mcmd, d, F, M, aw);
+                    rk4_step<Real, true>(sp.model, s.y, F, M, sp.substeps, aw);
+                } else {
+                    mix_and_clamp<Real>(sp.model, Fcmd, Mcmd, F, M);
+                    rk4_step<Real>(sp.model, s.y, F, M, sp.substeps);
+                }
                 renormalise_quat<Real>(s.y);
                 Real reward;
                 int ep_len;
@@ -119,6 +131,7 @@ __global__ void __launch_bounds__(STEP_BLOCK, ManyOcc<Real>::MINB) env_step_many
                         s.episode += 1;
                         reset_env<Real, VER>(s, sp.rc, sp.seed, (uint64_t)(sp.env_id_offset + e));
                         make_obs<Real, VER>(s, sp.obs_scaled, obs);
+                        if constexpr (DYN) dyn_redraw(sp.dyn, sp.dyn_stride, sp.dr, (uint64_t)(sp.env_id_offset + e), s.episode, e, d);
                     }
                 }
             }
@@ -170,7 +183,7 @@ static int launch_many(qs_handle* h, const qs_step_many_args* a, cudaStream_t st
     p.ticket = h->ro_ticket;
     cudaError_t err = cudaSuccess;
     QS_FOR_VARIANT(h, {
-        auto k = env_step_many_kernel<Real, VER>;
+        auto k = p.sp.dyn ? env_step_many_kernel<Real, VER, true> : env_step_many_kernel<Real, VER, false>;
         const unsigned grid = step_grid(h, k, STEP_BLOCK);
         k<<<grid, STEP_BLOCK, 0, st>>>(p);
     });

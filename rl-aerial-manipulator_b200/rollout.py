@@ -31,6 +31,9 @@ class FusedRollout:
                  store_obs_norm: bool = False, norm_eps: float = 1e-8, norm_clip: float = 10.0):
         if env.precision != "f32" or env.integrator != "rk4":
             raise ValueError("FusedRollout needs a float32 / RK4 env")
+        if getattr(env, "dynamics_randomization", None) is not None:
+            raise ValueError("FusedRollout: the fused rollout kernel has no dynamics randomisation; step the env with a policy "
+                             "forward + env.step (QuadPPO does), or disarm it")
         self.env, self.policy, self.vecnorm = env, policy, vecnorm
         self.lib = env.lib
         self.mode = {"mean": _cabi.SAMPLE_MEAN, "noise": _cabi.SAMPLE_NOISE, "philox": _cabi.SAMPLE_PHILOX}[sample]

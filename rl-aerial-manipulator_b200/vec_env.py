@@ -114,13 +114,14 @@ class QuadVecEnv(_SB3VecEnv):
     def __init__(self, num_envs: int = 8, env_version: int = 2, precision: str = "f32", integrator: str = "rk4",
                  substeps: int = 1, obs_scaled: bool = True, device: int | None = None, seed: int = 0,
                  env_id_offset: int = 0, monitor: bool = True, info_mode: str = "dict", v2_random_waypoints: bool = False,
-                 pipeline_chunks: int | None = None):
+                 pipeline_chunks: int | None = None, dynamics_randomization: dict | None = None):
         """pipeline_chunks: split a step into this many env sub-ranges, each on its own stream -- actions of chunk c+1 are copied
         up while chunk c steps and its observations come down, so the PCIe link works in both directions at once.
-        None: 4 from 262,144 envs, else 1."""
+        None: 4 from 262,144 envs, else 1.  dynamics_randomization: see BatchedQuadEnv."""
         self.sim = BatchedQuadEnv(num_envs, env_version=env_version, precision=precision, integrator=integrator,
                                   substeps=substeps, obs_scaled=obs_scaled, auto_reset=True, device=device,
-                                  env_id_offset=env_id_offset, seed=seed, v2_random_waypoints=v2_random_waypoints)
+                                  env_id_offset=env_id_offset, seed=seed, v2_random_waypoints=v2_random_waypoints,
+                                  dynamics_randomization=dynamics_randomization)
         d = self.sim.obs_dim
         observation_space = _box(-np.inf, np.inf, (d,), np.float32)      # rl_env_scaledObs.py:14-17
         action_space = _box(np.array([0, -1, -1, -1], dtype=np.float32), np.array([2.0, 1, 1, 1], dtype=np.float32))  # :20-24
