@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY -- restatement of Stable-Baselines3's PPO minibatch update (SB3 2.6.0 `PPO.train`, as the reference
 calls it: initial-implementation-v1/rl_train_vecN.py:13-36, initial-implementation-v2/rl_train.py:27-56), twice:
 
-  * NumPy float64, forward AND hand-derived backward (`minibatch_grads`, `clip_grad_norm`, `adam_step`, `update`): the
-    checker of the CUDA update kernel (csrc/qs_ppo.cu);
+  * NumPy float64, forward AND hand-derived backward (`minibatch_grads`, `clip_grad_norm`, `adam_step`, `update`; `train_pass`
+    for a whole PPO.train): the checker of the CUDA update kernel (csrc/qs_ppo.cu);
   * torch autograd (`TorchActorCritic`, `ppo_loss`, `torch_update`): the same update the way SB3 itself computes it
     (nn.Linear / Tanh modules, autograd, clip_grad_norm_, torch.optim.Adam(eps=1e-5)); pins the NumPy backward
     (tests/test_ppo.py) and is the second checker of the kernel.
@@ -44,7 +44,8 @@ def _mlp_backward(sd, net, acts, d_out, grads):
 def minibatch_grads(sd, obs, actions, old_logp, advantages, returns, clip_range=0.2, ent_coef=0.0, vf_coef=0.5,
                     normalize_advantage=True):
     """One minibatch of PPO.train (clip_range_vf=None): returns (stats, grads) with stats = loss, policy_gradient_loss,
-    value_loss, entropy_loss and grads keyed like the SB3 state dict."""
+    value_loss, entropy_loss, clip_fraction, approx_kl and grads keyed like the SB3 state dict.  clip_fraction and approx_kl
+    are SB3's diagnostics: mean(|ratio - 1| > clip_range) and mean((ratio - 1) - log_ratio)."""
     sd = {k: np.asarray(v, np.float64) for k, v in sd.items()}
     obs, actions = np.asarray(obs, np.float64), np.asarray(actions, np.float64)
     old_logp, adv, ret = (np.asarray(a, np.float64) for a in (old_logp, advantages, returns))
@@ -58,7 +59,8 @@ def minibatch_grads(sd, obs, actions, old_logp, advantages, returns, clip_range=
     z = (actions - mean) / np.exp(log_std)
     logp = (-0.5 * z ** 2 - log_std - 0.5 * LOG_2PI).sum(1)
     entropy = (0.5 + 0.5 * LOG_2PI + log_std).sum()
-    ratio = np.exp(logp - old_logp)
+    log_ratio = logp - old_logp
+    ratio = np.exp(log_ratio)
     s1, s2 = adv * ratio, adv * np.clip(ratio, 1 - clip_range, 1 + clip_range)
     pg = -np.minimum(s1, s2).mean()
     vf = ((returns - values) ** 2).mean()
@@ -79,7 +81,9 @@ def minibatch_grads(sd, obs, actions, old_logp, advantages, returns, clip_range=
     grads["value_net.weight"] = d_val.T @ va[3]
     grads["value_net.bias"] = d_val.sum(0)
     _mlp_backward(sd, "value_net", va, d_val @ sd["value_net.weight"], grads)
-    return {"loss": loss, "policy_gradient_loss": pg, "value_loss": vf, "entropy_loss": ent}, grads
+    stats = {"loss": loss, "policy_gradient_loss": pg, "value_loss": vf, "entropy_loss": ent,
+             "clip_fraction": float(np.mean(np.abs(ratio - 1.0) > clip_range)), "approx_kl": float(np.mean((ratio - 1.0) - log_ratio))}
+    return stats, grads
 
 
 def clip_grad_norm(grads, max_norm):
@@ -110,13 +114,35 @@ def adam_step(sd, grads, state, lr, betas=(0.9, 0.999), eps=1e-5):
         sd[k] = sd[k] - (lr / bc1) * m / (np.sqrt(v) / math.sqrt(bc2) + eps)
 
 
-def update(sd, state, batch, lr=2e-4, clip_range=0.2, ent_coef=0.0, vf_coef=0.5, max_grad_norm=0.5, normalize_advantage=True):
-    """One full minibatch update in float64; sd (float64 dict) and state are modified in place.  Returns the loss statistics."""
+def update(sd, state, batch, lr=2e-4, clip_range=0.2, ent_coef=0.0, vf_coef=0.5, max_grad_norm=0.5, normalize_advantage=True,
+           betas=(0.9, 0.999), eps=1e-5):
+    """One full minibatch update in float64; sd (float64 dict) and state are modified in place.  Returns the loss statistics
+    with the pre-clip gradient norm and the minibatch size."""
     stats, grads = minibatch_grads(sd, *batch, clip_range=clip_range, ent_coef=ent_coef, vf_coef=vf_coef,
                                    normalize_advantage=normalize_advantage)
     stats["grad_norm"] = clip_grad_norm(grads, max_grad_norm)
-    adam_step(sd, grads, state, lr)
+    stats["batch_size"] = len(batch[0])
+    adam_step(sd, grads, state, lr, betas=betas, eps=eps)
     return stats
+
+
+def minibatches(perm, batch_size):
+    """RolloutBuffer.get(batch_size): consecutive slices of one epoch's permutation, the ragged last one kept."""
+    total = len(perm)
+    bs = min(batch_size, total)
+    return [perm[start:start + bs] for start in range(0, total, bs)]
+
+
+def train_pass(sd, state, buffers, perms, batch_size, **hp):
+    """PPO.train in float64: one epoch per permutation in `perms`, each cut into minibatches by `minibatches`, one `update`
+    per minibatch with one Adam state threaded through all of them.  `buffers` = (obs, actions, old_logp, advantages,
+    returns), flattened to rows.  sd and state are modified in place; returns every minibatch's statistics in order."""
+    buffers = tuple(np.asarray(b, np.float64) for b in buffers)
+    out = []
+    for perm in perms:
+        for idx in minibatches(np.asarray(perm), batch_size):
+            out.append(update(sd, state, tuple(b[idx] for b in buffers), **hp))
+    return out
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -165,14 +191,21 @@ def ppo_loss(values, logp, entropy, old_logp, advantages, returns, clip_range: f
 
 
 def torch_update(net, opt, batch, clip_range=0.2, ent_coef=0.0, vf_coef=0.5, max_grad_norm=0.5, normalize_advantage=True):
-    """One minibatch update with autograd + clip_grad_norm_ + opt.step(); returns (loss, pg, vf, ent, grad_norm) as floats."""
+    """One minibatch update with autograd + clip_grad_norm_ + opt.step(); returns (loss, pg, vf, ent, grad_norm, clip_fraction,
+    approx_kl) as floats, the last two computed as SB3 2.6.0's PPO.train does."""
+    import torch
     import torch.nn as nn
 
     obs, act, oldlp, adv, ret = batch
     values, logp, entropy = net.evaluate_actions(obs, act)
     loss, pg, vf, ent = ppo_loss(values, logp, entropy, oldlp, adv, ret, clip_range, ent_coef, vf_coef, normalize_advantage)
+    with torch.no_grad():
+        log_ratio = logp - oldlp
+        ratio = torch.exp(log_ratio)
+        clip_fraction = torch.mean((torch.abs(ratio - 1) > clip_range).float())
+        approx_kl = torch.mean((ratio - 1) - log_ratio)
     opt.zero_grad(set_to_none=False)
     loss.backward()
     gn = nn.utils.clip_grad_norm_(net.parameters(), max_grad_norm)
     opt.step()
-    return tuple(float(x.detach()) for x in (loss, pg, vf, ent, gn))
+    return tuple(float(x.detach()) for x in (loss, pg, vf, ent, gn, clip_fraction, approx_kl))

@@ -64,6 +64,95 @@ def test_numpy_ppo_update_matches_torch_autograd():
         assert err < 1e-12, err
 
 
+def f64_state_dict(D, seed):
+    return {k: v.astype(np.float64) for k, v in perturbed_state_dict(D, seed).items()}
+
+
+@pytest.mark.parametrize("normalize_advantage", [True, False])
+@pytest.mark.parametrize("case", ["random", "one_row", "constant_advantage"])
+def test_numpy_minibatch_stats_and_grads_match_torch_autograd(case, normalize_advantage):
+    """minibatch_grads against torch autograd in float64 for both advantage settings, including SB3's two diagnostics
+    (clip_fraction, approx_kl) and the edges of the normalisation: a one-row minibatch (SB3 skips the normalisation, since
+    torch.std of one element is NaN) and constant advantages (std 0: (A - mean) / (0 + 1e-8) = 0)."""
+    from oracle import ppo_oracle as po
+    D, B = 20, {"random": 37, "one_row": 1, "constant_advantage": 64}[case]
+    rng = np.random.default_rng(B)
+    sd = f64_state_dict(D, 4)
+    batch = [np.asarray(x, np.float64) for x in random_minibatch(rng, B, D, sd)]
+    if case == "constant_advantage":
+        batch[3][:] = np.float32(1.7)             # a float32 buffer value: its mean is exact in float64, so A - mean = 0 exactly
+    hp = dict(clip_range=0.15, ent_coef=0.01, vf_coef=0.7, normalize_advantage=normalize_advantage)
+    stats, grads = po.minibatch_grads(sd, *batch, **hp)
+    net = po.make_torch_actor_critic(sd, D, torch.float64)
+    opt = torch.optim.SGD(net.parameters(), lr=0.0)
+    t = po.torch_update(net, opt, tuple(torch.from_numpy(x) for x in batch), max_grad_norm=1e30, **hp)   # coef 1: unclipped
+    for i, k in enumerate(("loss", "policy_gradient_loss", "value_loss", "entropy_loss")):
+        assert math.isfinite(stats[k]) and abs(stats[k] - t[i]) <= 1e-12 * max(1.0, abs(t[i])), (k, stats[k], t[i])
+    assert abs(stats["clip_fraction"] - t[5]) < 1e-7                    # SB3 takes the mean of a float32 mask
+    assert abs(stats["approx_kl"] - t[6]) <= 1e-12 * max(1.0, abs(t[6]))
+    for name, p in net.named_parameters():
+        np.testing.assert_allclose(grads[name], p.grad.numpy(), rtol=1e-10, atol=1e-13, err_msg=name)
+    if case == "random":
+        assert 0.0 < stats["clip_fraction"] < 1.0 and stats["approx_kl"] > 0.0        # both sides of the clip range populated
+    if case == "constant_advantage" and normalize_advantage:
+        assert stats["policy_gradient_loss"] == 0.0 and not grads["action_net.weight"].any()
+
+
+def test_numpy_update_passes_betas_and_eps_to_adam():
+    """update(betas=, eps=) reaches adam_step: six updates against torch.optim.Adam with the same non-default betas / eps / lr
+    and a clipping max_grad_norm, float64, parameters and both moments equal to rounding."""
+    from oracle import ppo_oracle as po
+    D, B = 17, 50
+    rng = np.random.default_rng(6)
+    sd = f64_state_dict(D, 8)
+    hp = dict(clip_range=0.2, ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.3)
+    net = po.make_torch_actor_critic(sd, D, torch.float64)
+    opt = torch.optim.Adam(net.parameters(), lr=1e-3, betas=(0.8, 0.95), eps=1e-7)
+    st = po.adam_init(sd)
+    for it in range(6):
+        batch = tuple(np.asarray(x, np.float64) for x in random_minibatch(rng, B, D, sd))
+        s = po.update(sd, st, batch, lr=1e-3, betas=(0.8, 0.95), eps=1e-7, **hp)
+        t = po.torch_update(net, opt, tuple(torch.from_numpy(x) for x in batch), **hp)
+        assert abs(s["grad_norm"] - t[4]) < 1e-10 * t[4] and t[4] > hp["max_grad_norm"] and s["batch_size"] == B
+    for name, p in net.named_parameters():
+        np.testing.assert_allclose(sd[name], p.detach().numpy(), rtol=0, atol=1e-12, err_msg=name)
+        np.testing.assert_allclose(st["m"][name], opt.state[p]["exp_avg"].numpy(), rtol=1e-9, atol=1e-15, err_msg=name)
+        np.testing.assert_allclose(st["v"][name], opt.state[p]["exp_avg_sq"].numpy(), rtol=1e-9, atol=1e-18, err_msg=name)
+    assert st["step"] == 6 == int(opt.state[next(net.parameters())]["step"])
+
+
+@pytest.mark.parametrize("batch_size", [32, 23, 100])
+def test_numpy_train_pass_matches_torch_training_loop(batch_size):
+    """train_pass (PPO.train restated: n_epochs over given permutations, minibatches cut as RolloutBuffer.get cuts them) against
+    the same loop over torch_update in float64.  70 rows: batch 32 leaves a ragged 6-row minibatch, 23 a one-row one, 100 (larger
+    than the buffer) one minibatch of all rows per epoch."""
+    from oracle import ppo_oracle as po
+    D, total, n_epochs = 20, 70, 3
+    rng = np.random.default_rng(batch_size)
+    sd = f64_state_dict(D, 9)
+    buffers = tuple(np.asarray(x, np.float64) for x in random_minibatch(rng, total, D, sd))
+    perms = [rng.permutation(total) for _ in range(n_epochs)]
+    hp = dict(lr=3e-4, clip_range=0.2, ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5)
+    net = po.make_torch_actor_critic(sd, D, torch.float64)
+    opt = torch.optim.Adam(net.parameters(), lr=hp["lr"], eps=1e-5)
+    st = po.adam_init(sd)
+    stats = po.train_pass(sd, st, buffers, perms, batch_size, **hp)
+    sizes = [len(i) for i in po.minibatches(perms[0], batch_size)]
+    assert sum(sizes) == total and sizes[:-1] == [min(batch_size, total)] * (len(sizes) - 1)
+    assert len(stats) == n_epochs * len(sizes) == st["step"] and [s["batch_size"] for s in stats[-len(sizes):]] == sizes
+    tb = tuple(torch.from_numpy(x) for x in buffers)
+    k = 0
+    for perm in perms:
+        for idx in po.minibatches(perm, batch_size):
+            t = po.torch_update(net, opt, tuple(x[torch.from_numpy(idx)] for x in tb), **{k_: v for k_, v in hp.items() if k_ != "lr"})
+            for i, key in enumerate(("loss", "policy_gradient_loss", "value_loss", "entropy_loss", "grad_norm", "clip_fraction", "approx_kl")):
+                tol = 1e-7 if key == "clip_fraction" else 1e-10 * max(1.0, abs(t[i]))      # SB3: mean of a float32 mask
+                assert abs(stats[k][key] - t[i]) <= tol, (k, key, stats[k][key], t[i])
+            k += 1
+    for name, p in net.named_parameters():
+        np.testing.assert_allclose(sd[name], p.detach().numpy(), rtol=0, atol=1e-12, err_msg=name)
+
+
 def test_init_and_packing_roundtrip():
     from rl_aerial_manipulator_b200.policy import pack_params, unpack_params
     from rl_aerial_manipulator_b200.ppo import init_state_dict
@@ -95,6 +184,46 @@ def test_gae_kernel_vs_sb3_restatement():
                              dones, 0.995, 0.9)
         np.testing.assert_allclose(adv.cpu().numpy(), a_np, rtol=1e-4, atol=1e-3)
         np.testing.assert_allclose(ret.cpu().numpy(), r_np, rtol=1e-4, atol=1e-3)
+
+
+# T, n, gamma, lambda, P(episode start), P(last done)
+GAE_EDGES = {
+    "reference_shape": (2048, 8, 0.995, 0.9, 0.01, 0.1),          # v1/rl_train_vecN.py: 8 envs x n_steps 2048
+    "undiscounted": (2048, 8, 1.0, 1.0, 0.002, 0.0),                # gamma = lambda = 1: advantages sum rewards over whole episodes
+    "every_step_a_start": (64, 1000, 0.995, 0.9, 1.0, 0.1),
+    "all_last_dones": (64, 1000, 0.995, 0.9, 0.05, 1.0),
+    "one_env": (300, 1, 0.995, 0.9, 0.01, 1.0),
+    "ragged_block": (50, 257, 0.995, 0.9, 0.1, 0.5),               # 256-thread blocks: one env in a second block
+}
+# the kernel is SB3's float32 recurrence: each of the T steps adds a few roundings of its operands, which accumulate like a
+# random walk.  Bound: sqrt(T) * 2^-24 * (max|rewards| + max|values| + max|advantages|); worst measured on an NVIDIA B200 (1000 W
+# power limit): 0.18 of it (gamma = lambda = 1, T = 2048).
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("case", list(GAE_EDGES))
+def test_gae_kernel_edges_vs_sb3_restatement(case):
+    """qs_gae at the reference's own shape, gamma = lambda = 1, episode starts at every step, every env done at the end, one env
+    and a ragged last block, against the float64 restatement within a bound that grows with sqrt(T)."""
+    from rl_aerial_manipulator_b200.ppo import gae
+    T, n, gamma, lam, p_start, p_done = GAE_EDGES[case]
+    rng = np.random.default_rng(T + n)
+    rewards = (rng.normal(size=(T, n)) * 10).astype(np.float32)
+    values = (rng.normal(size=(T, n)) * 50).astype(np.float32)
+    starts = (rng.random((T, n)) < p_start).astype(np.uint8)
+    last_values = (rng.normal(size=n) * 50).astype(np.float32)
+    dones = (rng.random(n) < p_done).astype(np.uint8)
+    c = lambda a: torch.from_numpy(a).cuda()
+    adv, ret = gae(c(rewards), c(values), c(starts), c(last_values), c(dones), gamma, lam)
+    a_np, r_np = sb3_gae(rewards.astype(np.float64), values.astype(np.float64), starts.astype(np.float64), last_values.astype(np.float64),
+                         dones, gamma, lam)
+    if p_start == 1.0:                       # every next step is a new episode: delta without bootstrap, no carried advantage
+        np.testing.assert_allclose(a_np[:-1], rewards[:-1].astype(np.float64) - values[:-1], rtol=0, atol=1e-12)
+    scale = np.abs(rewards).max() + np.abs(values).max() + np.abs(a_np).max()
+    bound = np.sqrt(T) * 2.0 ** -24 * scale
+    err_a, err_r = np.abs(adv.cpu().numpy() - a_np).max(), np.abs(ret.cpu().numpy() - r_np).max()
+    print(f"measured gae {case}: {err_a / bound:.4f} {err_r / bound:.4f} of the bound {bound:.3g}")
+    assert err_a <= bound and err_r <= bound, (err_a, err_r, bound)
 
 
 PPO_HP = dict(clip_range=0.2, ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5)
