@@ -207,7 +207,7 @@ int qs_reset_uniforms(qs_handle* h, const int64_t* env_ids, const int32_t* episo
  *   k_m = 1 + mass_rel*(2u0-1),  k_I = 1 + inertia_rel*(2u1-1),  eta_i = 1 + thrust_rel*(2u_{2+i}-1),  f_wind_j = wind*(2u_{6+j}-1)
  * in float64 with round-to-nearest products and sums (stored rounded to float on a QS_F32 handle).
  * Valid: 0 <= mass_rel < 1, 0 <= inertia_rel < 1, 0 <= thrust_rel <= 1 (eta = 0 is a dead motor), wind >= 0, all finite.
- * RK4 handles only; while armed, qs_rollout_step and the QS_STEP_F32_TMA opt-in kernel refuse (QS_EINVAL).
+ * RK4 handles only; while armed, qs_rollout_step refuses (QS_EINVAL).
  * qs_dynamics_randomization: cfg NULL disarms.  May be called before or after the first qs_reset; on a reset handle it draws every
  *   env's parameters for its current episode.
  * qs_get_dynamics / qs_set_dynamics: f64[n, QS_DYN_PARAMS] device rows (k_m, k_I, eta[4], f_wind[3]); set values hold until that
@@ -262,21 +262,19 @@ const char* qs_vecnorm_last_error(void);
  *   actions    f32[n,4] unclipped (what SB3 stores)    actions_clipped f32[n,4] or NULL (clip_lo/clip_hi f32[4], host)
  *   values f32[n]    logp f32[n]
  *   impl       QS_POLICY_FP32: CUDA-core FFMA kernel, float32 throughout;
- *              QS_POLICY_TENSOR: tcgen05/TMEM kernel, split-float16 operands (hi+lo, 3 MMAs per k-step) + float32
- *                                accumulation: float32-level accuracy (values within 2e-3 of float64 on |V| <= 2800);
- *              QS_POLICY_TENSOR_FAST: tcgen05/TMEM kernel, single float16 operands + MUFU.TANH (means within 3e-2,
+ *              QS_POLICY_TENSOR: tcgen05/TMEM kernel (the warp-specialised pipeline of qs_rollout_step, policy part only),
+ *                                split-float16 operands (hi+lo, 3 MMAs per k-step) + float32 accumulation: float32-level
+ *                                accuracy (values within 2e-3 of float64 on |V| <= 2800);
+ *              QS_POLICY_TENSOR_FAST: tcgen05/TMEM three-chain kernel, single float16 operands + MUFU.TANH (means within 3e-2,
  *                                values within ~1e-2 |V|max);
+ *              QS_POLICY_TENSOR_PIPELINE: the same as QS_POLICY_TENSOR;
  *              QS_POLICY_AUTO: TENSOR for n >= 16384, FP32 below
  */
 #define QS_POLICY_AUTO 0
 #define QS_POLICY_FP32 1
 #define QS_POLICY_TENSOR 2
 #define QS_POLICY_TENSOR_FAST 3
-#define QS_POLICY_TENSOR_PIPELINE 4 /* QS_POLICY_TENSOR arithmetic on the warp-specialised pipeline of qs_rollout_step (policy part only) */
-#define QS_POLICY_TENSOR_CHAINS 5   /* QS_POLICY_TENSOR arithmetic on the three-chain kernel (qs_policy_tc.cu) */
-#ifndef QS_POLICY_TENSOR_DEFAULT_PIPELINE
-#define QS_POLICY_TENSOR_DEFAULT_PIPELINE 1 /* which of the two QS_POLICY_TENSOR / AUTO run (r02: pipeline 296 us, chains 308 us per 1M envs) */
-#endif
+#define QS_POLICY_TENSOR_PIPELINE 4
 int64_t qs_policy_param_count(int obs_dim);
 int qs_policy_forward(const float* params, int obs_dim, const float* obs, const float* noise, int64_t n,
                       const double* norm_stats, float norm_eps, float norm_clip, float* obs_norm_out,

@@ -17,8 +17,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_obj")
 LIBDIR = os.path.join(HERE, "lib")
-# QS_NVCC_DEFINES="-DX=1 ..." + QS_LIB_TAG=foo build an experimental variant lib/libquadsim_foo.so (A/B runs on the GPU box;
-# load it with QS_LIB_PATH).  The product build uses neither.
+# QS_NVCC_DEFINES="-DQS_RO_TRACE=1 ..." + QS_LIB_TAG=foo build a trace variant lib/libquadsim_foo.so (the clock64 phase traces of
+# tools/rollout_trace.py and tools/policy_trace3.py; load it with QS_LIB_PATH).  The product build uses neither.
 TAG = os.environ.get("QS_LIB_TAG", "")
 DEFINES = os.environ.get("QS_NVCC_DEFINES", "").split()
 OBJ = OBJ + ("_" + TAG if TAG else "")

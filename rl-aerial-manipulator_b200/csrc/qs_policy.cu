@@ -226,11 +226,11 @@ static size_t policy_smem_bytes(int obs) {
 
 thread_local char g_policy_error[256] = "";
 
-// tensor-core path (qs_policy_tc.cu): precise = split-float16 (float32 accuracy), else single float16
-int launch_policy_tc(int precise, const float* params, int obs_dim, const float* obs, const float* noise, int64_t n,
-                     const double* norm_stats, float norm_eps, float norm_clip, float* obs_norm_out, float* actions,
-                     float* actions_clipped, const float* clip_lo, const float* clip_hi, float* values, float* logp,
-                     cudaStream_t stream, const char** err_out);
+// tensor-core paths: single float16 (qs_policy_tc.cu), split-float16 with float32 accuracy (qs_rollout_policy.cu)
+int launch_policy_tc(const float* params, int obs_dim, const float* obs, const float* noise, int64_t n, const double* norm_stats,
+                     float norm_eps, float norm_clip, float* obs_norm_out, float* actions, float* actions_clipped,
+                     const float* clip_lo, const float* clip_hi, float* values, float* logp, cudaStream_t stream,
+                     const char** err_out);
 int launch_policy_pipeline(const float* params, int obs_dim, const float* obs, const float* noise, int64_t n, const double* norm_stats,
                            float norm_eps, float norm_clip, float* obs_norm_out, float* actions, float* actions_clipped,
                            const float* clip_lo, const float* clip_hi, float* values, float* logp, cudaStream_t stream,
@@ -260,7 +260,7 @@ int qs_policy_forward(const float* params, int obs_dim, const float* obs, const 
         snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward: obs, noise, actions, actions_clipped and obs_norm_out must be 16-byte aligned");
         return QS_EINVAL;
     }
-    if (impl < 0 || impl > 5) {
+    if (impl < 0 || impl > 4) {
         snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward: impl must be one of QS_POLICY_*");
         return QS_EINVAL;
     }
@@ -268,17 +268,13 @@ int qs_policy_forward(const float* params, int obs_dim, const float* obs, const 
     // to fill the SMs (profiles/r01/policy_paths.md); below that the FFMA kernel's finer 64-env tiles do
     if (impl >= QS_POLICY_TENSOR || (impl == QS_POLICY_AUTO && n >= 16384)) {
         const char* msg = nullptr;
-        // float32-accurate tensor mode: the warp-specialised pipeline (qs_rollout.cu) or the chain kernels (qs_policy_tc.cu); both
-        // stay selectable (QS_POLICY_TENSOR_PIPELINE / _CHAINS) for A/B measurements, QS_POLICY_TENSOR and AUTO take the default
-        const bool pipeline = impl == QS_POLICY_TENSOR_PIPELINE || ((impl == QS_POLICY_TENSOR || impl == QS_POLICY_AUTO) && QS_POLICY_TENSOR_DEFAULT_PIPELINE);
-        if (pipeline) {
-            const int rc = launch_policy_pipeline(params, obs_dim, obs, noise, n, norm_stats, norm_eps, norm_clip, obs_norm_out, actions,
-                                                  actions_clipped, clip_lo, clip_hi, values, logp, (cudaStream_t)stream, &msg);
-            if (rc != QS_OK && msg) snprintf(g_policy_error, sizeof(g_policy_error), "%s", msg);
-            return rc;
-        }
-        const int rc = launch_policy_tc(impl != QS_POLICY_TENSOR_FAST, params, obs_dim, obs, noise, n, norm_stats, norm_eps, norm_clip,
-                                        obs_norm_out, actions, actions_clipped, clip_lo, clip_hi, values, logp, (cudaStream_t)stream, &msg);
+        // QS_POLICY_TENSOR_FAST: the three-chain kernel (qs_policy_tc.cu); the float32-accurate tensor mode (QS_POLICY_TENSOR,
+        // _PIPELINE and AUTO): the warp-specialised pipeline (qs_rollout_policy.cu)
+        const int rc = impl == QS_POLICY_TENSOR_FAST
+                           ? launch_policy_tc(params, obs_dim, obs, noise, n, norm_stats, norm_eps, norm_clip, obs_norm_out, actions,
+                                              actions_clipped, clip_lo, clip_hi, values, logp, (cudaStream_t)stream, &msg)
+                           : launch_policy_pipeline(params, obs_dim, obs, noise, n, norm_stats, norm_eps, norm_clip, obs_norm_out, actions,
+                                                    actions_clipped, clip_lo, clip_hi, values, logp, (cudaStream_t)stream, &msg);
         if (rc != QS_OK && msg) snprintf(g_policy_error, sizeof(g_policy_error), "%s", msg);
         return rc;
     }

@@ -10,71 +10,33 @@
 // error to ~1e-3 on |V| <= 2800 -- the same as torch's own float32 forward -- while the tensor pipe stays far from
 // saturated (the kernel is bound by the epilogue's MUFU work, not by MMA issue).
 //
-// Two kernels share this file: the two-chain kernel described next and the three-chain variant further down (the default).
-//
-// Layout: one persistent CTA per SM, two independent 256-thread groups, one 128-env tile per group (UMMA M=128, one env
-// per TMEM lane).  Each row is served by two threads (warps w and w+4 of a group share a TMEM lane quadrant) that take
-// alternate 32-column chunks of every epilogue, so 16 warps per SM keep the MUFU pipe fed while the other group's MMAs run.  Shared memory holds only the weights (float16 hi and lo, canonical K-major no-swizzle
-// core-matrix layout: offset(row, kchunk) = kchunk*rows*16 + row*16 bytes, LBO = rows*16, SBO = 128) and the float32
-// biases/heads.  Per group 256 TMEM columns:
-//     [  0,128)  layer-1 accumulator, overwritten IN PLACE by its own activations: each 32-column float32 chunk a thread
-//                reads becomes 16 columns of packed hi + 16 columns of packed lo (the A operand of layer 2);
-//                later reused as the layer-3 accumulator
-//     [128,192)  layer-2 accumulator -> in place -> A operand of layer 3
-//     [192,200)  the constant chunk (1, 0, ..., 0): A operand of the bias k-step of layers 2 and 3
-//     [224,256)  observation tile, hi | lo  (A operand of layer 1, kept for both nets); column k = OBS holds 1.0 (bias)
+// Layout: one persistent CTA per SM, three independent 128-env tiles ("chains", see policy_forward_tc3_kernel).  Shared memory holds
+// only the weights (float16 hi and lo, canonical K-major no-swizzle core-matrix layout: offset(row, kchunk) = kchunk*rows*16 +
+// row*16 bytes, LBO = rows*16, SBO = 128) and the float32 biases/heads.
 // In PRECISE mode weights and biases are pre-multiplied by 2*log2(e), so the accumulator IS the exponent of
 // tanh(x) = 1 - 2/(2^acc + 1); four elements share one reciprocal (tanh4_from_exponents): 5 MUFU per 4 tanh, then the hi/lo
 // split (LOP3, FADD, 2 F2FP per pair).  Hidden activations never touch shared memory: tcgen05.ld -> registers -> tanh, split
 // -> tcgen05.st.
 //
-// Scheduling, as measured with the clock64 phase trace (QS_TC_TRACE, tools/policy_trace.py): a tile is a serial chain
-// MMA -> epilogue -> MMA ... per group, so the two groups are the only overlap there is.  (1) The MMAs are issued by an elected
+// The kernel is launched in single-float16 mode only (QS_POLICY_TENSOR_FAST).  The float32-accurate forward (QS_POLICY_TENSOR)
+// runs on the warp-specialised pipeline kernel (qs_rollout_policy.cu), which measured faster than this kernel in PRECISE mode
+// (296 vs 308 us per 1M envs, profiles/r02/README.md).
+//
+// Scheduling, as measured with the clock64 phase trace (QS_TC_TRACE, tools/policy_trace3.py): (1) The MMAs are issued by an elected
 // lane under a WARP-UNIFORM branch: from a divergent `if (thread == 0)` each UTCHMMA cost an ELECT/R2UR waterfall (~100 cycles
-// per MMA, 8.7k of a tile's 23k cycles).  (2) The groups take turns on the MUFU-bound part of the epilogues (named barriers).
-// (3) The observation tile is staged one tile ahead (loaded, normalised, split and stored to TMEM by the half of the group that
-// does not issue MMAs, while the critic's layer-2 MMAs run); the tile after that is prefetched into L2.
+// per MMA, 8.7k of a tile's 23k cycles).  (2) The observation tile is staged one tile ahead (loaded, normalised, split and stored to
+// TMEM while the layer-2 MMAs of the critic run); the tile after that is prefetched into L2.
 #include "../../include/quadsim.h"
 #include "qs_tc.cuh"
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <stdlib.h>
 
 namespace qs {
 namespace tc {
 
 // (operand layouts, tcgen05/TMEM helpers, tanh and split routines: qs_tc.cuh)
-// QS_TC_TRACE (experimental builds only): threads 0 and 128 (the MMA issuer) of each group of CTA 0 stamp clock64 at every phase boundary of their
-// fourth tile; qs_policy_debug_trace() copies the stamps out.  See tools/policy_trace.py.
-#ifdef QS_TC_TRACE
-__device__ long long g_trace[2][2][64];
-#define QS_TR() do { if (tr_on && tr_i < 64) g_trace[g][tg >> 7][tr_i++] = clock64(); } while (0)
-#else
-#define QS_TR() do { } while (0)
-#endif
-
-// Ping-pong between the two groups (the scheme FlashAttention-3 uses for softmax vs GEMM): a group runs an epilogue
-// (MUFU-bound) only while it holds the turn, so the other group's MMA wait / loads / stores fall under it instead of both
-// groups idling the XU pipe at the same moments.  Barrier 3+g is "group g may run its epilogue": g syncs on it, the other
-// group arrives on it when its own epilogue ends.
-#ifdef QS_TC_EXPERIMENT_NO_TURNS     // timing experiment only: both groups free-running
-__device__ __forceinline__ void turn_wait(int) {}
-__device__ __forceinline__ void turn_pass(int) {}
-#else
-__device__ __forceinline__ void turn_wait(int g) { asm volatile("bar.sync %0, 512;" ::"r"(3 + g) : "memory"); }
-__device__ __forceinline__ void turn_pass(int g) { asm volatile("bar.arrive %0, 512;" ::"r"(3 + (g ^ 1)) : "memory"); }
-#endif
-// The turn starts once the accumulator chunk is in registers (the TMEM load needs no turn).  QS_TC_WIDE_TURN=1: it ends after
-// the activations are stored back; 0: right after the tanh math (split + TMEM store under the other group's turn).
-#ifndef QS_TC_WIDE_TURN
-#define QS_TC_WIDE_TURN 1
-#endif
-__device__ __forceinline__ void turn_pass_wide(int g) { if (QS_TC_WIDE_TURN) turn_pass(g); }
-__device__ __forceinline__ void turn_pass_narrow(int g) { if (!QS_TC_WIDE_TURN) turn_pass(g); }
-__device__ __forceinline__ void group_bar(int g) { asm volatile("bar.sync %0, 256;" ::"r"(g + 1) : "memory"); }
-
 struct Args {
     const float* params;
     const float* obs;
@@ -90,36 +52,7 @@ struct Args {
     float lo[4], hi[4];
 };
 
-// all MMAs of one layer: K elements from TMEM chunks of 32 (hi at +0, lo at +16), weights at wb_hi / wb_lo
-// `one_col` != 0: one more k-step whose A operand is the constant chunk (1,0,...) and whose B chunk holds the bias.
-template <bool PRECISE>
-__device__ __forceinline__ void issue_layer(uint32_t d_col, uint32_t a_col, int K, uint32_t wb_hi, uint32_t wb_lo, uint32_t b_lbo, int N,
-                                            uint32_t one_col) {
-    const uint32_t idesc = make_idesc(N);
-    uint32_t acc = 0;
-#ifdef QS_TC_EXPERIMENT_NO_MMA      // timing experiment only: how much of the kernel is MMA issue + execution
-    return;
-#endif
-    if (one_col) {
-        const int ks = K / 16;
-        umma_ts(d_col, one_col, make_desc(wb_hi + ks * 2 * b_lbo, b_lbo, 128), idesc, 0);
-        if (PRECISE) umma_ts(d_col, one_col, make_desc(wb_lo + ks * 2 * b_lbo, b_lbo, 128), idesc, 1);
-        acc = 1;
-    }
-    for (int ks = 0; ks < K / 16; ++ks) {
-        const uint32_t a_hi = a_col + 32u * (ks >> 1) + 8u * (ks & 1);
-        const uint64_t bh = make_desc(wb_hi + ks * 2 * b_lbo, b_lbo, 128);
-        umma_ts(d_col, a_hi, bh, idesc, acc);
-        acc = 1;
-        if (PRECISE) {
-            const uint64_t bl = make_desc(wb_lo + ks * 2 * b_lbo, b_lbo, 128);
-            umma_ts(d_col, a_hi, bl, idesc, 1);
-            umma_ts(d_col, a_hi + 16u, bh, idesc, 1);
-        }
-    }
-}
-
-// Observation row e -> (normalise) -> split float16 -> this lane's TMEM columns [COL_X, COL_X + 32): the A operand of layer 1.
+// Observation row e -> (normalise) -> split float16 -> this lane's 32 TMEM columns at x_addr: the A operand of layer 1.
 // Also pulls the row this thread will need one tile later into L2.
 template <int OBS, bool PRECISE>
 __device__ __forceinline__ void stage_obs_row(const Args& p, int64_t e, bool live, int64_t tile_stride_rows, uint32_t x_addr,
@@ -167,287 +100,17 @@ __device__ __forceinline__ void stage_obs_row(const Args& p, int64_t e, bool liv
     put32<PRECISE>(x_addr, x);
 }
 
-template <int OBS, bool PRECISE>
-__global__ void __launch_bounds__(THREADS, 1) policy_forward_tc_kernel(const Args p) {
-    extern __shared__ __align__(128) unsigned char smem[];
-    __shared__ uint32_t s_tmem_base;
-    __shared__ __align__(8) uint64_t s_bars[2];
-    __shared__ float s_mean[32], s_mean_lo[32], s_istd[32];
-    __shared__ __align__(16) float s_part[GROUPS][ROWS][NACT];                 // head partial sums of the second thread of each row
-    constexpr int OFF_LO = W_SET;                                 // lo parts follow the hi parts
-    constexpr int OFF_CONST = PRECISE ? 2 * W_SET : W_SET;
-    const int tid = threadIdx.x;
-    const int g = tid >> 8, tg = tid & 255, t = tg & 127, half = tg >> 7, warp = tid >> 5;   // t: env row, half: which chunks
-    const Blob B{OBS};
-    float* sC = reinterpret_cast<float*>(smem + OFF_CONST);
-
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&s_tmem_base)), "r"(TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-    }
-    if (tid == 0) {
-        mbar_init(smem_u32(&s_bars[0]), 1);
-        mbar_init(smem_u32(&s_bars[1]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    for (int net = 0; net < 2; ++net) {
-        const float sc = PRECISE ? 2.8853900817779268f : 1.0f;     // 2*log2(e): accumulators come out as exponents of 2
-        stage_weights<PRECISE>(p.params + B.w1(net), p.params + B.b1(net), OBS, OBS, K1, N1, sc, smem + OFF_W1 + net * W1_BYTES,
-                               smem + OFF_LO + OFF_W1 + net * W1_BYTES, tid);
-        stage_weights<PRECISE>(p.params + B.w2(net), p.params + B.b2(net), N1, N1, N1 + KB, N2, sc, smem + OFF_W2 + net * W2_BYTES,
-                               smem + OFF_LO + OFF_W2 + net * W2_BYTES, tid);
-        stage_weights<PRECISE>(p.params + B.w3(net), p.params + B.b3(net), N2, N2, N2 + KB, N3, sc, smem + OFF_W3 + net * W3_BYTES,
-                               smem + OFF_LO + OFF_W3 + net * W3_BYTES, tid);
-        for (int i = tid; i < N3 * NACT; i += THREADS) sC[C_WH + net * N3 * NACT + i] = __ldg(p.params + B.wh(net) + i);
-        if (tid < NACT) sC[C_BH + net * NACT + tid] = __ldg(p.params + B.bh(net) + tid);
-    }
-    if (tid < NACT) sC[C_LS + tid] = __ldg(p.params + B.log_std() + tid);
-    if (tid < OBS) {
-        double m = 0.0, is = 1.0;
-        if (p.norm) {
-            m = p.norm[1 + tid];
-            is = 1.0 / sqrt(p.norm[1 + OBS + tid] + (double)p.norm_eps);
-        }
-        s_mean[tid] = (float)m;
-        s_mean_lo[tid] = (float)(m - (double)(float)m);
-        s_istd[tid] = (float)is;
-    }
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    // warp-uniform copies for the MMA issuer (one warp of each group): everything the MMAs take derives from these
-    const int warp_u = __shfl_sync(0xffffffffu, tid >> 5, 0);
-    const int g_u = warp_u >> 3;
-    const bool issuer_warp = (warp_u & 7) == 4;                       // a warp of the half that does not stage observations
-    const uint32_t tmem_u = s_tmem_base + (uint32_t)g_u * 256u;
-    const uint32_t bar_u = smem_u32(&s_bars[0]) + 8u * (uint32_t)g_u;
-    const uint32_t tmem = s_tmem_base + (uint32_t)g * 256u;             // this group's 256 columns (lane field 0)
-    const uint32_t lane_addr = tmem + ((uint32_t)(t & ~31) << 16);     // this warp's lane quadrant
-    const uint32_t bar = smem_u32(&s_bars[g]);
-    const uint32_t sbase = smem_u32(smem);
-    uint32_t phase = 0;
-    constexpr uint32_t B1_LBO = N1 * 16, B2_LBO = N2 * 16;
-
-    {   // the constant A chunk (1, 0, ..., 0) of the bias k-steps: 8 columns of packed float16 per lane, written once
-        uint32_t one[16];
-#pragma unroll
-        for (int j = 0; j < 16; ++j) one[j] = 0u;
-        one[0] = 0x00003C00u;                                          // (1.0h, 0.0h)
-        if (half == 0) tmem_st16(lane_addr + COL_ONE, one);
-        tmem_st_wait();
-    }
-    const int64_t n_tiles = (p.n + ROWS - 1) / ROWS;
-    const int64_t tile_stride = (int64_t)gridDim.x * GROUPS;
-    if (g == 1) turn_pass(1);                                          // group 0 takes the first turn
-    // The observation tile is staged one tile ahead: the first one here, every later one inside the previous tile while the
-    // layer-2 MMAs of its critic run (X is dead once the critic's layer-1 MMAs have completed).
-    {
-        const int64_t tile = (int64_t)blockIdx.x * GROUPS + g;
-        if (tile < n_tiles && half == 0) {
-            const int64_t e = tile * ROWS + t;
-            stage_obs_row<OBS, PRECISE>(p, e, e < p.n, tile_stride * ROWS, lane_addr + COL_X, s_mean, s_mean_lo, s_istd);
-        }
-        tmem_st_wait();
-        tc_fence_before();
-        group_bar(g);
-    }
-    // both groups run the same number of rounds (group 0 never has fewer tiles); a group without a tile in the last
-    // round only keeps the turn moving
-    for (int64_t tile0 = (int64_t)blockIdx.x * GROUPS; tile0 < n_tiles; tile0 += tile_stride) {
-        const int64_t tile = tile0 + g;
-        if (tile >= n_tiles) {
-            for (int k = 0; k < 6; ++k) { turn_wait(g); turn_pass(g); }
-            continue;
-        }
-        const int64_t e = tile * ROWS + t;
-        const bool live = e < p.n;
-#ifdef QS_TC_TRACE
-        const bool tr_on = blockIdx.x == 0 && tile0 == (int64_t)gridDim.x * GROUPS * 3 && (tg == 0 || tg == 128);
-        int tr_i = 0;
-#endif
-        QS_TR();                                                        // 0: tile start
-        float mean[NACT] = {0.f, 0.f, 0.f, 0.f};
-        float value = 0.f;
-#pragma unroll 1
-        for (int net = 0; net < 2; ++net) {
-            // ---------------- layer 1: X[128 x 32] . W1^T -> R1[128 columns]
-            QS_TR();                                                    // a: before issue
-            if (issuer_warp) {
-                tc_fence_after();
-                if (elect_one()) {
-                    issue_layer<PRECISE>(tmem_u + COL_R1, tmem_u + COL_X, K1, sbase + OFF_W1 + net * W1_BYTES, sbase + OFF_LO + OFF_W1 + net * W1_BYTES, B1_LBO, N1, 0);
-                    umma_commit(bar_u);
-                }
-            }
-            QS_TR();                                                    // b: issued
-            __syncwarp();
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            __syncwarp();
-            tc_fence_after();
-            QS_TR();                                                    // c: MMAs complete
-            // The turn covers the MUFU work only; TMEM loads, the hi/lo split and the TMEM stores run outside it (or under
-            // the next load), i.e. under the other group's tanh.  This thread's chunks: half and half + 2 of the four.
-            {
-                static_assert(N1 / 32 == 4, "two chunks per thread");
-                uint32_t v[32];
-                float y[32];
-                const uint32_t c0 = lane_addr + COL_R1 + half * 32, c1 = c0 + 64;
-                tmem_ld32(c0, v);
-                tmem_ld_wait32(v);
-                turn_wait(g);
-                QS_TR();                                                // d: loaded, has the turn
-                tanh32<PRECISE>(v, y);
-                tmem_ld32(c1, v);
-                put32<PRECISE>(c0, y);                                   // in place: hi | lo
-                tmem_ld_wait32(v);
-                tanh32<PRECISE>(v, y);
-                turn_pass_narrow(g);
-                put32<PRECISE>(c1, y);
-                turn_pass_wide(g);
-            }
-            QS_TR();                                                    // e: epilogue done
-            tmem_st_wait();
-            tc_fence_before();
-            group_bar(g);
-            QS_TR();                                                    // f: group barrier passed
-            // ---------------- layer 2: H1[128 x 128] . W2^T -> R2[64 columns]
-            QS_TR();
-            if (issuer_warp) {
-                tc_fence_after();
-                if (elect_one()) {
-                    issue_layer<PRECISE>(tmem_u + COL_R2, tmem_u + COL_R1, N1, sbase + OFF_W2 + net * W2_BYTES, sbase + OFF_LO + OFF_W2 + net * W2_BYTES, B2_LBO, N2, tmem_u + COL_ONE);
-                    umma_commit(bar_u);
-                }
-            }
-            if (net == 1 && half == 0 && tile + tile_stride < n_tiles) {   // next tile's observations, under these MMAs
-                const int64_t en = (tile + tile_stride) * ROWS + t;
-                stage_obs_row<OBS, PRECISE>(p, en, en < p.n, tile_stride * ROWS, lane_addr + COL_X, s_mean, s_mean_lo, s_istd);
-            }
-            QS_TR();                                                    // b: issued
-            __syncwarp();
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            __syncwarp();
-            tc_fence_after();
-            QS_TR();                                                    // c: MMAs complete
-            {
-                uint32_t v[32];
-                float y[32];
-                tmem_ld32(lane_addr + COL_R2 + half * 32, v);
-                tmem_ld_wait32(v);
-                turn_wait(g);
-                QS_TR();                                                // d: loaded, has the turn
-                tanh32<PRECISE>(v, y);
-                turn_pass_narrow(g);
-                put32<PRECISE>(lane_addr + COL_R2 + half * 32, y);
-                turn_pass_wide(g);
-            }
-            QS_TR();                                                    // e: epilogue done
-            tmem_st_wait();
-            tc_fence_before();
-            group_bar(g);
-            QS_TR();                                                    // f: group barrier passed
-            // ---------------- layer 3: H2[128 x 64] . W3^T -> R1[first 64 columns], then the float32 head
-            QS_TR();
-            if (issuer_warp) {
-                tc_fence_after();
-                if (elect_one()) {
-                    issue_layer<PRECISE>(tmem_u + COL_R1, tmem_u + COL_R2, N2, sbase + OFF_W3 + net * W3_BYTES, sbase + OFF_LO + OFF_W3 + net * W3_BYTES, B2_LBO, N3, tmem_u + COL_ONE);
-                    umma_commit(bar_u);
-                }
-            }
-            QS_TR();                                                    // b: issued
-            __syncwarp();
-            mbar_wait(bar, phase);
-            phase ^= 1;
-            __syncwarp();
-            tc_fence_after();
-            QS_TR();                                                    // c: MMAs complete
-            float o[NACT];
-#pragma unroll
-            for (int j = 0; j < NACT; ++j) o[j] = half == 0 ? sC[C_BH + net * NACT + j] : 0.f;
-            {
-                const int cb = half;
-                uint32_t v[32];
-                float y[32];
-                tmem_ld32(lane_addr + COL_R1 + cb * 32, v);
-                tmem_ld_wait32(v);
-                turn_wait(g);
-                QS_TR();                                                // d: loaded, has the turn
-                tanh32<PRECISE>(v, y);
-                turn_pass(g);                                           // the float32 head below is FMA-pipe work: outside the turn
-                const float4* wh = reinterpret_cast<const float4*>(sC + C_WH + net * N3 * NACT + cb * 32 * NACT);
-#pragma unroll
-                for (int k = 0; k < 32; ++k) {
-                    const float4 w = wh[k];
-                    o[0] = fmaf(y[k], w.x, o[0]);
-                    o[1] = fmaf(y[k], w.y, o[1]);
-                    o[2] = fmaf(y[k], w.z, o[2]);
-                    o[3] = fmaf(y[k], w.w, o[3]);
-                }
-            }
-            if (half == 1) *reinterpret_cast<float4*>(&s_part[g][t][0]) = make_float4(o[0], o[1], o[2], o[3]);
-            QS_TR();
-            tc_fence_before();   // the next MMAs overwrite TMEM columns this thread has just read
-            group_bar(g);
-            QS_TR();
-            if (half == 0) {
-                const float4 q = *reinterpret_cast<const float4*>(&s_part[g][t][0]);
-                if (net == 0) {
-                    mean[0] = o[0] + q.x; mean[1] = o[1] + q.y; mean[2] = o[2] + q.z; mean[3] = o[3] + q.w;
-                } else {
-                    value = o[0] + q.x;
-                }
-            }
-        }
-        if (live && half == 0) {
-            const float ls[4] = {sC[C_LS], sC[C_LS + 1], sC[C_LS + 2], sC[C_LS + 3]};
-            float4 eps = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (p.noise) eps = __ldcs(reinterpret_cast<const float4*>(p.noise) + e);
-            float4 a;
-            a.x = fmaf(__expf(ls[0]), eps.x, mean[0]);
-            a.y = fmaf(__expf(ls[1]), eps.y, mean[1]);
-            a.z = fmaf(__expf(ls[2]), eps.z, mean[2]);
-            a.w = fmaf(__expf(ls[3]), eps.w, mean[3]);
-            const float HALF_LOG_2PI = 0.9189385332046727f;
-            const float lp = -0.5f * (eps.x * eps.x + eps.y * eps.y + eps.z * eps.z + eps.w * eps.w) - (ls[0] + ls[1] + ls[2] + ls[3]) -
-                             4.0f * HALF_LOG_2PI;
-            __stcs(reinterpret_cast<float4*>(p.actions) + e, a);       // rollout-buffer outputs stream past L2; the clipped actions
-                                                                        // the env step reads next stay cacheable
-            if (p.actions_clipped) {
-                float4 c;
-                c.x = fminf(fmaxf(a.x, p.lo[0]), p.hi[0]);
-                c.y = fminf(fmaxf(a.y, p.lo[1]), p.hi[1]);
-                c.z = fminf(fmaxf(a.z, p.lo[2]), p.hi[2]);
-                c.w = fminf(fmaxf(a.w, p.lo[3]), p.hi[3]);
-                reinterpret_cast<float4*>(p.actions_clipped)[e] = c;
-            }
-            __stcs(p.values + e, value);
-            __stcs(p.logp + e, lp);
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) {
-        tc_fence_after();
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(s_tmem_base), "r"(TMEM_COLS));
-    }
-}
-
-
 // =====================================================================================================================
-// Three-chain variant.  A tile is a serial chain MMA -> epilogue -> MMA ..., so throughput is the number of chains in flight
-// per SM, and TMEM (512 columns) is what limits it.  Here a chain needs 160 columns instead of 232:
+// The kernel.  A tile is a serial chain MMA -> epilogue -> MMA ..., so throughput is the number of chains in flight per SM, and
+// TMEM (512 columns) is what limits it.  Here a chain needs 160 columns instead of the 232 of whole-layer accumulators:
 //     [  0, 64)  R_a: layer-1 accumulator, one 64-output HALF at a time -> in place -> A operand of a partial layer 2;
 //                later the layer-3 accumulator
 //     [ 64,128)  R_2: layer-2 accumulator (sum of the two partial products) -> in place -> A operand of layer 3
 //     [128,160)  observation tile hi | lo
 // and column 480 holds the constant (1, 0, ...) chunk for all chains.  Layer 2 is accumulated as the halves of layer 1 finish:
 //     L1a -> tanh -> [L2 (+)= H1a.W2[0:64]  and  L1b, issued back to back: MMAs execute in issue order] -> tanh -> L2 += H1b.W2[64:128]
-// Three 128-thread groups (one thread per env row, 168 registers available), one tile each, no turns: with one warp per
-// scheduler and chain the MUFU contention inside a group is gone and the three chains interleave on their own.
+// Three 128-thread groups (one thread per env row, 168 registers available), one tile each: with one warp per scheduler and
+// chain the three chains interleave on their own, without turns between the groups.
 #ifdef QS_TC_TRACE
 __device__ long long g_trace3[3][2][80];
 #define QS_TR3() do { if (tr_on && tr_i < 80) g_trace3[g][t >> 5][tr_i++] = clock64(); } while (0)
@@ -463,9 +126,6 @@ template <bool PRECISE>
 __device__ __forceinline__ void issue_part(uint32_t d_col, uint32_t a_col, int n_ks, int b_ks0, uint32_t wb_hi, uint32_t wb_lo, uint32_t b_lbo,
                                            int N, uint32_t acc, uint32_t one_col, int bias_ks) {
     const uint32_t idesc = make_idesc(N);
-#ifdef QS_TC_EXPERIMENT_NO_MMA
-    return;
-#endif
     if (one_col) {
         umma_ts(d_col, one_col, make_desc(wb_hi + bias_ks * 2 * b_lbo, b_lbo, 128), idesc, acc);
         acc = 1;
@@ -492,31 +152,14 @@ template <bool PRECISE>
 __device__ __forceinline__ void epilogue64(uint32_t col) {
     uint32_t v0[32], v1[32];
     float y[32];
-#ifdef QS_TC_EXPERIMENT_NO_LD      // timing experiments only (results are garbage): what does the TMEM load / store traffic cost
-#pragma unroll
-    for (int i = 0; i < 32; ++i) { v0[i] = 0x3f000000u + col + i; v1[i] = 0x3e800000u + col + i; }
-#else
     tmem_ld32(col, v0);
     tmem_ld32(col + 32, v1);
-#endif
     tmem_ld_wait32(v0);
     tanh32<PRECISE>(v0, y);
-#ifdef QS_TC_EXPERIMENT_NO_ST
-    float acc = 0.f;
-#pragma unroll
-    for (int i = 0; i < 32; ++i) acc += y[i];
-#else
     put32<PRECISE>(col, y);
-#endif
     tmem_ld_wait32(v1);
     tanh32<PRECISE>(v1, y);
-#ifdef QS_TC_EXPERIMENT_NO_ST
-#pragma unroll
-    for (int i = 0; i < 32; ++i) acc += y[i];
-    if (acc == 123.456f) put32<PRECISE>(col, y);
-#else
     put32<PRECISE>(col + 32, y);
-#endif
 }
 
 template <int OBS, bool PRECISE>
@@ -755,9 +398,6 @@ __global__ void __launch_bounds__(THREADS3, 1) policy_forward_tc3_kernel(const A
 }  // namespace tc
 
 #ifdef QS_TC_TRACE
-extern "C" int qs_policy_debug_trace(long long* out_host) {
-    return (int)cudaMemcpyFromSymbol(out_host, tc::g_trace, sizeof(tc::g_trace));
-}
 extern "C" int qs_policy_debug_trace3(long long* out_host) {
     return (int)cudaMemcpyFromSymbol(out_host, tc::g_trace3, sizeof(tc::g_trace3));
 }
@@ -765,31 +405,23 @@ extern "C" int qs_policy_debug_trace3(long long* out_host) {
 
 thread_local char g_policy_tc_error[256] = "";
 
-template <int OBS, bool PRECISE>
+// single-float16 mode (PRECISE = false) only: see the head of this file
+template <int OBS>
 static cudaError_t launch_three(const tc::Args& a, int sms, cudaStream_t stream) {
-    const int smem = (PRECISE ? 2 : 1) * tc::W_SET + tc::C_TOTAL * 4 + 64;
-    cudaError_t err = cudaFuncSetAttribute(tc::policy_forward_tc3_kernel<OBS, PRECISE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    const int smem = tc::W_SET + tc::C_TOTAL * 4 + 64;
+    cudaError_t err = cudaFuncSetAttribute(tc::policy_forward_tc3_kernel<OBS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (err != cudaSuccess) return err;
     const int64_t tiles = (a.n + tc::ROWS - 1) / tc::ROWS;
     const int64_t ctas = (tiles + tc::G3 - 1) / tc::G3;
     const unsigned grid = (unsigned)(ctas < sms ? ctas : sms);
-    tc::policy_forward_tc3_kernel<OBS, PRECISE><<<grid, tc::THREADS3, smem, stream>>>(a);
+    tc::policy_forward_tc3_kernel<OBS, false><<<grid, tc::THREADS3, smem, stream>>>(a);
     return cudaGetLastError();
 }
 
-template <int OBS, bool PRECISE>
-static cudaError_t launch_one(const tc::Args& a, unsigned grid, cudaStream_t stream) {
-    const int smem = (PRECISE ? 2 : 1) * tc::W_SET + tc::C_TOTAL * 4 + 64;
-    cudaError_t err = cudaFuncSetAttribute(tc::policy_forward_tc_kernel<OBS, PRECISE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (err != cudaSuccess) return err;
-    tc::policy_forward_tc_kernel<OBS, PRECISE><<<grid, tc::THREADS, smem, stream>>>(a);
-    return cudaGetLastError();
-}
-
-int launch_policy_tc(int precise, const float* params, int obs_dim, const float* obs, const float* noise, int64_t n,
-                      const double* norm_stats, float norm_eps, float norm_clip, float* obs_norm_out, float* actions,
-                      float* actions_clipped, const float* clip_lo, const float* clip_hi, float* values, float* logp,
-                      cudaStream_t stream, const char** err_out) {
+int launch_policy_tc(const float* params, int obs_dim, const float* obs, const float* noise, int64_t n, const double* norm_stats,
+                     float norm_eps, float norm_clip, float* obs_norm_out, float* actions, float* actions_clipped,
+                     const float* clip_lo, const float* clip_hi, float* values, float* logp, cudaStream_t stream,
+                     const char** err_out) {
     using namespace tc;
     Args a;
     a.params = params; a.obs = obs; a.noise = noise; a.norm = norm_stats; a.obs_norm_out = obs_norm_out;
@@ -799,19 +431,9 @@ int launch_policy_tc(int precise, const float* params, int obs_dim, const float*
     int dev = 0, sms = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const int64_t tiles = (n + ROWS - 1) / ROWS;
-    const int64_t ctas = (tiles + GROUPS - 1) / GROUPS;
-    const unsigned grid = (unsigned)(ctas < sms ? ctas : sms);
-    cudaError_t err;
-    // QS_POLICY_TC_CHAINS=2 selects the two-chain kernel (kept for comparison); default: three chains
-    static const bool three = []() { const char* e = getenv("QS_POLICY_TC_CHAINS"); return !(e && e[0] == '2'); }();
-    if (three) {
-        if (obs_dim == 20) err = precise ? launch_three<20, true>(a, sms, stream) : launch_three<20, false>(a, sms, stream);
-        else err = precise ? launch_three<17, true>(a, sms, stream) : launch_three<17, false>(a, sms, stream);
-    } else if (obs_dim == 20) err = precise ? launch_one<20, true>(a, grid, stream) : launch_one<20, false>(a, grid, stream);
-    else err = precise ? launch_one<17, true>(a, grid, stream) : launch_one<17, false>(a, grid, stream);
+    const cudaError_t err = obs_dim == 20 ? launch_three<20>(a, sms, stream) : launch_three<17>(a, sms, stream);
     if (err != cudaSuccess) {
-        snprintf(g_policy_tc_error, sizeof(g_policy_tc_error), "policy_forward_tc_kernel: %s", cudaGetErrorString(err));
+        snprintf(g_policy_tc_error, sizeof(g_policy_tc_error), "policy_forward_tc3_kernel: %s", cudaGetErrorString(err));
         *err_out = g_policy_tc_error;
         return QS_ECUDA;
     }

@@ -43,30 +43,6 @@ __device__ __forceinline__ uint32_t real_as_u32(float v) { return __float_as_uin
 template <typename Real, int VER>
 __device__ __forceinline__ void pool_unpack(const Real* slot, EnvState<Real, VER>& s);
 
-// One warp tile (32 envs) of the pool staged in shared memory by one bulk copy (same layout as in HBM): plane v at stage +
-// v*512 (lane*16), tail plane t at stage + NVEC*512 + t*128 (lane*4).  Conflict-free LDS.128 per plane.
-template <typename Real, int VER>
-__device__ __forceinline__ void pool_load_staged(const unsigned char* stage, int lane, EnvState<Real, VER>& s) {
-    using L = PoolLayout<Real, VER>;
-    using V = typename VecOf<Real>::type;
-    Real slot[L::NVEC * L::W + (L::NTAIL ? L::NTAIL : 1)];
-#pragma unroll
-    for (int v = 0; v < L::NVEC; ++v) {
-        const V x = *reinterpret_cast<const V*>(stage + v * 512 + lane * 16);
-        if (L::W == 4) {
-            const float4 f = *reinterpret_cast<const float4*>(&x);
-            slot[4 * v + 0] = (Real)f.x; slot[4 * v + 1] = (Real)f.y; slot[4 * v + 2] = (Real)f.z; slot[4 * v + 3] = (Real)f.w;
-        } else {
-            const double2 f = *reinterpret_cast<const double2*>(&x);
-            slot[2 * v + 0] = (Real)f.x; slot[2 * v + 1] = (Real)f.y;
-        }
-    }
-#pragma unroll
-    for (int t = 0; t < L::NTAIL; ++t)
-        slot[L::NVEC * L::W + t] = *reinterpret_cast<const Real*>(stage + L::NVEC * 512 + t * 32 * (int)sizeof(Real) + lane * (int)sizeof(Real));
-    pool_unpack<Real, VER>(slot, s);
-}
-
 template <typename Real, int VER>
 __device__ __forceinline__ void pool_load(const void* __restrict__ base, int64_t n, int64_t e, EnvState<Real, VER>& s) {
     using L = PoolLayout<Real, VER>;

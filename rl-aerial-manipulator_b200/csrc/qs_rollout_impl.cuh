@@ -51,34 +51,22 @@ using namespace tc;
 // registers with setmaxnreg (warpgroups of 4 warps: MMA group gives, env and epilogue groups take).
 constexpr int EPI_SPLIT = QS_RO_EPI_SPLIT, ENV_SPLIT = QS_RO_ENV_SPLIT;
 // Which of the EPI_SPLIT warps of a (slot, quadrant) takes hidden-layer chunk ch (0-3: layer 1, 4-5: layer 2) and which take the two
-// head chunks.  Three warps: (c0, c3, head 0) | (c1, head 1, c4) | (c2, c5) -- 3 / 3 / 2 chunk units per job.
-constexpr int HEAD_SPLIT = EPI_SPLIT < 2 ? EPI_SPLIT : 2;
-__host__ __device__ constexpr int chunk_owner(int ch) { return EPI_SPLIT == 3 ? (ch < 4 ? ch % 3 : (ch - 3) % 3) : ch % EPI_SPLIT; }
+// head chunks.
+static_assert(EPI_SPLIT == 1 || EPI_SPLIT == 2, "one or two epilogue warps per (slot, quadrant)");
+constexpr int HEAD_SPLIT = EPI_SPLIT;
+__host__ __device__ constexpr int chunk_owner(int ch) { return ch % EPI_SPLIT; }
 constexpr int EPI_WARPS = 8 * EPI_SPLIT, ENV_WARPS = 4 * ENV_SPLIT, MMA_WARPS = 2;
-// A/B switch (QS_RO_ENV_FIRST): which role gets the low warp ids -- the schedulers favour older (lower) warps when several are
-// ready, and the env warps' few MUFU ops queue behind the epilogue warps' thousands
-#ifndef QS_RO_ENV_FIRST
-#define QS_RO_ENV_FIRST 0
-#endif
-#ifndef QS_RO_LDBUF
-#define QS_RO_LDBUF 1
-#endif
-// QS_RO_LD_SPLIT: the epilogue loads a 32-column chunk as two 16-column halves and converts the first while the second is in
-// flight (tcgen05.ld latency off the warp's critical path); needs the k-step-local activation layout (see issue_chunk)
-#ifndef QS_RO_LD_SPLIT
-#define QS_RO_LD_SPLIT 0
-#endif
-// QS_RO_ST16: the epilogue stores a converted chunk with two 16-column tcgen05.st from ONE address register instead of eight 4-column
+// ST16: the epilogue stores a converted chunk with two 16-column tcgen05.st from ONE address register instead of eight 4-column
 // ones (each needs its address in a uniform register: 9 R2UR + 12 register moves per chunk in the SASS).  Policy build (80 registers):
 // 275.1 -> 266.5 us per 1M-env launch; the fused build's epilogue warps (72 / 88 registers) get slower with it (378 -> 392 us).
-#ifndef QS_RO_ST16
 #ifdef QS_RO_BUILD_POLICY
-#define QS_RO_ST16 1
+constexpr bool ST16 = true;
 #else
-#define QS_RO_ST16 0
+constexpr bool ST16 = false;
 #endif
-#endif
-constexpr int W_EPI0 = QS_RO_ENV_FIRST ? ENV_WARPS : 0, W_ENV0 = QS_RO_ENV_FIRST ? 0 : EPI_WARPS, W_MMA0 = EPI_WARPS + ENV_WARPS;
+// the schedulers favour older (lower) warps when several are ready: the epilogue warps, whose MUFU work is the critical path, get
+// the low warp ids
+constexpr int W_EPI0 = 0, W_ENV0 = EPI_WARPS, W_MMA0 = EPI_WARPS + ENV_WARPS;
 // the block is padded to whole groups of 4 warps: registers are allocated per 4 warps anyway (a 448 x 144 launch is refused)
 constexpr int RO_WARPS = ((EPI_WARPS + ENV_WARPS + MMA_WARPS + 3) / 4) * 4;
 constexpr int RO_THREADS = RO_WARPS * 32;
@@ -173,16 +161,10 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 // all issued instructions (ncu, profiles/r02) and starved the warps that had work.  So: the suspend-time hint of try_wait (the
 // thread sleeps in the barrier unit until the phase completes, the hint expires or -- as measured -- another barrier of the CTA is hit).
 // No nanosleep between polls: `nanosleep.u32` has a coarse granularity here (a 20 ns and a 500 ns request cost the same, and made
-// every hand-over slower: 294 -> 336 us for the policy part).
-#ifndef QS_RO_WAIT_HINT_NS
-#define QS_RO_WAIT_HINT_NS 20000
-#endif
-#ifndef QS_RO_BACKOFF_NS
-#define QS_RO_BACKOFF_NS 0
-#endif
+// every hand-over slower: 294 -> 336 us for the policy part).  Hint 0 (plain spin) / 1 us / 20 us: 293.5 / 294.6 / 293.7 us (r02).
+constexpr uint32_t WAIT_HINT_NS = 20000;
 __device__ __forceinline__ uint32_t mbar_try(uint32_t bar, uint32_t parity) {
     uint32_t ok;
-#if QS_RO_WAIT_HINT_NS > 0
     asm volatile(
         "{\n\t"
         ".reg .pred p;\n\t"
@@ -190,19 +172,8 @@ __device__ __forceinline__ uint32_t mbar_try(uint32_t bar, uint32_t parity) {
         "selp.u32 %0, 1, 0, p;\n\t"
         "}\n"
         : "=r"(ok)
-        : "r"(bar), "r"(parity), "r"((uint32_t)QS_RO_WAIT_HINT_NS)
+        : "r"(bar), "r"(parity), "r"(WAIT_HINT_NS)
         : "memory");
-#else
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}\n"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-#endif
     return ok;
 }
 // non-blocking probe
@@ -219,15 +190,11 @@ __device__ __forceinline__ uint32_t mbar_test(uint32_t bar, uint32_t parity) {
         : "memory");
     return ok;
 }
-// QS_RO_TIGHT_WAIT (r02): the whole bounded wait is ONE asm block -- try_wait (hinted), branch, counter -- 5 SASS instructions per
+// The whole bounded wait (r02) is ONE asm block -- try_wait (hinted), branch, counter -- 5 SASS instructions per
 // wake-up instead of the ~16 the C loop compiled to.  A parked warp is woken by every barrier event of the CTA (measured: ~7.7M
 // wake-ups per 1M-env launch), and with the epilogue warps busy back to back those wake-ups competed for issue slots that were
 // 72 % taken (ncu): the loop's length is a cost, not a detail.  The bound stays: 2^22 wake-ups (seconds), then the sticky status.
-#ifndef QS_RO_TIGHT_WAIT
-#define QS_RO_TIGHT_WAIT 1
-#endif
 __device__ __forceinline__ bool mbar_wait_slow(uint32_t bar, uint32_t parity, int code) {
-#if QS_RO_TIGHT_WAIT
     uint32_t ok;
     asm volatile(
         "{\n\t"
@@ -244,18 +211,9 @@ __device__ __forceinline__ bool mbar_wait_slow(uint32_t bar, uint32_t parity, in
         "selp.u32 %0, 1, 0, p;\n\t"
         "}\n"
         : "=r"(ok)
-        : "r"(bar), "r"(parity), "r"((uint32_t)(QS_RO_WAIT_HINT_NS > 0 ? QS_RO_WAIT_HINT_NS : 1000))
+        : "r"(bar), "r"(parity), "r"(WAIT_HINT_NS)
         : "memory");
     if (ok) return true;
-#else
-    for (uint32_t it = 0; it < (1u << 17); ++it) {                 // x (up to) 20 us per try: seconds, not minutes
-#if QS_RO_BACKOFF_NS > 0
-        __nanosleep(QS_RO_BACKOFF_NS);
-#endif
-        if (mbar_try(bar, parity)) return true;
-        if ((it & 0xFF) == 0xFF && *reinterpret_cast<volatile int*>(&g_ro_status) != 0) break;   // somebody else already gave up
-    }
-#endif
     atomicCAS(&g_ro_status, 0, code);
     return false;
 }
@@ -267,21 +225,15 @@ __device__ __forceinline__ bool mbar_wait_bounded(uint32_t bar, uint32_t parity,
 // period late): a hinted try_wait is woken by EVERY barrier event of the CTA -- measured 83 wake-ups per output wait, 2.7 M per
 // 1M-env launch, ~8 % of all issued instructions, taken from the epilogue warps' issue slots -- so this one sleeps on the timer
 // between probes instead (nanosleep is coarse, ~0.5-1 us: far below the tile period of ~5 us).
-#ifndef QS_RO_LAZY_WAIT_NS
-#define QS_RO_LAZY_WAIT_NS 600
-#endif
+constexpr uint32_t LAZY_WAIT_NS = 600;
 __device__ __forceinline__ bool mbar_wait_lazy(uint32_t bar, uint32_t parity, int code) {
-#if QS_RO_LAZY_WAIT_NS > 0
     if (mbar_test(bar, parity)) return true;
     for (uint32_t it = 0; it < (1u << 22); ++it) {                 // x ~1 us: seconds, then the sticky status
-        __nanosleep(QS_RO_LAZY_WAIT_NS);
+        __nanosleep(LAZY_WAIT_NS);
         if (mbar_test(bar, parity)) return true;
     }
     atomicCAS(&g_ro_status, 0, code);
     return false;
-#else
-    return mbar_wait_bounded(bar, parity, code);
-#endif
 }
 // D[tmem] (+)= A[smem] . B[smem]^T
 __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -294,17 +246,9 @@ __device__ __forceinline__ void umma_ss(uint32_t tmem_d, uint64_t adesc, uint64_
         : "memory");
 }
 // (a, b) -> packed float16 hi (round to nearest) and packed lo = exact remainders: F2FP + 2 FHFMA + F2FP per pair (the
-// LOP3 / FADD / 2 x F2FP sequence of qs_tc.cuh::split_h2 costs 6)
+// LOP3 / FADD / 2 x F2FP sequence of qs_tc.cuh::split_h2 costs 6; measured in its place: +2.6 %, r02)
 __device__ __forceinline__ void split_h2_rn(float a, float b, uint32_t& hi, uint32_t& lo) {
     asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(b), "f"(a));
-#ifdef QS_X_NOSPLIT                          // timing experiment only (wrong numerics): what the lo half costs
-    lo = hi ^ 0x3C003C00u;
-    return;
-#endif
-#ifdef QS_X_TRUNCSPLIT                       // A/B: hi by truncation (LOP3 on the ALU pipe), lo = exact remainder by FADD (r01's split)
-    split_h2(a, b, hi, lo);
-    return;
-#endif
     float la, lb;
     asm("{\n\t"
         ".reg .f16 l, h, m;\n\t"
@@ -365,13 +309,12 @@ __device__ __forceinline__ void issue_chunk(uint32_t d, uint32_t a_col, int ch, 
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
         const int ks = 2 * ch + j;
-        // activation layout inside a 32-column chunk: QS_RO_LD_SPLIT = 0: [hi k-step 0 | hi k-step 1 | lo 0 | lo 1] (8 columns each);
-        // = 1: [hi 0 | lo 0 | hi 1 | lo 1], i.e. each k-step's 16 activations stay inside their own 16 columns
-        const uint32_t a_hi = a_col + 32u * ch + (QS_RO_LD_SPLIT ? 16u : 8u) * j;
+        // activation layout inside a 32-column chunk: [hi k-step 0 | hi k-step 1 | lo 0 | lo 1] (8 columns each)
+        const uint32_t a_hi = a_col + 32u * ch + 8u * j;
         const uint64_t bh = make_desc(wh + ks * 2 * B_LBO, B_LBO, 128), bl = make_desc(wl + ks * 2 * B_LBO, B_LBO, 128);
         umma_ts(d, a_hi, bh, idesc, 1);
         umma_ts(d, a_hi, bl, idesc, 1);
-        umma_ts(d, a_hi + (QS_RO_LD_SPLIT ? 8u : 16u), bh, idesc, 1);
+        umma_ts(d, a_hi + 16u, bh, idesc, 1);
     }
 }
 
@@ -468,22 +411,6 @@ __device__ __forceinline__ void role_mma(const Ctx& c, int slot) {
 __device__ __forceinline__ void tmem_st4(uint32_t taddr, const uint32_t* v) {
     asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};\n" ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
 }
-// One 32-column accumulator chunk of this lane's row at `col`: tcgen05.ld -> tanh -> hi | lo split, stored in place over the chunk
-// (hi halves in columns [0,16), lo halves in [16,32)).  Eight activations at a time keep the live registers near 64.
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* v) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait16(uint32_t* v) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]), "+r"(v[9]),
-                   "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15])
-                 :
-                 : "memory");
-}
 // eight activations of this lane's row: tanh -> hi | lo packed halves stored at hi_col / lo_col (4 columns each)
 __device__ __forceinline__ void tanh_split8(const uint32_t* v, uint32_t hi_col, uint32_t lo_col) {
     float y[8];
@@ -494,48 +421,39 @@ __device__ __forceinline__ void tanh_split8(const uint32_t* v, uint32_t hi_col, 
     tmem_st4(hi_col, h);
     tmem_st4(lo_col, l);
 }
+// One 32-column accumulator chunk of this lane's row at `col`: tcgen05.ld -> tanh -> hi | lo split, stored in place over the chunk
+// (hi halves in columns [0,16), lo halves in [16,32)).  Eight activations at a time keep the live registers near 64.
 __device__ __forceinline__ void chunk_tanh_split(uint32_t col) {
     uint32_t v[32];
-#if QS_RO_LD_SPLIT
-    tmem_ld16(col, v);
-    tmem_ld_wait16(v);
-    tmem_ld16(col + 16u, v + 16);                     // in flight while the first 16 activations are converted (they stay inside columns [0, 16))
-    tanh_split8(v, col, col + 8u);
-    tanh_split8(v + 8, col + 4u, col + 12u);
-    tmem_ld_wait16(v + 16);
-    tanh_split8(v + 16, col + 16u, col + 24u);
-    tanh_split8(v + 24, col + 20u, col + 28u);
-#else
     tmem_ld32(col, v);
     tmem_ld_wait32(v);
-#if QS_RO_ST16                                   // A/B: two 16-column stores per chunk (one address, no per-store R2UR) instead of eight 4-column ones
-    uint32_t h[16], l[16];
+    if constexpr (ST16) {                        // two 16-column stores per chunk (one address, no per-store R2UR) instead of eight 4-column ones
+        uint32_t h[16], l[16];
 #pragma unroll
-    for (int sb = 0; sb < 4; ++sb) {
-        float y[8];
-        tanh8_from_exponents(v + 8 * sb, y);
+        for (int sb = 0; sb < 4; ++sb) {
+            float y[8];
+            tanh8_from_exponents(v + 8 * sb, y);
 #pragma unroll
-        for (int j = 0; j < 4; ++j) split_h2_rn(y[2 * j], y[2 * j + 1], h[4 * sb + j], l[4 * sb + j]);
+            for (int j = 0; j < 4; ++j) split_h2_rn(y[2 * j], y[2 * j + 1], h[4 * sb + j], l[4 * sb + j]);
+        }
+        asm volatile(
+            "{\n\t"
+            ".reg .b32 a2;\n\t"
+            "add.u32 a2, %0, 16;\n\t"
+            "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n\t"
+            "tcgen05.st.sync.aligned.32x32b.x16.b32 [a2], {%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};\n\t"
+            "}\n" ::"r"(col),
+            "r"(h[0]), "r"(h[1]), "r"(h[2]), "r"(h[3]), "r"(h[4]), "r"(h[5]), "r"(h[6]), "r"(h[7]), "r"(h[8]), "r"(h[9]), "r"(h[10]), "r"(h[11]), "r"(h[12]),
+            "r"(h[13]), "r"(h[14]), "r"(h[15]), "r"(l[0]), "r"(l[1]), "r"(l[2]), "r"(l[3]), "r"(l[4]), "r"(l[5]), "r"(l[6]), "r"(l[7]), "r"(l[8]), "r"(l[9]),
+            "r"(l[10]), "r"(l[11]), "r"(l[12]), "r"(l[13]), "r"(l[14]), "r"(l[15])
+            : "memory");
+    } else {
+#pragma unroll
+        for (int sb = 0; sb < 4; ++sb) tanh_split8(v + 8 * sb, col + 4u * sb, col + 16u + 4u * sb);
     }
-    asm volatile(
-        "{\n\t"
-        ".reg .b32 a2;\n\t"
-        "add.u32 a2, %0, 16;\n\t"
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n\t"
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [a2], {%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};\n\t"
-        "}\n" ::"r"(col),
-        "r"(h[0]), "r"(h[1]), "r"(h[2]), "r"(h[3]), "r"(h[4]), "r"(h[5]), "r"(h[6]), "r"(h[7]), "r"(h[8]), "r"(h[9]), "r"(h[10]), "r"(h[11]), "r"(h[12]),
-        "r"(h[13]), "r"(h[14]), "r"(h[15]), "r"(l[0]), "r"(l[1]), "r"(l[2]), "r"(l[3]), "r"(l[4]), "r"(l[5]), "r"(l[6]), "r"(l[7]), "r"(l[8]), "r"(l[9]),
-        "r"(l[10]), "r"(l[11]), "r"(l[12]), "r"(l[13]), "r"(l[14]), "r"(l[15])
-        : "memory");
-#else
-#pragma unroll
-    for (int sb = 0; sb < 4; ++sb) tanh_split8(v + 8 * sb, col + 4u * sb, col + 16u + 4u * sb);
-#endif
-#endif
 }
 
-// Order of a warp's work (QS_RO_DEFER_HEAD, r02): the head of job j-1 runs BETWEEN the layer-1 and the layer-2 epilogue of job j,
+// Order of a warp's work (DEFER_HEAD, r02): the head of job j-1 runs BETWEEN the layer-1 and the layer-2 epilogue of job j,
 //     E1(j) -> head(j-1) -> E2(j) -> E1(j+1) -> head(j) -> E2(j+1) -> ...
 // instead of E1(j) -> E2(j) -> head(j).  In the straight order the warp idles twice per job -- after E1 until the last two chunks'
 // MMAs have produced D2 (800-1,800 cycles) and after E2 until D3 (700-1,150; phase trace, profiles/r02) -- 40 % of a job.  Deferred,
@@ -543,18 +461,14 @@ __device__ __forceinline__ void chunk_tanh_split(uint32_t col) {
 // D1(j+1) (issued behind layer 2 of job j) under head(j-1) + E2(j).  Nothing else changes: D3 is not overwritten before layer 3 of
 // job j, which the MMA warp issues after E2(j) and after D3FREE, i.e. after head(j-1).  The env warps consume a tile's outputs one
 // iteration later to match (LAG in role_env).
-#ifndef QS_RO_DEFER_HEAD
-#define QS_RO_DEFER_HEAD 1
-#endif
-// QS_RO_HEAD_SCALAR_VF: the critic's head has one output -- a scalar weight and one FFMA per activation instead of the actor's float4 and
+constexpr uint32_t DEFER_HEAD = 1;
+// HEAD_SCALAR_VF: the critic's head has one output -- a scalar weight and one FFMA per activation instead of the actor's float4 and
 // four.  Policy build: 280.1 -> 276.2 us; the fused build (one epilogue warp per (slot, quadrant), larger code) gets slower with the
 // second head body (374.5 -> 389.9 us): off there.
-#ifndef QS_RO_HEAD_SCALAR_VF
 #ifdef QS_RO_BUILD_POLICY
-#define QS_RO_HEAD_SCALAR_VF 1
+constexpr bool HEAD_SCALAR_VF = true;
 #else
-#define QS_RO_HEAD_SCALAR_VF 0
-#endif
+constexpr bool HEAD_SCALAR_VF = false;
 #endif
 __device__ __forceinline__ void role_epilogue(const Ctx& c, int slot, int half, int quad, int lane, const float* sC, float4* s_mean, float* s_val) {
     const uint32_t tm = c.tmem + slot * SLOT_COLS + ((uint32_t)(quad * 32) << 16);
@@ -565,18 +479,17 @@ __device__ __forceinline__ void role_epilogue(const Ctx& c, int slot, int half, 
     RO_TRACE_INIT();
     // iteration `job` does E1(job), head(job - DEFER), E2(job); one extra iteration drains the last head
 #pragma unroll 1
-    for (uint32_t job = 0; job < njobs + QS_RO_DEFER_HEAD; ++job) {
+    for (uint32_t job = 0; job < njobs + DEFER_HEAD; ++job) {
         const uint32_t par = job & 1u;
         const bool live = job < njobs;
         // chunks 0-3: layer-1 accumulator D1 -> H1; chunks 4-5: layer-2 accumulator D2 -> H2 (D2 follows D1 in the slot's columns);
         // this warp takes every EPI_SPLIT-th chunk.  Each: tcgen05.ld -> tanh -> hi | lo in place -> signal the MMA warp.
 #pragma unroll 1
         for (int stage = 0; stage < 3; ++stage) {
-            if (stage == (QS_RO_DEFER_HEAD ? 1 : 2)) {
+            if (stage == (DEFER_HEAD ? 1 : 2)) {
                 // ---- head of job hj: layer-3 accumulator D3 -> tanh -> partial sums against the float32 head weights
-                if (QS_RO_DEFER_HEAD ? job == 0 : !live) continue;
-                if (half >= HEAD_SPLIT) continue;                            // (with three warps the third has no head chunk)
-                const uint32_t hj = job - QS_RO_DEFER_HEAD, hpar = hj & 1u;
+                if (DEFER_HEAD ? job == 0 : !live) continue;
+                const uint32_t hj = job - DEFER_HEAD, hpar = hj & 1u;
                 const int net = (int)(hj & 1u);
                 const uint32_t k = hj >> 1;                                  // this slot's tile counter
                 if (!mbar_wait_bounded(c.bar(B_D3 + slot), hpar, role + B_D3 + 1)) return;
@@ -600,14 +513,11 @@ __device__ __forceinline__ void role_epilogue(const Ctx& c, int slot, int half, 
                     for (int sb = 0; sb < 4; ++sb) {
                         float y[8];
                         tanh8_from_exponents(v + 8 * sb, y);
-#if QS_RO_HEAD_SCALAR_VF
-                        if (net == 1) {                                      // the critic's head has ONE output: a scalar weight and one FFMA per activation
+                        if (HEAD_SCALAR_VF && net == 1) {                    // the critic's head has ONE output: a scalar weight and one FFMA per activation
                             const float* w1 = reinterpret_cast<const float*>(wh + 8 * sb);
 #pragma unroll
                             for (int q = 0; q < 8; ++q) o[0] = fmaf(y[q], w1[4 * q], o[0]);
-                        } else
-#endif
-                        {
+                        } else {
 #pragma unroll
                             for (int q = 0; q < 8; ++q) {
                                 const float4 w = wh[8 * sb + q];
@@ -631,7 +541,6 @@ __device__ __forceinline__ void role_epilogue(const Ctx& c, int slot, int half, 
                 // ---- E1 (first stage) or E2 of job `job`
                 if (!live) continue;
                 const bool first = stage == 0;
-                if (EPI_SPLIT == 3 && !first && half == 0) continue;         // owns no layer-2 chunk
                 if (!mbar_wait_bounded(c.bar((first ? B_D1 : B_D2) + slot), par, role + (first ? B_D1 : B_D2) + 1)) return;
                 tc_fence_after();
 #pragma unroll 1
@@ -769,10 +678,10 @@ __device__ __forceinline__ void role_env(const Ctx& c, const RoParams& p, int pa
         if (par < c.cnt && e0 < p.n) pool_load<float, VER>(sp.pool, sp.n, e0, s_nx);
     }
     // the X tile of local tile i + 2 is staged before tile i is stepped; the first iteration(s) only stage (one call site: code size)
-    // With the deferred head (QS_RO_DEFER_HEAD) the outputs of a tile appear one job later, so this warp consumes them one of its
+    // With the deferred head (DEFER_HEAD) the outputs of a tile appear one job later, so this warp consumes them one of its
     // iterations later too (LAG): staging the X tile of a later tile must not queue behind the wait for them (measured: every
     // second job stalled ~4,000 cycles for its X tile otherwise).  The X buffers are released early (by the critic's layer-1 commit).
-    constexpr int LAG = QS_RO_DEFER_HEAD ? STRIDE : 0;
+    constexpr int LAG = DEFER_HEAD ? STRIDE : 0;
     RO_TRACE_INIT();
 #pragma unroll 1
     for (int j = par - 2; j < c.cnt + LAG; j += STRIDE) {

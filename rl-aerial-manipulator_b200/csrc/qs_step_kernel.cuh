@@ -75,21 +75,9 @@ constexpr int STEP_BLOCK = 128;
 // 65.2 / 72.4 us; prefetch 2/3/4/5 CTAs: 62.2 / 54.6 / 60.0 / 68.9 us (5: spills).  The kernel is half issue (~26 us of
 // instructions per SM), half HBM latency: what it needs is loads in flight, not resident warps.
 // float64 and LSODA need the registers more than the occupancy.
-#ifndef QS_STEP_MINB_F32
-#define QS_STEP_MINB_F32 3
-#endif
-#ifndef QS_STEP_PREFETCH_F32
-#define QS_STEP_PREFETCH_F32 1
-#endif
 template <typename Real, int INTEG> struct StepOcc { static constexpr int MINB = 1; static constexpr bool PREFETCH = false; };
-#ifndef QS_STEP_MINB_F64
-#define QS_STEP_MINB_F64 3
-#endif
-#ifndef QS_STEP_PREFETCH_F64
-#define QS_STEP_PREFETCH_F64 0
-#endif
-template <> struct StepOcc<double, 0> { static constexpr int MINB = QS_STEP_MINB_F64; static constexpr bool PREFETCH = QS_STEP_PREFETCH_F64 != 0; };
-template <> struct StepOcc<float, 0> { static constexpr int MINB = QS_STEP_MINB_F32; static constexpr bool PREFETCH = QS_STEP_PREFETCH_F32 != 0; };
+template <> struct StepOcc<double, 0> { static constexpr int MINB = 3; static constexpr bool PREFETCH = false; };
+template <> struct StepOcc<float, 0> { static constexpr int MINB = 3; static constexpr bool PREFETCH = true; };
 
 // Row-major [32, OBS] tile of one warp -> global, 128 bits per lane per store.
 template <int OBS>
@@ -164,18 +152,6 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
             if (wn < n_warp_tiles && lane < N_DYN * LINES)
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(p.dyn + (lane / LINES) * p.dyn_stride + wn * 32 + (lane % LINES) * (128 / (int)sizeof(Real))));
         }
-#ifdef QS_STEP_L2_PREFETCH          // A/B: no register prefetch, but the next tile's record and actions are pulled into L2
-        if (!PREFETCH) {
-            using L = PoolLayout<Real, VER>;
-            const int64_t wn = wt + warps_total;
-            if (wn < n_warp_tiles) {
-                constexpr int LINES = (L::TILE_BYTES + 127) / 128;
-                const unsigned char* rec = reinterpret_cast<const unsigned char*>(p.pool) + wn * (int64_t)L::TILE_BYTES;
-                for (int l = lane; l < LINES; l += 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(rec + l * 128));
-                if (lane < 4) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const unsigned char*>(p.actions + wn * 128) + lane * 128));
-            }
-        }
-#endif
         if (live) {
             if (!PREFETCH) {
                 pool_load<Real, VER>(p.pool, p.n, e, s);
@@ -270,188 +246,6 @@ __global__ void __launch_bounds__(STEP_BLOCK, StepOcc<Real, INTEG>::MINB) env_st
             double a = 0.0;
 #pragma unroll
             for (int w = 0; w < STEP_BLOCK / 32; ++w) a += s_mom[w][threadIdx.x];
-            p.mom_partial[(int64_t)blockIdx.x * 2 * OBS + threadIdx.x] = a;
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------------------
-// float32 / RK4 throughput kernel with a TMA-fed shared-memory pipeline.
-//
-// Same per-env body as env_step_kernel, but the hidden state and the action of a warp tile (32 envs: NVEC x 512 B planes,
-// the tail plane, 512 B of actions) are brought in by cp.async.bulk (UBLKCP) into a per-warp ring of STAGES tiles, each
-// guarded by its own mbarrier.  The copies of the next STAGES-1 tiles are always in flight while the current one is
-// integrated, without holding them in registers -- env_step_kernel needs ~100 B per lane in flight to cover the ~1 us HBM
-// latency and measured 0.74 of the copy bandwidth; register double-buffering got 0.79 at 159 registers.
-//
-// MEASURED SLOWER than the register-prefetch kernel (1M envs: 2 stages x 4/5/6 CTAs = 61.5 / 62.7 / 65.7 us vs 54.6 us): seven
-// 512-byte bulk copies per tile issued by one lane, an mbarrier wait and a shared-memory round trip cost more than they
-// hide.  Kept as an opt-in (QS_STEP_F32_TMA=1) with its own parity test so the comparison stays reproducible.
-// ------------------------------------------------------------------------------------------------------------------
-#ifndef QS_TMA_STAGES
-#define QS_TMA_STAGES 2
-#endif
-constexpr int TMA_STAGES = QS_TMA_STAGES;   // tiles in flight per warp (incl. the current one); A/B in profiles/r01/README.md
-
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
-        "@P1 bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t"
-        "}\n" ::"r"(bar), "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
-
-template <int VER>
-struct TmaStage {
-    using L = PoolLayout<float, VER>;
-    static constexpr int ACT_OFF = L::NVEC * 512 + L::NTAIL * 128;
-    static constexpr int BYTES = ACT_OFF + 512;
-};
-
-// lane 0 of a warp: request tile `wt` (rows valid envs) into `stage`
-template <int VER>
-__device__ __forceinline__ void tma_request(const StepParams<float>& p, int64_t wt, unsigned char* stage, uint64_t* bar) {
-    using L = PoolLayout<float, VER>;
-    const int64_t e0 = wt * 32;
-    const int64_t rem = p.n - e0;
-    const uint32_t rows = rem < 32 ? (uint32_t)rem : 32u;
-    const uint32_t vbytes = rows * 16u;
-    const uint32_t b = smem_addr(bar), d = smem_addr(stage);
-    mbar_expect_tx(b, (uint32_t)L::TILE_BYTES + vbytes);
-    const unsigned char* base = reinterpret_cast<const unsigned char*>(p.pool);
-    bulk_g2s(d, base + wt * (int64_t)L::TILE_BYTES, (uint32_t)L::TILE_BYTES, b);     // the whole tile record is one contiguous block
-    bulk_g2s(d + TmaStage<VER>::ACT_OFF, p.actions + e0 * 4, vbytes, b);
-}
-
-template <int VER, bool MOMENTS>
-__global__ void __launch_bounds__(STEP_BLOCK, 4) env_step_tma_kernel(const StepParams<float> p) {
-    using Real = float;
-    constexpr int OBS = EnvTraits<VER>::OBS;
-    constexpr int WARPS = STEP_BLOCK / 32;
-    constexpr int SB = TmaStage<VER>::BYTES;
-    __shared__ __align__(128) unsigned char s_stage[WARPS][TMA_STAGES][SB];
-    __shared__ __align__(8) uint64_t s_bar[WARPS][TMA_STAGES];
-    __shared__ float s_tile[WARPS][32 * (OBS + 1)];
-    __shared__ double s_mom[MOMENTS ? WARPS : 1][2 * OBS];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t warps_total = (int64_t)gridDim.x * WARPS;
-    const int64_t n_warp_tiles = (p.n + 31) / 32;
-    float* tile = s_tile[warp];
-    double m1 = 0.0, m2 = 0.0, G = 0.0;
-    if (MOMENTS && lane < OBS) {
-        if (p.mom_prev && p.mom_prev[0] > 0.0) G = p.mom_prev[1 + lane];
-        else if (p.mom_stats) G = p.mom_stats[1 + lane];
-    }
-    const int64_t wt0 = (int64_t)blockIdx.x * WARPS + warp;
-    if (lane == 0) {
-#pragma unroll
-        for (int st = 0; st < TMA_STAGES; ++st) mbar_init(smem_addr(&s_bar[warp][st]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#pragma unroll
-        for (int st = 0; st < TMA_STAGES; ++st)
-            if (wt0 + st * warps_total < n_warp_tiles) tma_request<VER>(p, wt0 + st * warps_total, s_stage[warp][st], &s_bar[warp][st]);
-    }
-    __syncwarp();
-
-    int it = 0;
-    for (int64_t wt = wt0; wt < n_warp_tiles; wt += warps_total, ++it) {
-        const int st = it % TMA_STAGES;
-        const uint32_t parity = (uint32_t)(it / TMA_STAGES) & 1u;
-        const int64_t e0 = wt * 32;
-        const int64_t e = e0 + lane;
-        const bool live = e < p.n;
-        mbar_wait_parity(smem_addr(&s_bar[warp][st]), parity);
-        EnvState<Real, VER> s;
-        float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (live) {
-            pool_load_staged<Real, VER>(s_stage[warp][st], lane, s);
-            a4 = *reinterpret_cast<const float4*>(s_stage[warp][st] + TmaStage<VER>::ACT_OFF + lane * 16);
-        }
-        __syncwarp();                                   // every lane has its tile in registers: the stage can be refilled
-        if (lane == 0 && wt + (int64_t)TMA_STAGES * warps_total < n_warp_tiles)
-            tma_request<VER>(p, wt + (int64_t)TMA_STAGES * warps_total, s_stage[warp][st], &s_bar[warp][st]);
-        float obs[OBS];
-        if (live) {
-            const float act[4] = {a4.x, a4.y, a4.z, a4.w};
-            Real Fcmd, Mcmd[3], F, M[3];
-            scale_action<Real>(p.model, act, p.scale_f32, Fcmd, Mcmd);
-            mix_and_clamp<Real>(p.model, Fcmd, Mcmd, F, M);
-            rk4_step<Real>(p.model, s.y, F, M, p.substeps);
-            renormalise_quat<Real>(s.y);
-            Real reward;
-            int ep_len;
-            const uint32_t flags = step_logic<Real, VER>(s, reward, ep_len);
-            s.ep_ret += reward;
-            make_obs<Real, VER>(s, p.obs_scaled, obs);
-            p.reward_out[e] = reward;
-            p.flags_out[e] = (uint8_t)flags;
-            if (flags & (FLAG_TERMINATED | FLAG_TRUNCATED)) {
-                if (p.term_obs_out) {
-                    float* row = p.term_obs_out + e * OBS;
-#pragma unroll
-                    for (int i = 0; i < OBS; ++i) row[i] = obs[i];
-                }
-                if (p.ep_ret_out) p.ep_ret_out[e] = s.ep_ret;
-                if (p.ep_len_out) p.ep_len_out[e] = ep_len;
-                if (p.auto_reset) {
-                    s.episode += 1;
-                    reset_env<Real, VER>(s, p.rc, p.seed, (uint64_t)(p.env_id_offset + e));
-                    make_obs<Real, VER>(s, p.obs_scaled, obs);
-                }
-            }
-            pool_store<Real, VER>(p.pool, p.n, e, s);
-#pragma unroll
-            for (int i = 0; i < OBS; ++i) tile[lane * (OBS + 1) + i] = obs[i];
-        }
-        __syncwarp();
-        const int64_t rem = p.n - e0;
-        const int rows = rem < 32 ? (int)rem : 32;
-        warp_store_rows<OBS>(p.obs_out + e0 * OBS, tile, lane, rows);
-        if (MOMENTS && lane < OBS) {
-            const float Lc = tile[lane];
-            double t1 = 0.0, t2 = 0.0;
-#pragma unroll
-            for (int r0 = 0; r0 < 32; r0 += 8) {
-                float a1 = 0.f, a2 = 0.f;
-#pragma unroll
-                for (int r = r0; r < r0 + 8; ++r) {
-                    const float v = r < rows ? tile[r * (OBS + 1) + lane] - Lc : 0.f;
-                    a1 += v;
-                    a2 = fmaf(v, v, a2);
-                }
-                t1 += (double)a1;
-                t2 += (double)a2;
-            }
-            const double dl = (double)Lc - G;
-            m1 += t1 + (double)rows * dl;
-            m2 += t2 + 2.0 * dl * t1 + (double)rows * dl * dl;
-        }
-        __syncwarp();
-    }
-    if (MOMENTS) {
-        if (lane < OBS) { s_mom[warp][lane] = m1; s_mom[warp][OBS + lane] = m2; }
-        __syncthreads();
-        if (threadIdx.x < 2 * OBS) {
-            double a = 0.0;
-#pragma unroll
-            for (int w = 0; w < WARPS; ++w) a += s_mom[w][threadIdx.x];
             p.mom_partial[(int64_t)blockIdx.x * 2 * OBS + threadIdx.x] = a;
         }
     }

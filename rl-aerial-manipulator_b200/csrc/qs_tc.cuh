@@ -1,4 +1,4 @@
-// qs_tc.cuh -- tcgen05 / TMEM / mbarrier helpers and the MlpPolicy operand layouts shared by the policy-forward kernels
+// qs_tc.cuh -- tcgen05 / TMEM / mbarrier helpers and the MlpPolicy operand layouts shared by the policy-forward kernel
 // (qs_policy_tc.cu) and the fused rollout kernel (qs_rollout.cu).  sm_100a only.
 #pragma once
 #include <cuda_fp16.h>
@@ -8,7 +8,7 @@
 namespace qs {
 namespace tc {
 
-constexpr int ROWS = 128, GROUPS = 2, GROUP_THREADS = 2 * ROWS, THREADS = GROUP_THREADS * GROUPS;   // two threads per env row
+constexpr int ROWS = 128;
 constexpr int K1 = 32;
 constexpr int N1 = 128, N2 = 64, N3 = 64, NACT = 4;
 // B operands carry the bias as one extra input: layer 1 uses the spare padding column k = OBS of X (set to 1.0); layers 2/3
@@ -20,7 +20,6 @@ constexpr int OFF_W1 = 0, OFF_W2 = 2 * W1_BYTES, OFF_W3 = OFF_W2 + 2 * W2_BYTES;
 constexpr int C_B1 = 0, C_B2 = C_B1 + 2 * N1, C_B3 = C_B2 + 2 * N2, C_WH = C_B3 + 2 * N3, C_BH = C_WH + 2 * N3 * NACT,
               C_LS = C_BH + 2 * NACT, C_TOTAL = C_LS + NACT;
 constexpr int TMEM_COLS = 512;
-constexpr uint32_t COL_R1 = 0, COL_R2 = 128, COL_ONE = 192, COL_X = 224;
 
 struct Blob {
     int obs;
@@ -125,137 +124,37 @@ __device__ __forceinline__ float tanh_mufu(float x) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-// u = 2*log2(e)*x (the scale lives in the weights): tanh(x) = 1 - 2/(2^u + 1).  ex2.approx/rcp.approx, abs error ~1e-7;
-// u -> +inf gives 1, u -> -inf gives -1 without branches.
-__device__ __forceinline__ float tanh_from_exponent(float u) {
-    float t, r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(u));
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(t + 1.0f));
-    return fmaf(-2.0f, r, 1.0f);
-}
-// Four tanh on one MUFU.RCP: with a_i = 2^min(u_i,30) + 1 (tanh is 1.0f to the last bit beyond u = 30, and the clamp keeps
-// the product of four below 2^124), 1/a = (b*c*d) / (a*b*c*d).  5 MUFU per 4 elements instead of 8; the extra FMULs run on the
-// FMA pipe, which the epilogue leaves idle.  Error: ~3 ulp of 1/a <= 2e-7 absolute.
-#ifndef QS_TC_RCP_SHARE
-#define QS_TC_RCP_SHARE 4
-#endif
-// 2^u on the FMA pipe (Cody-Waite: n = round(u) by the 1.5 * 2^23 trick, degree-5 minimax of 2^f on [-0.5, 0.5], exponent added as an
-// integer).  u is clamped to [-126, 126].  Experimental (QS_X_POLY = how many of every four exponentials take this route).
-__device__ __forceinline__ float ex2_poly(float u) {
-    u = fminf(fmaxf(u, -126.0f), 126.0f);
-    const float magic = 12582912.0f;                       // 1.5 * 2^23
-    const float nf = u + magic;
-    const float f = u - (nf - magic);
-    float pz = 1.3333558146e-3f;
-    pz = fmaf(pz, f, 9.6181291076e-3f);
-    pz = fmaf(pz, f, 5.5504108665e-2f);
-    pz = fmaf(pz, f, 2.4022650696e-1f);
-    pz = fmaf(pz, f, 6.9314718056e-1f);
-    pz = fmaf(pz, f, 1.0f);
-    return __int_as_float(__float_as_int(pz) + (__float_as_int(nf) << 23));
-}
-// QS_TC_TANH_SAT (r02): the clamp, the +1 and a power-of-two scale in ONE instruction: a_i' = sat(2^u_i * s + s) = min(2^u_i + 1, 2^31) * s
+// Four tanh on one MUFU.RCP.  u_i = 2*log2(e)*x_i (the scale lives in the weights): tanh(x) = 1 - 2/a with a = 2^u + 1, and
+// 1/a = (b*c*d) / (a*b*c*d): 5 MUFU per 4 elements instead of 8; the extra FMULs run on the FMA pipe, which the epilogue leaves
+// idle.  Error: ~3 ulp of 1/a <= 2e-7 absolute.
+// The clamp, the +1 and a power-of-two scale are ONE instruction (r02): a_i' = sat(2^u_i * s + s) = min(2^u_i + 1, 2^31) * s
 // with s = 2^-31 (FFMA.SAT; exact scaling, the same rounding as the add), so a_i' lies in [2^-31, 1], the product of four in
 // [2^-124, 1] (no overflow, no flush), and beyond 2^u + 1 = 2^31 tanh is 1.0f to the last bit anyway.  The scale comes back with
-// the -2 of tanh = 1 - 2/a: 1/a_i = s / a_i'.  19 instructions per four activations instead of 23 (MIN and FADD gone).
+// the -2 of tanh = 1 - 2/a: 1/a_i = s / a_i'.  19 instructions per four activations instead of 23 for an explicit min and FADD.
 // A NaN exponent leaves the group non-finite (sat flushes NaN to 0 -> 1/0), which the next layer's MMAs spread over the row.
-#ifndef QS_TC_TANH_SAT
-#define QS_TC_TANH_SAT 1
-#endif
 __device__ __forceinline__ void tanh4_from_exponents(const uint32_t* v, float* y) {
     float a[4];
-#if QS_TC_TANH_SAT
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         float t;
-#if defined(QS_X_NOEX2)                      // timing experiments only (wrong numerics): what the XU pipe costs
-        t = __uint_as_float(v[i]) * 0.001f;
-#elif defined(QS_X_POLY)
-        if (i < QS_X_POLY) t = ex2_poly(__uint_as_float(v[i])); else
         asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(__uint_as_float(v[i])));
-#else
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(__uint_as_float(v[i])));
-#endif
         asm("fma.rn.ftz.sat.f32 %0, %1, %2, %2;" : "=f"(a[i]) : "f"(t), "f"(4.656612873077393e-10f));     // 2^-31
     }
     const float p = a[0] * a[1], q = a[2] * a[3];
     float r;
-#ifdef QS_X_NORCP
-    r = p * q * 0.37f;
-#else
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(p * q));
-#endif
     r *= -9.313225746154785e-10f;            // -2 s = -2^-30
-#else
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        float t, u;
-        asm("min.NaN.f32 %0, %1, %2;" : "=f"(u) : "f"(__uint_as_float(v[i])), "f"(30.0f));   // NaN stays NaN, like torch
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(u));
-        a[i] = t + 1.0f;
-    }
-    const float p = a[0] * a[1], q = a[2] * a[3];
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(p * q));
-    r *= -2.0f;
-#endif
     const float rp = r * q, rq = r * p;      // -2/(a0 a1), -2/(a2 a3)
     y[0] = fmaf(rp, a[1], 1.0f);
     y[1] = fmaf(rp, a[0], 1.0f);
     y[2] = fmaf(rq, a[3], 1.0f);
     y[3] = fmaf(rq, a[2], 1.0f);
 }
-// Eight tanh on one MUFU.RCP (r02): two groups of four as above, each group's product P (in [2^-124, 1]) lifted by 2^62 into
-// [2^-62, 2^62] so that the product of both stays inside [2^-124, 2^124]; 1/P_a = P_b * rcp(P_a P_b).  A MUFU costs ~4.75 issue
-// cycles in this instruction mix on B200 and an FMUL ~0.54 (profiles/r02/pipe_rates_b200.txt), so trading half a reciprocal per four
-// activations for 2.5 multiplications should pay -- measured: 279.3 vs 279.7 us per 1M-env launch on one box, i.e. nothing, for one
-// more rounding on the way to 1/a (<= ~6e-7 absolute on tanh instead of ~2e-7).  Off by default (QS_TC_RCP8=1 builds it).
-#ifndef QS_TC_RCP8
-#define QS_TC_RCP8 0
-#endif
+// Eight tanh as two groups of four.  One MUFU.RCP for all eight (each group's product lifted by 2^62 so that both fit one float)
+// measured 279.3 vs 279.7 us per 1M-env launch on B200 (r02), i.e. nothing, for one more rounding on the way to 1/a.
 __device__ __forceinline__ void tanh8_from_exponents(const uint32_t* v, float* y) {
-#if QS_TC_RCP8 && QS_TC_TANH_SAT && !defined(QS_X_NOEX2) && !defined(QS_X_POLY) && !defined(QS_X_NORCP)
-    float a[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        float t;
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(__uint_as_float(v[i])));
-        asm("fma.rn.ftz.sat.f32 %0, %1, %2, %2;" : "=f"(a[i]) : "f"(t), "f"(4.656612873077393e-10f));     // 2^-31
-    }
-    const float p0 = a[0] * a[1], q0 = a[2] * a[3], p1 = a[4] * a[5], q1 = a[6] * a[7];
-    const float P0 = (p0 * 4.611686018427388e18f) * q0, P1 = (p1 * 4.611686018427388e18f) * q1;          // 2^62 * (a0 a1 a2 a3)
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(P0 * P1));
-    const float c = -4294967296.0f;                                   // -2 s 2^62 = -2^32
-    const float i0 = (r * P1) * c, i1 = (r * P0) * c;                 // -2 s / (a0 a1 a2 a3), -2 s / (a4 a5 a6 a7)
-    const float rp0 = i0 * q0, rq0 = i0 * p0, rp1 = i1 * q1, rq1 = i1 * p1;
-    y[0] = fmaf(rp0, a[1], 1.0f);
-    y[1] = fmaf(rp0, a[0], 1.0f);
-    y[2] = fmaf(rq0, a[3], 1.0f);
-    y[3] = fmaf(rq0, a[2], 1.0f);
-    y[4] = fmaf(rp1, a[5], 1.0f);
-    y[5] = fmaf(rp1, a[4], 1.0f);
-    y[6] = fmaf(rq1, a[7], 1.0f);
-    y[7] = fmaf(rq1, a[6], 1.0f);
-#else
     tanh4_from_exponents(v, y);
     tanh4_from_exponents(v + 4, y + 4);
-#endif
-}
-__device__ __forceinline__ void tanh2_from_exponents(const uint32_t* v, float* y) {   // A/B variant: 3 MUFU per 2 elements
-    float a[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        float t, u;
-        asm("min.NaN.f32 %0, %1, %2;" : "=f"(u) : "f"(__uint_as_float(v[i])), "f"(60.0f));
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(t) : "f"(u));
-        a[i] = t + 1.0f;
-    }
-    float r;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(a[0] * a[1]));
-    r *= -2.0f;
-    y[0] = fmaf(r, a[1], 1.0f);
-    y[1] = fmaf(r, a[0], 1.0f);
 }
 __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
     const __half2 h = __floats2half2_rn(a, b);
@@ -272,7 +171,7 @@ __device__ __forceinline__ void split_h2(float a, float b, uint32_t& hi, uint32_
 
 // weights [K][N] float32 (input-major blob) -> float16 hi (and lo) canonical B operands [N rows][KP], zero padded;
 // input index `kbias` carries the bias (its A element is the constant 1); everything is multiplied by `scale`
-template <bool PRECISE, int NT = THREADS>
+template <bool PRECISE, int NT>
 __device__ __forceinline__ void stage_weights(const float* __restrict__ w, const float* __restrict__ bias, int K, int kbias, int KP, int N,
                                               float scale, unsigned char* dst_hi, unsigned char* dst_lo, int tid) {
     for (int i = tid; i < (KP / 8) * N; i += NT) {
@@ -293,21 +192,13 @@ __device__ __forceinline__ void stage_weights(const float* __restrict__ w, const
 // one loaded 32-column accumulator chunk of this thread's row (bias already inside) -> tanh (float32 in y)
 template <bool PRECISE>
 __device__ __forceinline__ void tanh32(const uint32_t* v, float* y) {
-#ifdef QS_TC_EXPERIMENT_NO_TANH   // timing experiment only: how much of the kernel is XU work
-#pragma unroll
-    for (int i = 0; i < 32; ++i) y[i] = __uint_as_float(v[i]) * 0.001f;
-#else
-    if (PRECISE && QS_TC_RCP_SHARE == 4) {
+    if (PRECISE) {
 #pragma unroll
         for (int i = 0; i < 32; i += 4) tanh4_from_exponents(v + i, y + i);
-    } else if (PRECISE && QS_TC_RCP_SHARE == 2) {
-#pragma unroll
-        for (int i = 0; i < 32; i += 2) tanh2_from_exponents(v + i, y + i);
     } else {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) y[i] = PRECISE ? tanh_from_exponent(__uint_as_float(v[i])) : tanh_mufu(__uint_as_float(v[i]));
+        for (int i = 0; i < 32; ++i) y[i] = tanh_mufu(__uint_as_float(v[i]));
     }
-#endif
 }
 
 // y[32] -> packed float16 hi (16 columns at taddr) and, if PRECISE, lo (16 columns at taddr + 16): in place over the chunk

@@ -81,13 +81,14 @@ def unpack_params(blob: np.ndarray, obs_dim: int) -> dict:
     return sd
 
 
-IMPL = {"auto": 0, "fp32": 1, "tensor": 2, "tensor_fast": 3, "tensor_pipeline": 4, "tensor_chains": 5}
+IMPL = {"auto": 0, "fp32": 1, "tensor": 2, "tensor_fast": 3, "tensor_pipeline": 4}
 
 
 class MlpPolicyKernel:
-    """impl: "fp32" = CUDA-core FFMA kernel (float32 throughout); "tensor" = tcgen05/TMEM kernel with split-float16
-    operands (float32-level accuracy); "tensor_fast" = tcgen05/TMEM, single float16 operands + MUFU.TANH;
-    "auto" = "tensor" for batches >= 16384 envs, "fp32" below."""
+    """impl: "fp32" = CUDA-core FFMA kernel (float32 throughout); "tensor" (or its alias "tensor_pipeline") = the
+    warp-specialised tcgen05/TMEM pipeline kernel with split-float16 operands (float32-level accuracy); "tensor_fast" =
+    the three-chain tcgen05/TMEM kernel, single float16 operands + MUFU.TANH; "auto" = "tensor" for batches >= 16384 envs,
+    "fp32" below."""
 
     def __init__(self, state_dict: dict, obs_dim: int, device, impl: str = "auto"):
         self.impl = IMPL[impl]

@@ -45,6 +45,20 @@ def test_no_cpu_fallback(lib):
         BatchedQuadEnv(4)
 
 
+def test_policy_forward_rejects_an_unknown_impl(lib):
+    """impl outside QS_POLICY_AUTO..QS_POLICY_TENSOR_PIPELINE (0..4) is QS_EINVAL; the argument checks return before any
+    device memory is touched, so aligned dummy pointers suffice."""
+    from rl_aerial_manipulator_b200.policy import _bind
+    _bind(lib)
+    dummy = C.c_void_p(1 << 20)
+    box = (C.c_float * 4)()
+    for impl in (5, 6, -1):
+        rc = lib.qs_policy_forward(dummy, 20, dummy, dummy, 1, None, 1e-8, 10.0, None, dummy, dummy, C.byref(box), C.byref(box),
+                                   dummy, dummy, impl, None)
+        assert rc == -1, (impl, rc)
+        assert b"impl must be one of QS_POLICY_*" in lib.qs_policy_last_error()
+
+
 def test_config_constants_match_reference_values():
     c = qsim.make_config()
     assert c.mass == 0.18 and c.g == 9.81 and c.dt == 1 / 200

@@ -547,33 +547,6 @@ def test_config1_shipped_v1_policy_flies_the_course(golden_dir, precision, integ
     env.close()
 
 
-def test_tma_pipeline_kernel_matches_default_kernel():
-    """The opt-in TMA-fed float32 kernel (QS_STEP_F32_TMA=1) is bit-identical to the default register-prefetch kernel.
-    The switch is read once per process, so the TMA run happens in a child interpreter."""
-    import subprocess
-    import sys
-    code = (
-        "import torch, sys, os\n"
-        "sys.path.insert(0, os.getcwd())\n"
-        "from rl_aerial_manipulator_b200.batched_env import BatchedQuadEnv\n"
-        "env = BatchedQuadEnv(4099, env_version=2, precision='f32', seed=31)\n"
-        "env.reset()\n"
-        "g = torch.Generator(device='cuda').manual_seed(5)\n"
-        "acc = torch.zeros(3, dtype=torch.float64, device='cuda')\n"
-        "for t in range(150):\n"
-        "    a = torch.rand((4099, 4), device='cuda', generator=g) * torch.tensor([0.7, 2, 2, 2], device='cuda') - torch.tensor([0, 1, 1, 1.0], device='cuda')\n"
-        "    out = env.step(a.float())\n"
-        "    acc += torch.stack([out.obs.double().sum(), out.reward.double().sum(), out.flags.double().sum()])\n"
-        "print(' '.join(repr(float(x)) for x in acc))\n")
-    outs = []
-    for tma in ("0", "1"):
-        env = dict(os.environ, QS_STEP_F32_TMA=tma)
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=300)
-        assert r.returncode == 0, r.stderr[-2000:]
-        outs.append(r.stdout.strip().splitlines()[-1])
-    assert outs[0] == outs[1], outs
-
-
 def test_chunked_host_pipeline_equals_single_launch(golden_dir):
     """QuadVecEnv(pipeline_chunks=4) (qs_step_range on four streams) and predict_host(pipeline_chunks=4) return exactly what the
     single-launch paths return: sub-ranges of whole warp tiles are independent."""

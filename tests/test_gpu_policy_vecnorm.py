@@ -255,25 +255,3 @@ def test_step_kernel_merges_running_statistics_itself():
         assert abs(stats[merge][0] - (1e-4 + 25 * 20000)) < 1e-6
         env.close()
     np.testing.assert_array_equal(stats[True], stats[False])
-
-
-@pytest.mark.gpu
-def test_two_chain_policy_kernel_still_matches(golden_dir):
-    """The two-chain tcgen05 kernel (QS_POLICY_TC_CHAINS=2; the default is the three-chain one) against the same goldens:
-    the switch is read once per process, so the check runs in a child process."""
-    import subprocess, sys
-    code = (
-        "import os, numpy as np, torch\n"
-        "from rl_aerial_manipulator_b200.policy import MlpPolicyKernel\n"
-        f"z = np.load(os.path.join({golden_dir!r}, 'policy_v2.npz'))\n"
-        "for impl, ta, tv in (('tensor', 1e-4, 1e-2), ('tensor_fast', 6e-2, 20.0)):\n"
-        f"    pol = MlpPolicyKernel.from_npz(os.path.join({golden_dir!r}, 'policy_v2.npz'), device='cuda', impl=impl)\n"
-        "    obs = torch.from_numpy(np.tile(z['obs'], (40, 1))).cuda()\n"
-        "    a, v, _ = pol.forward(obs)\n"
-        "    assert np.abs(a.cpu().numpy() - np.tile(z['mean_f64'], (40, 1))).max() < ta\n"
-        "    assert np.abs(v.cpu().numpy() - np.tile(z['value_f64'], 40)).max() < tv\n"
-        "print('TWO_CHAIN_OK')\n")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", code], cwd=root, env=dict(os.environ, QS_POLICY_TC_CHAINS="2"), capture_output=True,
-                       text=True, timeout=300)
-    assert r.returncode == 0 and "TWO_CHAIN_OK" in r.stdout, (r.stdout[-1500:], r.stderr[-1500:])

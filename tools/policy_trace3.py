@@ -1,18 +1,17 @@
 """Phase timeline of the three-chain tcgen05 policy kernel (library built with -DQS_TC_TRACE):
     QS_LIB_TAG=trace QS_NVCC_DEFINES="-DQS_TC_TRACE" python -m rl_aerial_manipulator_b200._build
-    QS_LIB_PATH=.../lib/libquadsim_trace.so python tools/policy_trace3.py [tensor|tensor_fast]
+    QS_LIB_PATH=.../lib/libquadsim_trace.so python tools/policy_trace3.py
 Threads 0 (MMA issuer warp) and 32 of the three groups of CTA 0, fourth tile: clock64 stamps relative to the earliest."""
 import ctypes as C, os, sys
 sys.path.insert(0, os.getcwd())
 import numpy as np, torch
 from rl_aerial_manipulator_b200.policy import MlpPolicyKernel
 from rl_aerial_manipulator_b200._cabi import load_library
-impl = sys.argv[1] if len(sys.argv) > 1 else "tensor"
 n = 1 << 20
 g = torch.Generator(device="cuda").manual_seed(0)
 obs = torch.randn((n, 20), device="cuda", generator=g) * 0.7
 noise = torch.randn((n, 4), device="cuda", generator=g)
-pol = MlpPolicyKernel.from_npz("tests/golden/policy_v2.npz", device="cuda", impl=impl)
+pol = MlpPolicyKernel.from_npz("tests/golden/policy_v2.npz", device="cuda", impl="tensor_fast")
 for _ in range(3): pol.forward(obs, noise)
 torch.cuda.synchronize()
 lib = load_library()

@@ -1,5 +1,5 @@
 """Timing of the rollout step variants on one B200 (CUDA events around CUDA-graph replays, 1,048,576 envs by default):
-policy forward alone (chain kernel vs pipeline kernel), separate-launch rollout step, fused rollout step.
+policy forward alone (pipeline kernel), separate-launch rollout step, fused rollout step.
     python tools/rollout_time.py [n_envs] [steps]"""
 import os
 import sys
@@ -50,16 +50,17 @@ rms.attach(env, merge=True)
 gen = torch.Generator(device="cuda").manual_seed(0)
 noise = torch.randn((n, 4), device="cuda", generator=gen)
 res = {}
-for impl in ("tensor_chains", "tensor_pipeline"):
-    pol = MlpPolicyKernel.from_npz(NPZ, device="cuda", impl=impl)
-    res[f"policy {impl}"] = timed(lambda: pol.forward(env.obs, noise))
-    res[f"policy {impl} + vecnorm"] = timed(lambda: pol.forward(env.obs, noise, norm_stats=rms.stats))
-
-    def separate():
-        pol.forward(env.obs, noise, norm_stats=rms.stats)
-        env.step(pol.actions_clipped)
-    res[f"separate rollout step ({impl})"] = timed(separate)
 pol = MlpPolicyKernel.from_npz(NPZ, device="cuda", impl="tensor_pipeline")
+res["policy"] = timed(lambda: pol.forward(env.obs, noise))
+res["policy + vecnorm"] = timed(lambda: pol.forward(env.obs, noise, norm_stats=rms.stats))
+
+
+def separate():
+    pol.forward(env.obs, noise, norm_stats=rms.stats)
+    env.step(pol.actions_clipped)
+
+
+res["separate rollout step"] = timed(separate)
 for sample in ("noise", "philox"):
     fused = FusedRollout(env, pol, vecnorm=rms, sample=sample)
     res[f"fused rollout step ({sample})"] = timed((lambda: fused.step(noise)) if sample == "noise" else (lambda: fused.step()))
