@@ -434,6 +434,47 @@ int qs_step_moments_exchange(qs_handle* h, qs_xchg* x, double* stats);
 int qs_xchg_destroy(qs_xchg* x);
 const char* qs_xchg_last_error(void);
 
+/* Evaluation --------------------------------------------------------------------------------------------
+ * Replaces the episode accounting of stable_baselines3.common.evaluation.evaluate_policy(model, env, n_eval_episodes) (SB3 2.6.0;
+ * reference call site initial-implementation-v1/rl_train_vecN.py:42, `evaluate_policy(model, env, 10)`) on the device, so that an
+ * evaluation loop of qs_policy_forward (or qs_policy_forward_philox) -> qs_step -> qs_eval_record can be captured as a CUDA graph.
+ * SB3's rule: after env.reset(), env i of G records its first target(i) = (n_eval_episodes + i) // G finished episodes (Monitor's
+ * return and length), in completion order and, within one step, in env index order; the loop runs while any env is below its
+ * target.  With n_eval_episodes = q*G + r (0 <= r < G):  target(i) = q + [i >= G - r],  and env i's first output slot is
+ * base(i) = q*i + max(0, i - (G - r)).  A shard of envs [env_id_offset, env_id_offset + n) of G = n_global owns the slots
+ * [base(env_id_offset), base(env_id_offset + n)) of the whole evaluation; its output buffers hold exactly those, env e's k-th
+ * recorded episode at slot base(env_id_offset + e) - base(env_id_offset) + k.
+ *   count      i32[n]  episodes recorded per env (zeroed by qs_eval_begin)
+ *   state      i32[QS_EVAL_STATE_WORDS] device words: [0] completion step (the number of qs_eval_record calls since qs_eval_begin;
+ *              advanced by the last CTA of each launch, so graph replays count), [1] remaining = envs of the shard still below their
+ *              target (the loop is done at 0), [2] internal
+ *   flags / ep_return / ep_len   qs_step's outputs of the step just taken (ep_return f32 or f64 = the handle's precision)
+ *   ret_out f64 / len_out i32 / flags_out u8 (QS_FLAG_* of the finishing step) / step_out i32 (completion step): [slots]
+ * qs_eval_begin: zeroes count and the step word, sets remaining to the shard's envs with target > 0.
+ * qs_eval_record: once per env step, right after qs_step.  Sorting the records by (step_out, global env id) gives SB3's order.
+ */
+#define QS_EVAL_STATE_WORDS 4
+typedef struct qs_eval_args {
+    int64_t n;                /* envs of this shard */
+    int64_t env_id_offset;    /* global id of local env 0 */
+    int64_t n_global;         /* envs over all shards (G) */
+    int64_t n_eval_episodes;  /* >= 1 */
+    int32_t return_is_f64;    /* ep_return is f64 (1) or f32 (0) */
+    int32_t reserved;
+    const uint8_t* flags;
+    const void* ep_return;
+    const int32_t* ep_len;
+    int32_t* count;
+    int32_t* state;
+    double* ret_out;
+    int32_t* len_out;
+    uint8_t* flags_out;
+    int32_t* step_out;
+} qs_eval_args;
+int qs_eval_begin(const qs_eval_args* a, void* stream);
+int qs_eval_record(const qs_eval_args* a, void* stream);
+const char* qs_eval_last_error(void);
+
 /* Batched PID baseline controller ----------------------------------------------------------------------
  * Replaces `run(quad, des_state, dt)` of initial-implementation-v2/PID Controller/pid_controller.py:37-115 for all envs of a
  * handle at once: position PID -> commanded acceleration -> thrust F and desired roll/pitch; attitude PID -> moments M.

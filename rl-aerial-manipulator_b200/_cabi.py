@@ -121,6 +121,17 @@ class QsPpoHyper(C.Structure):
                 ("normalize_advantage", C.c_int32), ("reserved", C.c_int32)]
 
 
+EVAL_STATE_WORDS = 4
+
+
+class QsEvalArgs(C.Structure):
+    """qs_eval_args of include/quadsim.h."""
+    _fields_ = [("n", C.c_int64), ("env_id_offset", C.c_int64), ("n_global", C.c_int64), ("n_eval_episodes", C.c_int64),
+                ("return_is_f64", C.c_int32), ("reserved", C.c_int32),
+                ("flags", C.c_void_p), ("ep_return", C.c_void_p), ("ep_len", C.c_void_p), ("count", C.c_void_p), ("state", C.c_void_p),
+                ("ret_out", C.c_void_p), ("len_out", C.c_void_p), ("flags_out", C.c_void_p), ("step_out", C.c_void_p)]
+
+
 class QsPidGains(C.Structure):
     """qs_pid_gains of include/quadsim.h (order x, y, z, phi, theta, psi)."""
     _fields_ = [("kp", C.c_double * 6), ("kd", C.c_double * 6), ("ki", C.c_double * 6), ("max_integral", C.c_double)]
@@ -190,9 +201,12 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.qs_pid_default_gains.restype = None
     lib.qs_pid_run.argtypes = [vp, C.POINTER(QsPidGains), C.c_double] + [vp] * 8 + [i32, vp]
     lib.qs_pid_run.restype = C.c_int
+    lib.qs_eval_begin.argtypes = [C.POINTER(QsEvalArgs), vp]
+    lib.qs_eval_record.argtypes = [C.POINTER(QsEvalArgs), vp]
+    lib.qs_eval_last_error.restype = C.c_char_p
     for name in ("qs_create", "qs_destroy", "qs_obs_dim", "qs_reset", "qs_step", "qs_get_state", "qs_set_state",
                  "qs_reset_uniforms", "qs_lsoda_stats", "qs_step_moments", "qs_dynamics_randomization", "qs_get_dynamics",
-                 "qs_set_dynamics"):
+                 "qs_set_dynamics", "qs_eval_begin", "qs_eval_record"):
         getattr(lib, name).restype = C.c_int
     if lib.qs_abi_version() != QS_ABI_VERSION:
         raise RuntimeError(f"libquadsim ABI {lib.qs_abi_version()} != binding ABI {QS_ABI_VERSION}; rebuild")

@@ -417,10 +417,15 @@ class QuadPPO:
                     self.opt.update(obs, act, oldlp, adv, ret, idx)
         return {k: v for k, v in self.opt.read_stats().items()}
 
-    def learn(self, total_timesteps: int, log=None):
+    def learn(self, total_timesteps: int, log=None, callback=None):
+        """callback: an evaluation.EvalCallback (its eval/* results join the log dict), or None."""
+        if callback is not None:
+            callback.init_callback(self)
         while self.num_timesteps < total_timesteps:
             self.collect_rollouts()
             info = self.train()
+            if callback is not None:
+                info.update(callback.after_train(self))
             if log:
                 log(dict(info, timesteps=self.num_timesteps, ep_rew_mean=self.ep_rew_mean, episodes=self.ep_count))
         return self
