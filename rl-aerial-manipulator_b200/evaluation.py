@@ -1,7 +1,8 @@
 """evaluate_policy and EvalCallback on the device.
 
 Replaces stable_baselines3.common.evaluation.evaluate_policy (SB3 2.6.0; reference call site
-initial-implementation-v1/rl_train_vecN.py:42, `evaluate_policy(model, env, 10)`) and SB3's EvalCallback for QuadPPO.
+initial-implementation-v1/rl_train_vecN.py:42, `evaluate_policy(model, env, 10)`) and SB3's EvalCallback and CheckpointCallback
+for QuadPPO.
 
 Every evaluation step is three launches: the shipped policy forward (`MlpPolicyKernel.forward`, or `forward_sampled` with in-kernel
 Philox noise), the shipped env step (`BatchedQuadEnv.step` on the box-clipped actions, as SB3's `predict` clips) and
@@ -12,6 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import os
 import warnings
 from dataclasses import dataclass
 
@@ -237,21 +239,35 @@ def evaluate_policy(policy: MlpPolicyKernel, env, n_eval_episodes: int = 10, det
     return mean_reward, std_reward
 
 
+def _vec_steps(ppo) -> int:
+    return ppo.num_timesteps // (ppo.env.n_envs * ppo.world)
+
+
+def _crossed(ppo, freq: int, bucket: int):
+    """(due, new bucket): due after the first train() that crosses a multiple of `freq` vec-env steps.  SB3's callbacks fire
+    mid-rollout; here the collection is one replayed CUDA graph and is not split, so they fire after the train() that follows."""
+    b = _vec_steps(ppo) // freq
+    return b != bucket, b
+
+
 class EvalCallback:
     """stable_baselines3 EvalCallback for QuadPPO.learn(callback=...): evaluates the current policy on `eval_env` (a BatchedQuadEnv
     other than the training env) every `eval_freq` vec-env steps and keeps a device copy of the best parameters and VecNormalize
-    statistics by mean reward.
+    statistics by mean reward.  best_model_save_path: on every new best, also write `best_model.zip` there (QuadPPO.save: the
+    parameters and Adam state of that evaluation) and, with VecNormalize, `best_model_vecnormalize.pkl` with its statistics.
 
     Unlike SB3, which evaluates in the middle of a rollout, the evaluation runs after the first train() that crosses a multiple of
     eval_freq: the collection is one replayed CUDA graph and is not split.  The callback flies its own MlpPolicyKernel over the
     training parameter blob (no output buffer, generator or Philox counter is shared with training, so training is unchanged) and
     reads the training VecNormalize observation statistics in place (sync_envs_normalization).  Single rank only."""
 
-    def __init__(self, eval_env, eval_freq: int, n_eval_episodes: int = 10, deterministic: bool = True):
+    def __init__(self, eval_env, eval_freq: int, n_eval_episodes: int = 10, deterministic: bool = True,
+                 best_model_save_path: str | None = None):
         if int(eval_freq) < 1:
             raise ValueError("eval_freq must be >= 1")
         self.eval_env, self.eval_freq = eval_env, int(eval_freq)
         self.n_eval_episodes, self.deterministic = int(n_eval_episodes), bool(deterministic)
+        self.best_model_save_path = best_model_save_path
         self.best_mean_reward = -math.inf
         self.last_mean_reward = -math.inf
         self.evaluations: list[dict] = []
@@ -265,23 +281,20 @@ class EvalCallback:
             raise ValueError("EvalCallback is single-rank only: evaluate the shards with evaluate(..., n_global=...) instead")
         if self.eval_env.obs_dim != ppo.env.obs_dim or self.eval_env.device != ppo.env.device:
             raise ValueError("EvalCallback: eval_env differs from the training env in observation size or device")
+        if self.best_model_save_path is not None:
+            os.makedirs(self.best_model_save_path, exist_ok=True)
         if self._ppo is not ppo:
             impl = {v: k for k, v in IMPL.items()}[ppo.policy.impl]
             self.policy = MlpPolicyKernel(ppo.policy.state_dict, ppo.env.obs_dim, ppo.env.device, impl=impl)
             self.policy.params = ppo.policy.params
             self._ppo = ppo
-            self._bucket = self._vec_steps() // self.eval_freq
-
-    def _vec_steps(self) -> int:
-        ppo = self._ppo
-        return ppo.num_timesteps // (ppo.env.n_envs * ppo.world)
+            self._bucket = _vec_steps(ppo) // self.eval_freq
 
     def after_train(self, ppo) -> dict:
         """Called by QuadPPO.learn after every train(); returns the eval/* entries of the log when it evaluated, else {}."""
-        bucket = self._vec_steps() // self.eval_freq
-        if bucket == self._bucket:
+        due, self._bucket = _crossed(ppo, self.eval_freq, self._bucket)
+        if not due:
             return {}
-        self._bucket = bucket
         vn = ppo.vecnorm
         res = evaluate(self.policy, self.eval_env, self.n_eval_episodes, self.deterministic, vecnorm=vn)
         rewards = res.episode_rewards()
@@ -294,6 +307,10 @@ class EvalCallback:
             self.best_mean_reward = mean_reward
             self._best = (ppo.policy.params.clone(), vn.obs_rms.stats.clone() if vn is not None else None,
                           vn.ret_rms.stats.clone() if vn is not None else None)
+            if self.best_model_save_path is not None:
+                path = self.best_model_save_path
+                ppo.save(os.path.join(path, "best_model.zip"),
+                         vecnormalize_path=os.path.join(path, "best_model_vecnormalize.pkl") if vn is not None else None)
         return out
 
     def best_state_dict(self) -> dict:
@@ -312,3 +329,39 @@ class EvalCallback:
                       ret_mean=float(r[1]), ret_var=float(r[2]), ret_count=float(r[0]))
             out["vecnorm"] = sd
         return out
+
+
+class CheckpointCallback:
+    """stable_baselines3 CheckpointCallback for QuadPPO.learn(callback=...): after the first train() that crosses each multiple of
+    `save_freq` vec-env steps (EvalCallback's rule), writes `{name_prefix}_{num_timesteps}_steps.zip` (QuadPPO.save: every
+    checkpoint resumes exactly with QuadPPO.load) and, with save_vecnormalize and a VecNormalize,
+    `{name_prefix}_vecnormalize_{num_timesteps}_steps.pkl` into save_path.  template_zip is passed to QuadPPO.save.  Reads device
+    state only, so training is unchanged.  Single rank (QuadPPO.save)."""
+
+    def __init__(self, save_freq: int, save_path: str, name_prefix: str = "rl_model", save_vecnormalize: bool = False,
+                 template_zip: str | None = None):
+        if int(save_freq) < 1:
+            raise ValueError("save_freq must be >= 1")
+        self.save_freq, self.save_path, self.name_prefix = int(save_freq), save_path, name_prefix
+        self.save_vecnormalize, self.template_zip = bool(save_vecnormalize), template_zip
+        self._ppo = None
+
+    def _path(self, kind: str, ext: str, steps: int) -> str:
+        return os.path.join(self.save_path, f"{self.name_prefix}_{kind}{steps}_steps.{ext}")
+
+    def init_callback(self, ppo) -> None:
+        if ppo.world > 1:
+            raise ValueError("CheckpointCallback is single-rank only")
+        os.makedirs(self.save_path, exist_ok=True)
+        if self._ppo is not ppo:
+            self._ppo = ppo
+            self._bucket = _vec_steps(ppo) // self.save_freq
+
+    def after_train(self, ppo) -> dict:
+        """Called by QuadPPO.learn after every train(); saves when due.  Adds nothing to the log."""
+        due, self._bucket = _crossed(ppo, self.save_freq, self._bucket)
+        if due:
+            vn = ppo.vecnorm if self.save_vecnormalize else None
+            ppo.save(self._path("", "zip", ppo.num_timesteps), template_zip=self.template_zip,
+                     vecnormalize_path=self._path("vecnormalize_", "pkl", ppo.num_timesteps) if vn is not None else None)
+        return {}

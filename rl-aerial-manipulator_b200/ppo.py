@@ -18,12 +18,15 @@ torch is the plumbing: device buffers, streams, the epoch permutation, the NCCL 
 from __future__ import annotations
 
 import ctypes as C
+import io
+import json
 import math
 
 import numpy as np
 import torch
 import torch.distributed as dist
 
+from . import sb3_compat
 from ._cabi import QsPpoHyper, load_library
 from .policy import MlpPolicyKernel, H1, H2, H3, NACT, unpack_params
 
@@ -179,6 +182,8 @@ class QuadPPO:
         self.env, self.vecnorm = env, vecnorm
         self.n_steps, self.batch_size, self.n_epochs = n_steps, batch_size, n_epochs
         self.gamma, self.gae_lambda = gamma, gae_lambda
+        self.clip_range, self.ent_coef, self.vf_coef, self.max_grad_norm = clip_range, ent_coef, vf_coef, max_grad_norm
+        self.learning_rate, self.normalize_advantage = learning_rate, normalize_advantage
         dev, n, d = env.device, env.n_envs, env.obs_dim
         sd = state_dict or init_state_dict(d, seed)
         self.world = dist.get_world_size() if dist.is_initialized() else 1
@@ -215,6 +220,7 @@ class QuadPPO:
         self._st_rew = torch.empty(n, **f32)
         self._rec_ws = torch.zeros(2 * 1024 + 1, dtype=torch.float64, device=dev)   # qs_rollout_record_post workspace (QS_RECORD_MAX_BLOCKS)
         self.num_timesteps = 0
+        self._n_updates = 0
         self._ep_stats = torch.zeros(2, dtype=torch.float64, device=dev)
         self._zero = torch.zeros((), dtype=torch.float64, device=dev)
         self.ep_rew_mean, self.ep_count = float("nan"), 0
@@ -346,14 +352,17 @@ class QuadPPO:
             self._last_obs = env.reset()
             if vn is not None and vn.norm_obs and vn.training:
                 vn.obs_rms.update(self._last_obs)                # VecNormalize.reset() updates the statistics too
-                # from here on the step kernel reduces its own observations and, where one launch can do it (one GPU, or several over
-                # the peer-memory exchange), the kernel that finishes them also merges them into the running statistics
-                rms = vn.obs_rms
-                vn.obs_rms.attach(env, merge=(rms._gathered is None or rms.exchange == "peer"))
+                self._attach_moments()
         self._ep_stats.zero_()
         if not (self._use_graph and self._collect_graph()):
             self._collect_eager()
         self._finish_rollout()
+
+    def _attach_moments(self):
+        """From here on the step kernel reduces its own observations and, where one launch can do it (one GPU, or several over the
+        peer-memory exchange), the kernel that finishes them also merges them into the running statistics."""
+        rms = self.vecnorm.obs_rms
+        rms.attach(self.env, merge=(rms._gathered is None or rms.exchange == "peer"))
 
     def _collect_eager(self):
         env, vn = self.env, self.vecnorm
@@ -415,17 +424,21 @@ class QuadPPO:
                     self.opt.update_sharded(obs, act, oldlp, adv, ret, idx)
                 else:
                     self.opt.update(obs, act, oldlp, adv, ret, idx)
+        self._n_updates += self.n_epochs
         return {k: v for k, v in self.opt.read_stats().items()}
 
     def learn(self, total_timesteps: int, log=None, callback=None):
-        """callback: an evaluation.EvalCallback (its eval/* results join the log dict), or None."""
-        if callback is not None:
-            callback.init_callback(self)
+        """Train until num_timesteps reaches total_timesteps (SB3's learn with reset_num_timesteps=False).  callback: an
+        evaluation.EvalCallback or CheckpointCallback, a list of them (called in order after every train(); their results join
+        the log dict), or None."""
+        callbacks = [] if callback is None else list(callback) if isinstance(callback, (list, tuple)) else [callback]
+        for cb in callbacks:
+            cb.init_callback(self)
         while self.num_timesteps < total_timesteps:
             self.collect_rollouts()
             info = self.train()
-            if callback is not None:
-                info.update(callback.after_train(self))
+            for cb in callbacks:
+                info.update(cb.after_train(self))
             if log:
                 log(dict(info, timesteps=self.num_timesteps, ep_rew_mean=self.ep_rew_mean, episodes=self.ep_count))
         return self
@@ -433,3 +446,128 @@ class QuadPPO:
     def state_dict(self) -> dict:
         """SB3-named policy parameters (feed to sb3_compat.save_policy_zip)."""
         return unpack_params(self.policy.params.detach().cpu().numpy(), self.env.obs_dim)
+
+    # ---- checkpoints ---------------------------------------------------------------------------------
+    HYPER = ("n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "clip_range", "ent_coef", "vf_coef", "max_grad_norm",
+             "learning_rate", "normalize_advantage")
+
+    def _resume_config(self) -> dict:
+        """What the exact-resume state depends on besides the hyper-parameters: the env's configuration and the VecNormalize mode."""
+        env, c, vn = self.env, self.env.cfg, self.vecnorm
+        return {"env_version": env.env_version, "precision": env.precision, "integrator": env.integrator, "substeps": int(c.substeps),
+                "obs_scaled": bool(c.obs_scaled), "action_scale_f32": bool(c.action_scale_f32), "auto_reset": bool(c.auto_reset),
+                "n_envs": env.n_envs, "env_id_offset": int(c.env_id_offset), "seed": env.seed,
+                "v2_random_waypoints": bool(c.v2_random_waypoints),
+                "dynamics_randomization": json.loads(json.dumps(env.dynamics_randomization, sort_keys=True)),
+                "vecnorm": None if vn is None else {"norm_obs": bool(vn.norm_obs), "norm_reward": bool(vn.norm_reward), "training": bool(vn.training)}}
+
+    def _resume_bytes(self) -> bytes:
+        """Every piece of device and host state that crosses an iteration boundary, as an .npz (see DESIGN "Checkpoints and resume")."""
+        env, vn = self.env, self.vecnorm
+        host = lambda t: t.detach().cpu().numpy()
+        m, v, step = self.opt.adam_state()
+        a = {"config": np.array(json.dumps(self._resume_config(), sort_keys=True)), "params": host(self.policy.params), "adam_m": host(m),
+             "adam_v": host(v), "adam_step": host(step), "generator": self.gen.get_state().numpy(),
+             "progress": np.array([self.num_timesteps, self.ep_count, self._n_updates], np.int64), "ep_rew_mean": np.float64(self.ep_rew_mean)}
+        if self._last_obs is not None:                       # collection has started: the env is mid-episode
+            a.update({f"env.{k}": host(t) for k, t in env.get_state().items()})
+            a["env_obs"], a["last_dones"] = host(env.obs), host(self._last_dones)
+            if env.dynamics_randomization is not None:
+                a["dynamics"] = host(env._dyn_rows())
+        if vn is not None:
+            a["obs_rms"], a["ret_rms"], a["returns"] = host(vn.obs_rms.stats), host(vn.ret_rms.stats), host(vn.returns)
+            if self._last_obs is not None and vn.norm_obs and vn.training:
+                a["obs_moments"] = host(vn.obs_rms._moments)
+        buf = io.BytesIO()
+        np.savez(buf, **a)
+        return buf.getvalue()
+
+    def _restore(self, a) -> None:
+        """Inverse of _resume_bytes on a freshly built QuadPPO: no env.reset(), no statistics update."""
+        want, have = json.loads(str(a["config"])), self._resume_config()
+        for k in want:
+            if want[k] != have.get(k):
+                raise ValueError(f"checkpoint was saved with {k} = {want[k]!r}, this env has {have.get(k)!r} "
+                                 "(resume_env_state=False resumes with a fresh env reset instead)")
+        env, vn = self.env, self.vecnorm
+        dev = lambda x: torch.from_numpy(np.asarray(x)).to(env.device)
+        m, v, step = self.opt.adam_state()
+        self.policy.params.copy_(dev(a["params"]))
+        m.copy_(dev(a["adam_m"]))
+        v.copy_(dev(a["adam_v"]))
+        step.copy_(dev(a["adam_step"]))
+        self.gen.set_state(torch.from_numpy(a["generator"]))
+        self.num_timesteps, self.ep_count, self._n_updates = (int(x) for x in a["progress"])
+        self.ep_rew_mean = float(a["ep_rew_mean"])
+        if vn is not None:
+            vn.obs_rms.stats.copy_(dev(a["obs_rms"]))
+            vn.ret_rms.stats.copy_(dev(a["ret_rms"]))
+            vn.returns.copy_(dev(a["returns"]))
+        if "env_obs" not in a:
+            return                                           # saved before the first collection: it resets the env as usual
+        env.set_state(**{k[4:]: a[k] for k in a.files if k.startswith("env.")})
+        if "dynamics" in a:                                  # after the pool: arming drew parameters for the episodes it found
+            d = a["dynamics"]
+            env.set_dynamics(mass_scale=d[:, 0], inertia_scale=d[:, 1], thrust_scale=d[:, 2:6], wind=d[:, 6:9])
+        env.obs.copy_(dev(a["env_obs"]))
+        self._last_dones.copy_(dev(a["last_dones"]))
+        self._last_obs = env.obs
+        if "obs_moments" in a:
+            self._attach_moments()                           # as collect_rollouts does after its first reset ...
+            vn.obs_rms._moments.copy_(dev(a["obs_moments"]))  # ... but centred where the interrupted run's next step would centre
+        torch.cuda.synchronize(env.device)
+
+    def save(self, path: str, template_zip: str | None = None, vecnormalize_path: str | None = None) -> None:
+        """model.save(path): an SB3 2.6.0 model zip (sb3_compat.save_model_zip) with the policy, the Adam state as
+        policy.optimizer.pth and the plain hyper-parameters in `data`, plus the exact-resume member (sb3_compat.RESUME_MEMBER)
+        that QuadPPO.load uses to continue bit for bit.  template_zip: an SB3 zip whose pickled `data` entries are kept (see
+        save_model_zip).  vecnormalize_path: also write the VecNormalize statistics as an SB3 vec_normalize.pkl.  Single rank."""
+        if self.world > 1:
+            raise ValueError("QuadPPO.save is single-rank only")
+        if vecnormalize_path is not None and self.vecnorm is None:
+            raise ValueError("vecnormalize_path given, but this QuadPPO has no VecNormalize")
+        torch.cuda.synchronize(self.env.device)
+        d = self.env.obs_dim
+        m, v, step = (t.cpu().numpy() for t in self.opt.adam_state())
+        opt_sd = sb3_compat.blobs_to_adam_state(m, v, int(step[0]), d, self.learning_rate)
+        data = {"num_timesteps": int(self.num_timesteps), "_n_updates": int(self._n_updates)}
+        for k in self.HYPER:
+            val = getattr(self, k)
+            data[k] = bool(val) if k == "normalize_advantage" else int(val) if k in ("n_steps", "batch_size", "n_epochs") else float(val)
+        sb3_compat.save_model_zip(path, self.state_dict(), opt_sd, data, template_zip, extra={sb3_compat.RESUME_MEMBER: self._resume_bytes()})
+        if vecnormalize_path is not None:
+            vn = self.vecnorm
+            sb3_compat.save_vecnormalize_pkl(vecnormalize_path, dict(vn.state_dict(), training=vn.training), self.env.n_envs, d)
+
+    @classmethod
+    def load(cls, path: str, env, vecnorm=None, resume_env_state: bool = True, **overrides) -> "QuadPPO":
+        """PPO.load(path, env): a QuadPPO on `env` with the zip's parameters, Adam state and num_timesteps; hyper-parameters from
+        the zip's `data` (plain entries; e.g. the reference's batch_size=128 is kept unless overridden), `overrides` (any QuadPPO
+        keyword) win.  When the zip carries QuadPPO.save's resume member and resume_env_state is True, training continues exactly
+        where it was saved (env, VecNormalize statistics, generator): an env whose configuration differs raises ValueError.
+        Otherwise (an SB3 zip, or resume_env_state=False) it resumes as PPO.load + learn(reset_num_timesteps=False) does: the env
+        is reset at the first collection, and VecNormalize statistics are the caller's (load_vecnormalize_pkl +
+        DeviceVecNormalize.load_state_dict).  Single rank."""
+        if dist.is_initialized() and dist.get_world_size() > 1:
+            raise ValueError("QuadPPO.load is single-rank only")
+        z = sb3_compat.read_model_zip(path)
+        data, policy_sd = z["data"], z["policy"]
+        kw = {k: data[k] for k in cls.HYPER if k in data and not isinstance(data[k], dict)}
+        kw.update(overrides)
+        ppo = cls(env, vecnorm, state_dict=policy_sd, **kw)
+        if z["optimizer"] is not None:
+            m, v, step, group = sb3_compat.adam_state_to_blobs(z["optimizer"], list(policy_sd), env.obs_dim)
+            if tuple(group.get("betas", (0.9, 0.999))) != (0.9, 0.999) or float(group.get("eps", 1e-5)) != 1e-5:
+                raise ValueError(f"optimizer has betas {group.get('betas')} and eps {group.get('eps')}; the update kernel runs "
+                                 "SB3's Adam(betas=(0.9, 0.999), eps=1e-5)")
+            dm, dv, dstep = ppo.opt.adam_state()
+            dm.copy_(torch.from_numpy(m))
+            dv.copy_(torch.from_numpy(v))
+            dstep.fill_(step)
+        ppo.num_timesteps = int(data.get("num_timesteps", 0))
+        ppo._n_updates = int(data.get("_n_updates", 0))
+        if resume_env_state and sb3_compat.RESUME_MEMBER in z["members"]:
+            with np.load(io.BytesIO(z["members"][sb3_compat.RESUME_MEMBER]), allow_pickle=False) as a:
+                ppo._restore(a)
+        torch.cuda.synchronize(env.device)
+        return ppo

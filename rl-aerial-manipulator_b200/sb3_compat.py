@@ -9,6 +9,10 @@
                             (stable_baselines3.common.vec_env.vec_normalize.VecNormalize, ...running_mean_std.RunningMeanStd,
                             gymnasium.spaces.box.Box) and the same attribute dictionary as the reference's pkl
   save_policy_zip           write an SB3 model zip by replacing `policy.pth` of a template zip (PPO.load-compatible)
+  adam_state_to_blobs /     policy.optimizer.pth (torch Adam state_dict over ActorCriticPolicy.parameters()) to and from the
+  blobs_to_adam_state       update kernel's Adam moments and step (blob layout of include/quadsim.h)
+  save_model_zip /          the whole SB3 model zip (data, policy.pth, policy.optimizer.pth, ...), used by QuadPPO.save / load
+  read_model_zip
 
 Reference call sites: initial-implementation-v1/rl_train_vecN.py:11,39 (VecNormalize(...), env.save("vec_normalize.pkl")),
 rl_checkpoint_train_vecN.py:22-28,63-64 (VecNormalize.load), runsim_vecN.py:24-26; model zips: v2/rl_train.py:33-35,
@@ -18,6 +22,7 @@ from __future__ import annotations
 
 import contextlib
 import io
+import json
 import pickle
 import sys
 import types
@@ -26,6 +31,7 @@ import zipfile
 import numpy as np
 import torch
 
+from .policy import H1, H2, H3, NACT, pack_params, unpack_params
 from .vec_env import LazyInfos, QuadVecEnv
 from .vec_normalize import DeviceVecNormalize
 
@@ -142,6 +148,162 @@ def save_policy_zip(template_zip: str, out_path: str, state_dict: dict) -> None:
     with zipfile.ZipFile(template_zip) as zin, zipfile.ZipFile(out_path, "w", zipfile.ZIP_DEFLATED) as zout:
         for item in zin.infolist():
             zout.writestr(item, buf.getvalue() if item.filename == "policy.pth" else zin.read(item.filename))
+
+
+# ---- policy.optimizer.pth: torch.optim.Adam.state_dict() over ActorCriticPolicy.parameters() ---------------------------------
+# parameters() yields the module's own parameter (log_std) first, then the submodules' in registration order; policy.pth's
+# state_dict keys come in the same order.
+SB3_PARAM_ORDER = ("log_std",) + tuple(f"mlp_extractor.{net}.{i}.{w}" for net in ("policy_net", "value_net") for i in (0, 2, 4)
+                                       for w in ("weight", "bias")) + ("action_net.weight", "action_net.bias", "value_net.weight", "value_net.bias")
+
+
+def pack_params_len(obs_dim: int) -> int:
+    """Floats in the parameter blob of include/quadsim.h (qs_policy_param_count), computed on the host."""
+    return sum(k_in * k_out + k_out for k_in, k_out in ((obs_dim, H1), (H1, H2), (H2, H3))) * 2 + 2 * (H3 * NACT + NACT) + NACT
+
+
+def _sb3_shapes(obs_dim: int) -> dict:
+    return {k: v.shape for k, v in unpack_params(np.zeros(pack_params_len(obs_dim), np.float32), obs_dim).items()}
+
+
+def adam_state_to_blobs(opt_state: dict, param_names, obs_dim: int):
+    """policy.optimizer.pth (a torch Adam state_dict) -> (m, v) float32 blobs in the layout of include/quadsim.h, the step count
+    and the first param_group without its `params`.  param_names: the parameter order (policy.pth's key order).  A state without
+    entries (an optimizer that never stepped) gives zero moments and step 0.  Raises ValueError on a parameter count or shape
+    that does not match the policy, or unequal per-parameter steps."""
+    names = list(param_names)
+    shapes = _sb3_shapes(obs_dim)
+    if sorted(names) != sorted(shapes):
+        raise ValueError(f"policy parameters {names} are not the {len(shapes)} of an SB3 MlpPolicy with {obs_dim} observations")
+    ids = [i for g in opt_state["param_groups"] for i in g["params"]]
+    if len(ids) != len(names):
+        raise ValueError(f"optimizer state covers {len(ids)} parameters, the policy has {len(names)}")
+    state = opt_state["state"]
+    if not state:
+        z = np.zeros(pack_params_len(obs_dim), np.float32)
+        return z, z.copy(), 0, {k: v for k, v in opt_state["param_groups"][0].items() if k != "params"}
+    m, v, steps = {}, {}, set()
+    for pid, name in zip(ids, names):
+        if pid not in state:
+            raise ValueError(f"optimizer state has no entry for parameter {pid} ({name})")
+        s = state[pid]
+        for key, out in (("exp_avg", m), ("exp_avg_sq", v)):
+            t = np.asarray(torch.as_tensor(s[key]).detach().cpu().float().numpy())
+            if t.shape != shapes[name]:
+                raise ValueError(f"{key} of {name}: shape {t.shape}, expected {shapes[name]}")
+            out[name] = t
+        steps.add(float(torch.as_tensor(s["step"]).item()))
+    if len(steps) != 1:
+        raise ValueError(f"optimizer state has unequal per-parameter steps {sorted(steps)}")
+    step = steps.pop()
+    if step < 0 or step != int(step):
+        raise ValueError(f"optimizer step {step} is not a non-negative integer")
+    group = {k: v for k, v in opt_state["param_groups"][0].items() if k != "params"}
+    return pack_params(m, obs_dim), pack_params(v, obs_dim), int(step), group
+
+
+def blobs_to_adam_state(m: np.ndarray, v: np.ndarray, step: int, obs_dim: int, lr: float, betas=(0.9, 0.999), eps: float = 1e-5,
+                        param_names=SB3_PARAM_ORDER) -> dict:
+    """(m, v, step) of the update kernel -> the state_dict of a real torch.optim.Adam(params, lr, betas, eps) over parameters of
+    SB3's shapes in `param_names` order: the installed torch's own format (param_groups, tensor steps)."""
+    n = pack_params_len(obs_dim)
+    m, v = np.asarray(m, np.float32), np.asarray(v, np.float32)
+    if m.shape != (n,) or v.shape != (n,):
+        raise ValueError(f"Adam moments must be float32[{n}], got {m.shape} and {v.shape}")
+    shapes = _sb3_shapes(obs_dim)
+    names = list(param_names)
+    if sorted(names) != sorted(shapes):
+        raise ValueError(f"param_names {names} are not the {len(shapes)} parameters of an SB3 MlpPolicy")
+    params = [torch.nn.Parameter(torch.zeros(shapes[k])) for k in names]
+    opt = torch.optim.Adam(params, lr=lr, betas=tuple(betas), eps=eps)
+    if int(step) > 0:
+        for p in params:
+            p.grad = torch.zeros_like(p)
+        opt.step()                                   # lets torch create its per-parameter state in its own format
+        sm, sv = unpack_params(m, obs_dim), unpack_params(v, obs_dim)
+        with torch.no_grad():
+            for p, k in zip(params, names):
+                st = opt.state[p]
+                st["step"].fill_(int(step))
+                st["exp_avg"].copy_(torch.from_numpy(sm[k]))
+                st["exp_avg_sq"].copy_(torch.from_numpy(sv[k]))
+    elif m.any() or v.any():
+        raise ValueError("Adam step 0 with nonzero moments")
+    return opt.state_dict()
+
+
+# ---- model zip ------------------------------------------------------------------------------------------------------------
+SB3_VERSION = "2.6.0"
+# `data` entries SB3 2.6.0 stores as plain JSON (not cloudpickled); clip_range is a pickled schedule in SB3's own zips and a
+# float in the ones written here
+PLAIN_DATA_FIELDS = ("num_timesteps", "_n_updates", "n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "ent_coef", "vf_coef",
+                     "max_grad_norm", "learning_rate", "normalize_advantage", "clip_range")
+# The exact-resume state (QuadPPO.save).  Not a .pth member: SB3's load_from_zip_file hands every *.pth member to set_parameters,
+# which rejects unknown names; other members are ignored.
+RESUME_MEMBER = "quadppo_resume.npz"
+
+
+def _torch_bytes(obj) -> bytes:
+    buf = io.BytesIO()
+    torch.save(obj, buf)
+    return buf.getvalue()
+
+
+def _system_info() -> str:
+    import platform
+    return (f"- OS: {platform.platform()} {platform.version()}\n- Python: {platform.python_version()}\n- Stable-Baselines3: {SB3_VERSION}\n"
+            f"- PyTorch: {torch.__version__}\n- GPU Enabled: {torch.cuda.is_available()}\n- Numpy: {np.__version__}\n")
+
+
+def save_model_zip(path: str, state_dict: dict, optimizer_state: dict, data: dict, template_zip: str | None = None,
+                   extra: dict | None = None) -> None:
+    """Write an SB3 2.6.0 model zip: data, policy.pth, policy.optimizer.pth, pytorch_variables.pth, _stable_baselines3_version,
+    system_info.txt, plus the `extra` members {name: bytes} (stored uncompressed).  policy.pth is written in SB3's parameter order
+    (SB3_PARAM_ORDER), which is also the order of the optimizer state; state_dict must hold exactly those parameters.
+
+    template_zip: an SB3 zip whose members are kept: of its `data`, only the entries of PLAIN_DATA_FIELDS that are plain JSON there
+    (or absent) are replaced -- pickled entries (policy_class, spaces, schedules) stay as they are -- and the two .pth members are
+    replaced.  The result is then as PPO.load-compatible as save_policy_zip's output.  Without a template, `data` holds the plain
+    fields only; whether SB3's PPO.load accepts such a zip (it reads policy_class and the spaces from `data`) is unverified."""
+    members = {}
+    if template_zip is not None:
+        with zipfile.ZipFile(template_zip) as zin:
+            members = {i.filename: zin.read(i.filename) for i in zin.infolist()}
+        d = json.loads(members["data"])
+        for k, val in data.items():
+            if not isinstance(d.get(k), dict):
+                d[k] = val
+    else:
+        d = dict(data)
+        members["pytorch_variables.pth"] = _torch_bytes({})
+        members["_stable_baselines3_version"] = SB3_VERSION.encode()
+        members["system_info.txt"] = _system_info().encode()
+    members["data"] = json.dumps(d, indent=4).encode()
+    if sorted(state_dict) != sorted(SB3_PARAM_ORDER):
+        raise ValueError(f"state_dict keys {sorted(state_dict)} are not the parameters of an SB3 MlpPolicy")
+    # SB3's key order (log_std first), whatever the caller's dict order: readers take the optimizer's parameter order from it
+    members["policy.pth"] = _torch_bytes({k: torch.as_tensor(np.asarray(state_dict[k])) for k in SB3_PARAM_ORDER})
+    members["policy.optimizer.pth"] = _torch_bytes(optimizer_state)
+    order = ["data", "policy.pth", "policy.optimizer.pth", "pytorch_variables.pth", "_stable_baselines3_version", "system_info.txt"]
+    names = [k for k in order if k in members] + [k for k in members if k not in order]
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_DEFLATED) as z:
+        for k in names:
+            z.writestr(k, members[k])
+        for k, b in (extra or {}).items():
+            z.writestr(k, b, compress_type=zipfile.ZIP_STORED)
+
+
+def read_model_zip(path: str) -> dict:
+    """An SB3 model zip -> {"data": the JSON dict (pickled entries left as SB3's {":type:", ":serialized:"} dicts),
+    "policy": policy.pth as an ordered dict of float32 arrays, "optimizer": the policy.optimizer.pth state_dict or None,
+    "members": {name: bytes} of every other member}."""
+    with zipfile.ZipFile(path) as z:
+        raw = {i.filename: z.read(i.filename) for i in z.infolist()}
+    load = lambda b: torch.load(io.BytesIO(b), weights_only=True, map_location="cpu")
+    policy = {k: v.detach().float().numpy() for k, v in load(raw.pop("policy.pth")).items()}
+    opt = raw.pop("policy.optimizer.pth", None)
+    return {"data": json.loads(raw.pop("data")) if "data" in raw else {}, "policy": policy,
+            "optimizer": load(opt) if opt is not None else None, "members": raw}
 
 
 class QuadVecNormalize:
