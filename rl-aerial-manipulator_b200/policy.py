@@ -88,7 +88,8 @@ class MlpPolicyKernel:
     """impl: "fp32" = CUDA-core FFMA kernel (float32 throughout); "tensor" (or its alias "tensor_pipeline") = the
     warp-specialised tcgen05/TMEM pipeline kernel with split-float16 operands (float32-level accuracy); "tensor_fast" =
     the three-chain tcgen05/TMEM kernel, single float16 operands + MUFU.TANH; "auto" = "tensor" for batches >= 16384 envs,
-    "fp32" below."""
+    "fp32" below.  The tensor kernels clamp each (normalised) observation to +-60,000, inside float16's range, before layer 1
+    ("fp32" does not); weights whose value times 2 log2(e) overflows float16 (|w| > ~22,700) are outside their supported range."""
 
     def __init__(self, state_dict: dict, obs_dim: int, device, impl: str = "auto"):
         self.impl = IMPL[impl]
