@@ -289,6 +289,16 @@ int qs_policy_forward_philox(const float* params, int obs_dim, const float* obs,
                              int64_t env_id_offset, const double* norm_stats, float norm_eps, float norm_clip,
                              float* obs_norm_out, float* actions, float* actions_clipped, const float* clip_lo,
                              const float* clip_hi, float* values, float* logp, void* stream);
+/* Population forward: K agents' MlpPolicy rollout forwards in ONE launch (the FFMA kernel of QS_POLICY_FP32, grid (tiles per agent,
+ * K)).  Replaces K calls of ActorCriticPolicy.forward, one per independently trained SB3 PPO model, on K consecutive row blocks
+ * of one env batch.  Agent a's CTAs load blob a and handle rows [a*n, (a+1)*n); rows are independent in the kernel (a fixed
+ * k-order per row), so every row is bit-identical to qs_policy_forward(impl = QS_POLICY_FP32) with that agent's blob.
+ *   params   f32[K][qs_policy_param_count(obs_dim)], 16-byte aligned
+ *   obs      f32[K*n, d]    noise f32[K*n, 4] or NULL    actions / actions_clipped f32[K*n, 4]    values / logp f32[K*n]
+ *   n        rows per agent; clip_lo / clip_hi as in qs_policy_forward.  No VecNormalize statistics. */
+int qs_policy_forward_pop(const float* params, int obs_dim, int K, const float* obs, const float* noise, int64_t n,
+                          float* actions, float* actions_clipped, const float* clip_lo, const float* clip_hi, float* values,
+                          float* logp, void* stream);
 const char* qs_policy_last_error(void);
 
 /* Fused rollout step -----------------------------------------------------------------------------------
@@ -406,6 +416,27 @@ int qs_ppo_apply(qs_ppo* o, float* params, const float* grad, const qs_ppo_hyper
 /* device pointers of the optimizer state (checkpointing, tests): Adam m, v f32[n_params], step i64[1], gradient buffer */
 int qs_ppo_state(qs_ppo* o, float** m, float** v, long long** step, float** grad);
 const char* qs_ppo_last_error(void);
+/* Population update: the minibatch update of K independent PPO agents in ONE launch.  Replaces one minibatch of PPO.train() of each
+ * of K SB3 PPO models that share n_steps, batch_size, n_epochs, gamma and gae_lambda but have their own parameters, Adam state and
+ * qs_ppo_hyper.  Grid (CTAs of one qs_ppo_update of B rows, K); blockIdx.y selects the agent, and per agent the CTA count,
+ * tiling and reduction order are those of qs_ppo_update, so each agent's parameters, Adam state and statistics are bit-identical
+ * to a qs_ppo_update on the same rows.  Single rank (no grad / apply split).
+ *   qs_ppo_pop_create  owns [K][n_params] Adam moments, [K] steps, per-agent slabs and a device qs_ppo_hyper[K] (SB3 defaults)
+ *   qs_ppo_pop_set_hyper  copies the host array hp[K] to the device with cudaMemcpyAsync on `stream` (stream ordered: the update
+ *                      launch reads the device copy, so it stays capturable and the values can change between iterations)
+ *   params             device f32[K][n_params], 16-byte aligned; updated in place
+ *   obs/actions/old_logp/advantages/returns   the shared flat rollout buffers, as in qs_ppo_update
+ *   idx                device i64, row a at idx + a * idx_stride: the B flat rows of agent a's minibatch (idx_stride >= B)
+ *   stats_out          device f32[K][8] (qs_ppo_update's statistics per agent) or NULL
+ *   qs_ppo_pop_state   device pointers: m, v f32[K][n_params], step i64[K] */
+typedef struct qs_ppo_pop qs_ppo_pop;
+int qs_ppo_pop_create(int device, int obs_dim, int K, qs_ppo_pop** out);
+int qs_ppo_pop_destroy(qs_ppo_pop* o);
+int qs_ppo_pop_set_hyper(qs_ppo_pop* o, const qs_ppo_hyper* hp, void* stream);
+int qs_ppo_pop_update(qs_ppo_pop* o, float* params, const float* obs, const float* actions, const float* old_logp,
+                      const float* advantages, const float* returns, const int64_t* idx, int64_t idx_stride, int64_t B,
+                      float* stats_out, void* stream);
+int qs_ppo_pop_state(qs_ppo_pop* o, float** m, float** v, long long** step);
 
 /* Peer-memory exchange of the VecNormalize moments (multi-GPU) --------------------------------------------
  * The only exchange step of the sharded env path is the 2d+1 doubles (n, mean[d], M2[d]) each rank contributes to the running

@@ -195,6 +195,16 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.qs_ppo_apply.argtypes = [vp, vp, vp, C.POINTER(QsPpoHyper), vp, vp]
     lib.qs_ppo_state.argtypes = [vp] + [C.POINTER(vp)] * 4
     lib.qs_ppo_last_error.restype = C.c_char_p
+    lib.qs_ppo_pop_create.argtypes = [i32, i32, i32, C.POINTER(vp)]
+    lib.qs_ppo_pop_destroy.argtypes = [vp]
+    lib.qs_ppo_pop_set_hyper.argtypes = [vp, C.POINTER(QsPpoHyper), vp]
+    lib.qs_ppo_pop_update.argtypes = [vp] * 8 + [i64, i64, vp, vp]
+    lib.qs_ppo_pop_state.argtypes = [vp] + [C.POINTER(vp)] * 3
+    for name in ("qs_ppo_pop_create", "qs_ppo_pop_destroy", "qs_ppo_pop_set_hyper", "qs_ppo_pop_update", "qs_ppo_pop_state"):
+        getattr(lib, name).restype = C.c_int
+    lib.qs_policy_forward_pop.argtypes = [vp, i32, i32, vp, vp, i64, vp, vp, C.POINTER(C.c_float * 4), C.POINTER(C.c_float * 4), vp, vp, vp]
+    lib.qs_policy_forward_pop.restype = C.c_int
+    lib.qs_policy_last_error.restype = C.c_char_p
     for name in ("qs_ppo_create", "qs_ppo_destroy", "qs_ppo_update", "qs_ppo_grad", "qs_ppo_apply", "qs_ppo_state"):
         getattr(lib, name).restype = C.c_int
     lib.qs_pid_default_gains.argtypes = [C.POINTER(QsPidGains)]

@@ -110,112 +110,28 @@ __device__ __forceinline__ void layer(const float* __restrict__ A /*[K][RS]*/, c
 
 template <int OBS>
 __global__ void __launch_bounds__(POLICY_THREADS, 1) policy_forward_ffma_kernel(const PolicyArgs p) {
-    constexpr int RS = TILE;                       // activation row stride (floats)
-    extern __shared__ __align__(16) float smem[];
-    const PolicyLayout L{OBS};
-    float* sP = smem;                              // parameters
-    const int ptotal = (L.total() + 3) & ~3;
-    float* sX = sP + ptotal;                       // [OBS][RS]   normalised obs tile, k-major (shared by both halves)
-    float* sHa = sX + OBS * RS;                    // per half: [128][RS] (H1, later H3) and [64][RS] (H2)
-    constexpr int HALF_FLOATS = H1 * RS + H2 * RS;
-    float* sOut = sHa + 2 * HALF_FLOATS;           // [TILE][8]: 4 means, value
-    __shared__ double s_mean[32], s_istd[32];   // float64 like SB3's normalize_obs (see qs_vecnorm.cu)
+#include "qs_policy_ffma_body.cuh"
+}
 
-    const int tid = threadIdx.x;
-    for (int i = tid; i < L.total(); i += POLICY_THREADS) sP[i] = __ldg(p.params + i);
-    if (tid < OBS) {
-        double m = 0.0, is = 1.0;
-        if (p.norm) {
-            m = p.norm[1 + tid];
-            is = 1.0 / sqrt(p.norm[1 + OBS + tid] + (double)p.norm_eps);
-        }
-        s_mean[tid] = m;
-        s_istd[tid] = is;
-    }
-    __syncthreads();
+// population: blockIdx.y = agent a, whose blob is params + a * pstride and whose rows are [a*n, (a+1)*n) of every row buffer.
+// Rows are independent in the body (a fixed k-order per row), so each row is what policy_forward_ffma_kernel computes for it.
+struct PolicyPopArgs {
+    PolicyArgs p;                    // agent 0's view; n = rows per agent
+    int64_t pstride;                 // floats between consecutive agents' blobs
+};
 
-    const int net = tid >> 7;                      // 0 actor, 1 critic
-    const int t = tid & 127;
-    float* H1s = sHa + net * HALF_FLOATS;
-    float* H2s = H1s + H1 * RS;
-    const int64_t n_tiles = (p.n + TILE - 1) / TILE;
-
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int64_t e0 = tile * TILE;
-        const int valid = (int)((p.n - e0) < TILE ? (p.n - e0) : TILE);
-        // ---- obs tile: coalesced global read, (normalise), transposed store
-        for (int i = tid; i < TILE * OBS; i += POLICY_THREADS) {
-            const int e = i / OBS, k = i - e * OBS;
-            float x = 0.f;
-            if (e < valid) {
-                x = __ldcs(p.obs + e0 * OBS + i);
-                if (p.norm) {
-                    x = (float)(((double)x - s_mean[k]) * s_istd[k]);
-                    x = fminf(fmaxf(x, -p.norm_clip), p.norm_clip);
-                    if (p.obs_norm_out) p.obs_norm_out[e0 * OBS + i] = x;
-                }
-            }
-            sX[k * RS + e] = x;
-        }
-        __syncthreads();
-        // ---- trunk (per half)
-        layer<OBS, H1, RS>(sX, sP + L.w1(net), sP + L.b1(net), H1s, t);
-        half_barrier(net);
-        layer<H1, H2, RS>(H1s, sP + L.w2(net), sP + L.b2(net), H2s, t);
-        half_barrier(net);
-        layer<H2, H3, RS>(H2s, sP + L.w3(net), sP + L.b3(net), H1s, t);   // H3 overwrites H1
-        half_barrier(net);
-        // ---- heads: actor 4 outputs, critic 1; thread t -> env t%64, output pair t/64
-        {
-            const int e = t & 63, pair = t >> 6;
-            const float* Wh = sP + L.wh(net);
-            if (net == 0) {
-                float m0 = sP[L.bh(0) + 2 * pair], m1 = sP[L.bh(0) + 2 * pair + 1];
-#pragma unroll 8
-                for (int k = 0; k < H3; ++k) {
-                    const float h = H1s[k * RS + e];
-                    m0 = fmaf(h, Wh[k * NACT + 2 * pair], m0);
-                    m1 = fmaf(h, Wh[k * NACT + 2 * pair + 1], m1);
-                }
-                sOut[e * 8 + 2 * pair] = m0;
-                sOut[e * 8 + 2 * pair + 1] = m1;
-            } else if (pair == 0) {
-                float v = sP[L.bh(1)];
-#pragma unroll 8
-                for (int k = 0; k < H3; ++k) v = fmaf(H1s[k * RS + e], Wh[k * NACT], v);
-                sOut[e * 8 + 4] = v;
-            }
-        }
-        __syncthreads();
-        // ---- sample, log-prob, clip, store (64 threads, one env each; float4 rows -> coalesced)
-        if (tid < valid) {
-            const int64_t e = e0 + tid;
-            const float4 mu = *reinterpret_cast<const float4*>(sOut + tid * 8);
-            const float ls[4] = {sP[L.log_std()], sP[L.log_std() + 1], sP[L.log_std() + 2], sP[L.log_std() + 3]};
-            float4 eps = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (p.noise) eps = __ldcs(reinterpret_cast<const float4*>(p.noise) + e);
-            float4 a;
-            a.x = fmaf(__expf(ls[0]), eps.x, mu.x);
-            a.y = fmaf(__expf(ls[1]), eps.y, mu.y);
-            a.z = fmaf(__expf(ls[2]), eps.z, mu.z);
-            a.w = fmaf(__expf(ls[3]), eps.w, mu.w);
-            const float HALF_LOG_2PI = 0.9189385332046727f;
-            const float lp = -0.5f * (eps.x * eps.x + eps.y * eps.y + eps.z * eps.z + eps.w * eps.w) - (ls[0] + ls[1] + ls[2] + ls[3]) -
-                             4.0f * HALF_LOG_2PI;
-            reinterpret_cast<float4*>(p.actions)[e] = a;
-            if (p.actions_clipped) {
-                float4 c;
-                c.x = fminf(fmaxf(a.x, p.lo[0]), p.hi[0]);
-                c.y = fminf(fmaxf(a.y, p.lo[1]), p.hi[1]);
-                c.z = fminf(fmaxf(a.z, p.lo[2]), p.hi[2]);
-                c.w = fminf(fmaxf(a.w, p.lo[3]), p.hi[3]);
-                reinterpret_cast<float4*>(p.actions_clipped)[e] = c;
-            }
-            p.values[e] = sOut[tid * 8 + 4];
-            p.logp[e] = lp;
-        }
-        __syncthreads();
-    }
+template <int OBS>
+__global__ void __launch_bounds__(POLICY_THREADS, 1) policy_forward_pop_kernel(const PolicyPopArgs q) {
+    const int64_t a = blockIdx.y, r0 = a * q.p.n;
+    PolicyArgs p = q.p;
+    p.params += a * q.pstride;
+    p.obs += r0 * OBS;
+    if (p.noise) p.noise += r0 * NACT;
+    p.actions += r0 * NACT;
+    if (p.actions_clipped) p.actions_clipped += r0 * NACT;
+    p.values += r0;
+    p.logp += r0;
+#include "qs_policy_ffma_body.cuh"
 }
 
 static size_t policy_smem_bytes(int obs) {
@@ -300,6 +216,48 @@ int qs_policy_forward(const float* params, int obs_dim, const float* obs, const 
     if (err == cudaSuccess) err = cudaGetLastError();
     if (err != cudaSuccess) {
         snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward: %s", cudaGetErrorString(err));
+        return QS_ECUDA;
+    }
+    return QS_OK;
+}
+
+int qs_policy_forward_pop(const float* params, int obs_dim, int K, const float* obs, const float* noise, int64_t n,
+                          float* actions, float* actions_clipped, const float* clip_lo, const float* clip_hi, float* values,
+                          float* logp, void* stream) {
+    if (!params || !obs || !actions || !values || !logp || n < 0 || K < 1 || K > 65535 || (obs_dim != 17 && obs_dim != 20)) {
+        snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward_pop: bad argument (obs_dim 17 or 20, 1 <= K <= 65535, n >= 0)");
+        return QS_EINVAL;
+    }
+    if ((reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(obs) | reinterpret_cast<uintptr_t>(noise) |
+         reinterpret_cast<uintptr_t>(actions) | reinterpret_cast<uintptr_t>(actions_clipped)) & 15) {
+        snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward_pop: params, obs, noise, actions and actions_clipped must be 16-byte aligned");
+        return QS_EINVAL;
+    }
+    if (n == 0) return QS_OK;
+    PolicyPopArgs q;
+    PolicyArgs& a = q.p;
+    a.params = params; a.obs = obs; a.noise = noise; a.norm = nullptr; a.obs_norm_out = nullptr;
+    a.actions = actions; a.actions_clipped = actions_clipped; a.values = values; a.logp = logp; a.n = n;
+    a.norm_eps = 0.f; a.norm_clip = 0.f;
+    for (int i = 0; i < 4; ++i) { a.lo[i] = clip_lo ? clip_lo[i] : -3.4e38f; a.hi[i] = clip_hi ? clip_hi[i] : 3.4e38f; }
+    q.pstride = PolicyLayout{obs_dim}.total();
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const size_t smem = policy_smem_bytes(obs_dim);
+    const int64_t tiles = (n + TILE - 1) / TILE;
+    const dim3 grid((unsigned)(tiles < sms ? tiles : sms), (unsigned)K);
+    cudaError_t err;
+    if (obs_dim == 20) {
+        err = cudaFuncSetAttribute(policy_forward_pop_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (err == cudaSuccess) policy_forward_pop_kernel<20><<<grid, POLICY_THREADS, smem, (cudaStream_t)stream>>>(q);
+    } else {
+        err = cudaFuncSetAttribute(policy_forward_pop_kernel<17>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (err == cudaSuccess) policy_forward_pop_kernel<17><<<grid, POLICY_THREADS, smem, (cudaStream_t)stream>>>(q);
+    }
+    if (err == cudaSuccess) err = cudaGetLastError();
+    if (err != cudaSuccess) {
+        snprintf(g_policy_error, sizeof(g_policy_error), "qs_policy_forward_pop: %s", cudaGetErrorString(err));
         return QS_ECUDA;
     }
     return QS_OK;

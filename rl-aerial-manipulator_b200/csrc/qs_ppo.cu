@@ -41,6 +41,16 @@ struct qs_ppo {
     long long* step;                // Adam step count (device: graph-capturable)
 };
 
+struct qs_ppo_pop {
+    int device, obs_dim, n_params, max_grid, K;
+    float *m, *v;                   // [K][n_params] Adam moments, blob layout
+    float* partial;                 // [K][max_grid][n_params] per-CTA gradient slabs
+    double* loss_partial;           // [K][max_grid][NSTAT]
+    unsigned int* ticket;           // [K]
+    long long* step;                // [K] Adam step counts
+    qs_ppo_hyper* hyper;            // [K] device copy of the hyper-parameters (qs_ppo_pop_set_hyper)
+};
+
 namespace qs {
 namespace ppo {
 
@@ -344,8 +354,9 @@ __device__ __forceinline__ void adam_apply(const Args& a, const float* __restric
     if (stats_extra && threadIdx.x == 0) *stats_extra = total;
 }
 
+// the whole update of one agent by the CTAs blockIdx.x = 0 .. gridDim.x - 1 (the solo kernel and the population kernel)
 template <int D>
-__global__ void __launch_bounds__(THREADS, 1) ppo_update_kernel(const Args a) {
+__device__ __forceinline__ void ppo_update_body(const Args& a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& s = *reinterpret_cast<Smem*>(smem_raw);
     const int tid = threadIdx.x;
@@ -532,6 +543,11 @@ __global__ void __launch_bounds__(THREADS, 1) ppo_update_kernel(const Args a) {
     if (a.apply) adam_apply(a, g, nsq, nullptr);
 }
 
+template <int D>
+__global__ void __launch_bounds__(THREADS, 1) ppo_update_kernel(const Args a) {
+    ppo_update_body<D>(a);
+}
+
 // several ranks: clipping + Adam on an already averaged gradient
 __global__ void __launch_bounds__(THREADS, 1) ppo_apply_kernel(const Args a, const float* __restrict__ grad) {
     __shared__ double red[40];
@@ -542,6 +558,48 @@ __global__ void __launch_bounds__(THREADS, 1) ppo_apply_kernel(const Args a, con
     }
     nsq = block_sum(nsq, red);
     adam_apply(a, grad, nsq, a.stats_out ? a.stats_out + 4 : nullptr);
+}
+
+// population: blockIdx.y = agent.  The agent's Args live in shared memory, so the body reads them like the solo kernel's
+// parameter-space Args instead of holding 15 per-agent pointers in registers.
+struct PopArgs {
+    float* params;                  // [K][n_params]
+    const float *obs, *actions, *old_logp, *adv, *ret;    // the shared flat rollout buffers
+    const int64_t* idx;             // [K][idx_stride]
+    int64_t idx_stride, B;
+    const qs_ppo_hyper* hp;         // device [K]
+    float *m, *v, *partial;         // [K][n_params], [K][n_params], [K][max_grid][n_params]
+    double* loss_partial;           // [K][max_grid][NSTAT]
+    float* stats_out;               // [K][NSTAT] or null
+    unsigned int* ticket;           // [K]
+    long long* step;                // [K]
+    int n_params, max_grid;
+};
+
+template <int D>
+__global__ void __launch_bounds__(THREADS, 1) ppo_update_pop_kernel(const PopArgs p) {
+    __shared__ Args a;
+    if (threadIdx.x == 0) {
+        const int k = blockIdx.y;
+        const size_t np = (size_t)p.n_params;
+        a.params = p.params + k * np;
+        a.obs = p.obs; a.actions = p.actions; a.old_logp = p.old_logp; a.adv = p.adv; a.ret = p.ret;
+        a.idx = p.idx + k * p.idx_stride;
+        a.B = p.B;
+        a.hp = p.hp[k];
+        a.m = p.m + k * np;
+        a.v = p.v + k * np;
+        a.partial = p.partial + (size_t)k * p.max_grid * np;
+        a.loss_partial = p.loss_partial + (size_t)k * p.max_grid * NSTAT;
+        a.grad_out = nullptr;
+        a.stats_out = p.stats_out ? p.stats_out + (size_t)k * NSTAT : nullptr;
+        a.ticket = p.ticket + k;
+        a.step = p.step + k;
+        a.n_params = p.n_params;
+        a.apply = 1;
+    }
+    __syncthreads();
+    ppo_update_body<D>(a);
 }
 
 static int fail(const char* what, cudaError_t err) {
@@ -569,6 +627,24 @@ static int launch_update(qs_ppo* o, float* params, const float* obs, const float
     }
     if (err == cudaSuccess) err = cudaGetLastError();
     if (err != cudaSuccess) return fail("ppo_update_kernel", err);
+    return QS_OK;
+}
+
+static int launch_update_pop(qs_ppo_pop* o, const PopArgs& a, cudaStream_t st) {
+    // per agent the grid of the solo kernel (launch_update): min(tiles, max_grid) CTAs, so every agent's tiling and slab-sum
+    // order, and with them its arithmetic, are those of qs_ppo_update
+    const int64_t tiles = (a.B + TS - 1) / TS;
+    const dim3 grid((unsigned)(tiles < o->max_grid ? tiles : o->max_grid), (unsigned)o->K);
+    cudaError_t err;
+    if (o->obs_dim == 20) {
+        err = cudaFuncSetAttribute(ppo_update_pop_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+        if (err == cudaSuccess) ppo_update_pop_kernel<20><<<grid, THREADS, sizeof(Smem), st>>>(a);
+    } else {
+        err = cudaFuncSetAttribute(ppo_update_pop_kernel<17>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+        if (err == cudaSuccess) ppo_update_pop_kernel<17><<<grid, THREADS, sizeof(Smem), st>>>(a);
+    }
+    if (err == cudaSuccess) err = cudaGetLastError();
+    if (err != cudaSuccess) return fail("ppo_update_pop_kernel", err);
     return QS_OK;
 }
 
@@ -672,6 +748,96 @@ int qs_ppo_apply(qs_ppo* o, float* params, const float* grad, const qs_ppo_hyper
     err = cudaGetLastError();
     if (err != cudaSuccess) return fail("ppo_apply_kernel", err);
     return QS_OK;
+}
+
+int qs_ppo_pop_destroy(qs_ppo_pop* o) {
+    if (!o) return QS_OK;
+    cudaSetDevice(o->device);
+    cudaDeviceSynchronize();
+    cudaFree(o->m); cudaFree(o->v); cudaFree(o->partial); cudaFree(o->loss_partial); cudaFree(o->ticket); cudaFree(o->step);
+    cudaFree(o->hyper);
+    delete o;
+    return QS_OK;
+}
+
+int qs_ppo_pop_create(int device, int obs_dim, int K, qs_ppo_pop** out) {
+    if (!out || (obs_dim != 17 && obs_dim != 20) || K < 1 || K > 65535) {
+        snprintf(g_error, sizeof(g_error), "qs_ppo_pop_create: bad argument (obs_dim 17 or 20, 1 <= K <= 65535)");
+        return QS_EINVAL;
+    }
+    cudaError_t err = cudaSetDevice(device);
+    if (err != cudaSuccess) return fail("qs_ppo_pop_create", err);
+    qs_ppo_pop* o = new (std::nothrow) qs_ppo_pop();
+    if (!o) { snprintf(g_error, sizeof(g_error), "qs_ppo_pop_create: out of host memory"); return QS_EINVAL; }
+    memset(o, 0, sizeof(*o));
+    o->device = device; o->obs_dim = obs_dim; o->n_params = qs_ppo_n_params(obs_dim); o->K = K;
+    int sms = 0;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    o->max_grid = sms > 0 ? sms : 148;
+    const size_t pb = sizeof(float) * (size_t)o->n_params * K;
+    qs_ppo_hyper* h = new (std::nothrow) qs_ppo_hyper[K];
+    if (!h) { delete o; snprintf(g_error, sizeof(g_error), "qs_ppo_pop_create: out of host memory"); return QS_EINVAL; }
+    for (int k = 0; k < K; ++k) qs_ppo_default_hyper(h + k);
+    if ((err = cudaMalloc(&o->m, pb)) != cudaSuccess || (err = cudaMalloc(&o->v, pb)) != cudaSuccess ||
+        (err = cudaMalloc(&o->partial, pb * o->max_grid)) != cudaSuccess ||
+        (err = cudaMalloc(&o->loss_partial, sizeof(double) * NSTAT * o->max_grid * K)) != cudaSuccess ||
+        (err = cudaMalloc(&o->ticket, sizeof(unsigned int) * K)) != cudaSuccess || (err = cudaMalloc(&o->step, sizeof(long long) * K)) != cudaSuccess ||
+        (err = cudaMalloc(&o->hyper, sizeof(qs_ppo_hyper) * K)) != cudaSuccess ||
+        (err = cudaMemset(o->m, 0, pb)) != cudaSuccess || (err = cudaMemset(o->v, 0, pb)) != cudaSuccess ||
+        (err = cudaMemset(o->ticket, 0, sizeof(unsigned int) * K)) != cudaSuccess ||
+        (err = cudaMemset(o->step, 0, sizeof(long long) * K)) != cudaSuccess ||
+        (err = cudaMemcpy(o->hyper, h, sizeof(qs_ppo_hyper) * K, cudaMemcpyHostToDevice)) != cudaSuccess ||
+        (err = cudaDeviceSynchronize()) != cudaSuccess) {
+        delete[] h;
+        qs_ppo_pop_destroy(o);
+        return fail("qs_ppo_pop_create", err);
+    }
+    delete[] h;
+    *out = o;
+    return QS_OK;
+}
+
+int qs_ppo_pop_set_hyper(qs_ppo_pop* o, const qs_ppo_hyper* hp, void* stream) {
+    if (!o || !hp) { snprintf(g_error, sizeof(g_error), "qs_ppo_pop_set_hyper: null argument"); return QS_EINVAL; }
+    cudaError_t err = cudaSetDevice(o->device);
+    if (err == cudaSuccess) err = cudaMemcpyAsync(o->hyper, hp, sizeof(qs_ppo_hyper) * o->K, cudaMemcpyHostToDevice, (cudaStream_t)stream);
+    if (err != cudaSuccess) return fail("qs_ppo_pop_set_hyper", err);
+    return QS_OK;
+}
+
+int qs_ppo_pop_state(qs_ppo_pop* o, float** m, float** v, long long** step) {
+    if (!o) { snprintf(g_error, sizeof(g_error), "qs_ppo_pop_state: null handle"); return QS_EINVAL; }
+    if (m) *m = o->m;
+    if (v) *v = o->v;
+    if (step) *step = o->step;
+    return QS_OK;
+}
+
+int qs_ppo_pop_update(qs_ppo_pop* o, float* params, const float* obs, const float* actions, const float* old_logp,
+                      const float* advantages, const float* returns, const int64_t* idx, int64_t idx_stride, int64_t B,
+                      float* stats_out, void* stream) {
+    if (!params || !obs || !actions || !old_logp || !advantages || !returns || !idx || B < 1 || idx_stride < B) {
+        snprintf(g_error, sizeof(g_error), "qs_ppo_pop_update: null argument, empty minibatch or idx_stride < B");
+        return QS_EINVAL;
+    }
+    if ((reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(actions)) & 15) {
+        snprintf(g_error, sizeof(g_error), "qs_ppo_pop_update: params and actions must be 16-byte aligned");
+        return QS_EINVAL;
+    }
+    if ((reinterpret_cast<uintptr_t>(idx) & 7) | (reinterpret_cast<uintptr_t>(stats_out) & 3)) {
+        snprintf(g_error, sizeof(g_error), "qs_ppo_pop_update: idx must be 8-byte and stats_out 4-byte aligned");
+        return QS_EINVAL;
+    }
+    if (!o) { snprintf(g_error, sizeof(g_error), "qs_ppo_pop_update: null handle"); return QS_EINVAL; }
+    const cudaError_t err = cudaSetDevice(o->device);
+    if (err != cudaSuccess) return fail("qs_ppo_pop_update", err);
+    PopArgs a;
+    memset(&a, 0, sizeof(a));
+    a.params = params; a.obs = obs; a.actions = actions; a.old_logp = old_logp; a.adv = advantages; a.ret = returns;
+    a.idx = idx; a.idx_stride = idx_stride; a.B = B; a.hp = o->hyper; a.m = o->m; a.v = o->v; a.partial = o->partial;
+    a.loss_partial = o->loss_partial; a.stats_out = stats_out; a.ticket = o->ticket; a.step = o->step;
+    a.n_params = o->n_params; a.max_grid = o->max_grid;
+    return launch_update_pop(o, a, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -40,5 +40,11 @@ T = 8
 r = torch.randn((T, n), device="cuda"); v = torch.randn((T, n), device="cuda")
 s = (torch.rand((T, n), device="cuda") < 0.1).to(torch.uint8)
 gae(r, v, s, torch.randn(n, device="cuda"), (torch.rand(n, device="cuda") < 0.1).to(torch.uint8), 0.995, 0.9)
+# population kernels: K agents at a ragged n (qs_policy_forward_pop), one population minibatch update (qs_ppo_pop_update)
+from rl_aerial_manipulator_b200.population import PopulationPPO
+pop = PopulationPPO(BatchedQuadEnv(3 * 37, env_version=2, seed=1), 3, [0, 1, 2], n_steps=5, batch_size=100, n_epochs=1, rollout_graph=False)
+pop.collect_rollouts()
+pop.train()
+pop.close()
 torch.cuda.synchronize()
 print("SANITIZE_SMOKE_DONE")
